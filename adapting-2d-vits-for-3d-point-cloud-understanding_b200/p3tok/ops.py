@@ -366,6 +366,7 @@ def fps_with_knn_prepare(x: torch.Tensor, start_idx: torch.Tensor, npoint: int) 
     c2 (B = 128) the preparation's 1024-thread sort shares SMs with FPS, whose dependent iterations are the critical
     path, and the step gets slower (0.972 -> 1.012 ms; c5 2.34 -> 2.38) - so "auto" overlaps only when 2 B <= #SMs.
     P3TOK_OVERLAP=0 / 1 forces back-to-back / overlapped."""
+    _need_cuda("fps_with_knn_prepare", x)         # before the stream calls below, which reject CPU devices
     if _use_culled_fps(int(x.shape[0]), int(x.shape[1]), npoint):
         # round 2: the preparation comes FIRST - FPS itself runs on the sorted blocks (p3tok_fps_sorted), then the kNN query
         ws = knn_prepare(x)

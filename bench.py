@@ -2,7 +2,7 @@
 """bench.py - tokenized clouds/sec of the point-patch tokenizer (FPS + kNN + gather/normalise + embed).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl p3tok|reference] [--workload c2|c2v|c1|c3|c4|c5|c5w]
-                    [--clouds uniform|clustered|both] [--token-dtype bf16|f32] [--precision bf16|fp32]
+                    [--clouds uniform|clustered|both] [--token-dtype bf16|f32] [--precision bf16|fp32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch of synthetic clouds.  Default workload = BASELINE.json
@@ -13,17 +13,19 @@ final token all-gather over NVLink timed inside `e2e_with_gather`; a short run o
 as `c5_strong` so the driver's 1/2/4/8-GPU sweep records the curve.
 
 Printed JSON line (rank 0):
-  value     whole-job clouds/s with inputs resident in HBM: K steps per timed window, device-timed (CUDA events on the
-            launching stream), max over ranks; windows are repeated until >= 1 s of device time and the MEDIAN window is
-            reported (a 20-step run of a 1 ms step is otherwise a 20 ms sample).
+  value     whole-job clouds/s with inputs resident in HBM: one timed window of exactly K steps, device-timed (CUDA events
+            on the launching stream), max over ranks.
   e2e       the same metric through the public serving call with HOST buffers: pinned H2D copy of the clouds and start
-            indices and D2H read of the tokens inside the timed region, every step.
+            indices and D2H read of the tokens inside the timed region, every step (again exactly K steps).
   roofline  the dominant kernel family (patch embedding) against the measured bf16 peak of MEASURED_PEAKS.json - the
             burst figure when the clock record shows burst conditions (no power cap), else the sustained one; both
             fractions are printed.  `traffic` = measured DRAM bytes of those kernels (ncu), from profiles/r02_traffic.json.
   cpu_baseline  the reference tokenizer's torch-CPU port (oracle/port.py) timed on this box's host cores.
-`--impl reference` times that port alone (the reference is pure Python and /root/reference does not travel to the GPU
-box; see DESIGN.md) and prints the same line with "impl": "reference".
+`--impl reference` times that port alone (the reference is pure Python; see DESIGN.md) and prints the same line with
+"impl": "reference".
+`--dump-outputs DIR` writes what the timed path returned in its last step as DIR/<name>.npy (float32; an output above
+64 MB is cut to a fixed, seeded sample of whole clouds).  The inputs depend on the arguments only, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -40,12 +42,26 @@ for _p in (ROOT, PKG):
     if _p not in sys.path:
         sys.path.insert(0, _p)
 
-import numpy as np  # noqa: E402,F401
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "tokenized clouds/sec (FPS+kNN+embed)"
 UNIT = "clouds/s"
-MIN_WINDOW_S = 1.0          # device-timed windows are repeated until this much time has been measured
+DUMP_MAX_BYTES = 64 * 10**6     # --dump-outputs: total size of the written arrays
+
+
+def dump_outputs(directory, outputs):
+    """Writes every tensor of `outputs` ({name: tensor}) as float32 <directory>/<name>.npy.  Each output gets an equal
+    share of DUMP_MAX_BYTES; one above its share is cut to a fixed sample of whole clouds (dim 0, seed 0), so the dump
+    stays comparable between runs with the same arguments."""
+    os.makedirs(directory, exist_ok=True)
+    arrays = {n: t.detach().float().cpu().numpy() for n, t in outputs.items()}
+    budget = (DUMP_MAX_BYTES - 4096 * len(arrays)) // len(arrays)           # 4 KB per file for the .npy header
+    for name, a in arrays.items():
+        if a.nbytes > budget:
+            keep = max(1, budget * a.shape[0] // a.nbytes)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 # name -> family, clouds per GPU (weak) or per job (strong), N, centres G, k, embed E, description
 WORKLOADS = {
@@ -286,8 +302,10 @@ def run_reference(args, w, rank, world):
             run(xt, stt)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            run(xt, stt)
+            out = run(xt, stt)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"tokens": out})
     v = sample * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -304,7 +322,7 @@ def run_reference(args, w, rank, world):
 
 
 class Harness:
-    """One workload on this rank's GPU: builds the model, the L2-defeating input pool and the graphs, and times windows."""
+    """One workload on this rank's GPU: builds the model, the L2-defeating input pool and the graphs, and times steps."""
 
     def __init__(self, w, B, precision, token_dtype, device, rank, world, kind, eager=False, streams=2):
         import torch.distributed as dist
@@ -361,34 +379,26 @@ class Harness:
                     self.step_dev(i)
             torch.cuda.synchronize()
 
-    def time_device_windows(self, steps, min_s=MIN_WINDOW_S, max_windows=400):
-        """[ms per window]: EXACTLY `steps` steps per window, barrier + synchronize on both sides, CUDA events on the
-        launching stream; windows repeat until `min_s` of device time has been measured (every rank runs the same count:
-        the decision is taken on the max-over-ranks running total)."""
-        out = []
-        total = 0.0
+    def time_device(self, steps):
+        """ms of EXACTLY `steps` steps, barrier + synchronize on both sides, CUDA events on the launching stream, max over
+        ranks.  `self.last_out` is what the last step returned."""
         with torch.no_grad():
-            while True:
-                self.barrier()
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                main = torch.cuda.current_stream(self.device)
-                e0.record()
-                multi = self.gdev is not None and self.dev_streams[0] is not None
-                if multi:
-                    for s_ in self.dev_streams:
-                        s_.wait_stream(main)           # the step streams start after the start event ...
-                for i in range(steps):
-                    self.step_dev(i + len(out))
-                if multi:
-                    for s_ in self.dev_streams:
-                        main.wait_stream(s_)           # ... and the end event is recorded after both have drained
-                e1.record()
-                self.barrier()
-                ms = self.reduce_max(e0.elapsed_time(e1))
-                out.append(ms)
-                total += ms
-                if total >= 1e3 * min_s or len(out) >= max_windows:
-                    return out
+            self.barrier()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            main = torch.cuda.current_stream(self.device)
+            e0.record()
+            multi = self.gdev is not None and self.dev_streams[0] is not None
+            if multi:
+                for s_ in self.dev_streams:
+                    s_.wait_stream(main)           # the step streams start after the start event ...
+            for i in range(steps):
+                self.last_out = self.step_dev(i)
+            if multi:
+                for s_ in self.dev_streams:
+                    main.wait_stream(s_)           # ... and the end event is recorded after both have drained
+            e1.record()
+            self.barrier()
+            return self.reduce_max(e0.elapsed_time(e1))
 
     def reduce_max(self, v):
         if self.world == 1:
@@ -415,27 +425,20 @@ class Harness:
         ho = self.graphs[0].host_output
         self.d2h_bytes = ho.numel() * ho.element_size()
 
-    def time_e2e_windows(self, steps, gather=None, min_s=MIN_WINDOW_S, max_windows=400):
-        """[ms per window] wall clock (the host is part of this number), barrier + synchronize on both sides.
+    def time_e2e(self, steps, gather=None):
+        """ms of EXACTLY `steps` steps, wall clock (the host is part of this number), barrier + synchronize on both sides.
         gather: optional callable(graph) enqueued after each step on the step's stream (the token all-gather)."""
-        out = []
-        total = 0.0
-        while True:
-            self.barrier()
-            t0 = time.perf_counter()
-            for i in range(steps):
-                g = self.graphs[i % len(self.graphs)]
-                g.replay()
-                if gather is not None:
-                    gather(g)
-            for g in self.graphs:
-                g.synchronize()
-            self.barrier()
-            ms = self.reduce_max(1e3 * (time.perf_counter() - t0))
-            out.append(ms)
-            total += ms
-            if total >= 1e3 * min_s or len(out) >= max_windows:
-                return out
+        self.barrier()
+        t0 = time.perf_counter()
+        for i in range(steps):
+            g = self.graphs[i % len(self.graphs)]
+            g.replay()
+            if gather is not None:
+                gather(g)
+        for g in self.graphs:
+            g.synchronize()
+        self.barrier()
+        return self.reduce_max(1e3 * (time.perf_counter() - t0))
 
     def copy_bandwidth(self):
         """Pinned H2D and D2H GB/s of this rank while every rank copies at once (names the e2e limiter at N > 1)."""
@@ -496,9 +499,11 @@ def run_p3tok(args, w, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    dev_windows = H.time_device_windows(args.steps)
+    dev_ms = H.time_device(args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"tokens": H.last_out})
     H.prepare_e2e()
-    e2e_windows = H.time_e2e_windows(args.steps)
+    e2e_ms = H.time_e2e(args.steps)
     clocks = sampler.stop() if rank == 0 else None
     with torch.no_grad():
         # the host-to-host graph and the device graph return the same tokens as the eager module call on the same clouds
@@ -518,9 +523,9 @@ def run_p3tok(args, w, rank, world, local_rank):
             for i in range(3):
                 H32.run(H32.pool[0], H32.st_pool[0])
         H32.prepare_e2e()
-        win = H32.time_e2e_windows(args.steps, min_s=0.3)
-        e2e_f32 = {"value": B * world * args.steps / (statistics.median(win) / 1e3), "unit": UNIT,
-                   "d2h_bytes_per_step": H32.d2h_bytes, "ms_per_step": statistics.median(win) / args.steps}
+        ms = H32.time_e2e(args.steps)
+        e2e_f32 = {"value": B * world * args.steps / (ms / 1e3), "unit": UNIT,
+                   "d2h_bytes_per_step": H32.d2h_bytes, "ms_per_step": ms / args.steps}
         del H32
     gather_info = None
     if world > 1:
@@ -530,7 +535,7 @@ def run_p3tok(args, w, rank, world, local_rank):
         def gather(g):
             with torch.cuda.stream(g.stream):
                 dist.all_gather_into_tensor(gbuf[0 if g is H.graphs[0] else 1], g.output)
-        win = H.time_e2e_windows(args.steps, gather=gather, min_s=0.5)
+        ms = H.time_e2e(args.steps, gather=gather)
         H.barrier()
         g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         g0.record()
@@ -538,22 +543,21 @@ def run_p3tok(args, w, rank, world, local_rank):
             dist.all_gather_into_tensor(gbuf[0], out0)
         g1.record()
         H.barrier()
-        gather_info = {"e2e_with_gather": B * world * args.steps / (statistics.median(win) / 1e3),
-                       "ms_per_step": statistics.median(win) / args.steps,
+        gather_info = {"e2e_with_gather": B * world * args.steps / (ms / 1e3),
+                       "ms_per_step": ms / args.steps,
                        "allgather_alone_ms": H.reduce_max(g0.elapsed_time(g1) / 5),
                        "gathered_bytes_per_rank": gbuf[0].numel() * gbuf[0].element_size()}
 
-    # ---- the other input kind (north star: uniform AND clustered clouds), shorter windows
+    # ---- the other input kind (north star: uniform AND clustered clouds)
     other = None
     if len(kinds) > 1:
         H2 = Harness(w, B, precision, tok_dtype, device, rank, world, kinds[1], args.eager, args.streams)
         H2.prepare_device_loop(3)
-        win = H2.time_device_windows(args.steps, min_s=0.3)
+        ms = H2.time_device(args.steps)
         H2.prepare_e2e()
-        ewin = H2.time_e2e_windows(args.steps, min_s=0.3)
-        other = {"clouds": kinds[1], "value": B * world * args.steps / (statistics.median(win) / 1e3),
-                 "ms_per_step": statistics.median(win) / args.steps,
-                 "e2e": B * world * args.steps / (statistics.median(ewin) / 1e3)}
+        ems = H2.time_e2e(args.steps)
+        other = {"clouds": kinds[1], "value": B * world * args.steps / (ms / 1e3), "ms_per_step": ms / args.steps,
+                 "e2e": B * world * args.steps / (ems / 1e3)}
         del H2
 
     # ---- per-stage device times (separate pass, CUDA events on the launching stream around every C-ABI call)
@@ -582,8 +586,6 @@ def run_p3tok(args, w, rank, world, local_rank):
 
     if rank != 0:
         return
-    dev_ms = statistics.median(dev_windows)
-    e2e_ms = statistics.median(e2e_windows)
     clouds = B * world * args.steps
     value = clouds / (dev_ms / 1e3)
     work = algorithmic_work(w)
@@ -611,13 +613,12 @@ def run_p3tok(args, w, rank, world, local_rank):
                    "step": "eager module call" if args.eager else
                            f"CUDA-graph replay of the module call, {args.streams} step(s) in flight on as many streams",
                    "host_cores_of_rank0": cores},
-        "timing": {"windows": len(dev_windows), "steps_per_window": args.steps, "timed_device_s": sum(dev_windows) / 1e3,
-                   "ms_per_step_min": min(dev_windows) / args.steps, "ms_per_step_max": max(dev_windows) / args.steps,
-                   "statistic": "median window", "e2e_windows": len(e2e_windows), "timed_e2e_s": sum(e2e_windows) / 1e3},
+        "timing": {"timed_steps": args.steps, "timed_device_s": dev_ms / 1e3, "timed_e2e_s": e2e_ms / 1e3,
+                   "statistic": "one timed run of --steps steps"},
         "e2e": {"value": clouds / (e2e_ms / 1e3), "unit": UNIT, "h2d_bytes_per_step": H.h2d_bytes,
                 "d2h_bytes_per_step": H.d2h_bytes, "ms_per_step": e2e_ms / args.steps,
                 "copy_GBps_per_rank_all_ranks_busy": {k: round(v, 1) for k, v in copy_bw.items()}},
-        "gpu_launches": int(H.launches_per_step * args.steps * len(dev_windows)),
+        "gpu_launches": int(H.launches_per_step * args.steps),
         "gpu_launches_per_step": int(H.launches_per_step),
         "clocks": clocks,
         "stage_ms_per_step": {k: round(v, 4) for k, v in sorted(stage_ms.items())},
@@ -663,19 +664,20 @@ def run_p3tok(args, w, rank, world, local_rank):
 
 def c5_strong_probe(args, rank, world, device, precision, tok_dtype):
     """BASELINE configs[4]: B = 4096 clouds per step split 4096/world per GPU, final all-gather of the (4096/world, 64, 256)
-    token shards inside the e2e step.  Short windows (0.3 s); strong scaling: value = 4096 clouds / max-over-ranks step time."""
+    token shards inside the e2e step, timed over --steps steps; strong scaling: value = 4096 clouds / max-over-ranks step
+    time."""
     import torch.distributed as dist
     w = dict(WORKLOADS["c5"])
     B = per_gpu_clouds(w, world)
     H = Harness(w, B, precision, tok_dtype, device, rank, world, "uniform")
     H.prepare_device_loop(3)
-    steps = 10
-    win = H.time_device_windows(steps, min_s=0.3)
+    steps = args.steps
+    ms = H.time_device(steps)
     H.prepare_e2e()
-    ewin = H.time_e2e_windows(steps, min_s=0.3)
+    ems = H.time_e2e(steps)
     res = {"workload": w["desc"], "scaling": "strong", "clouds_per_step": w["B"], "clouds_per_gpu": B,
-           "value": w["B"] * steps / (statistics.median(win) / 1e3), "ms_per_step": statistics.median(win) / steps,
-           "e2e": w["B"] * steps / (statistics.median(ewin) / 1e3), "e2e_ms_per_step": statistics.median(ewin) / steps,
+           "value": w["B"] * steps / (ms / 1e3), "ms_per_step": ms / steps,
+           "e2e": w["B"] * steps / (ems / 1e3), "e2e_ms_per_step": ems / steps,
            "h2d_bytes_per_step": H.h2d_bytes, "d2h_bytes_per_step": H.d2h_bytes}
     if world > 1:
         out0 = H.graphs[0].output
@@ -684,14 +686,15 @@ def c5_strong_probe(args, rank, world, device, precision, tok_dtype):
         def gather(g):
             with torch.cuda.stream(g.stream):
                 dist.all_gather_into_tensor(gbuf[0 if g is H.graphs[0] else 1], g.output)
-        gwin = H.time_e2e_windows(steps, gather=gather, min_s=0.3)
-        res["e2e_with_gather"] = w["B"] * steps / (statistics.median(gwin) / 1e3)
-        res["e2e_with_gather_ms_per_step"] = statistics.median(gwin) / steps
+        gms = H.time_e2e(steps, gather=gather)
+        res["e2e_with_gather"] = w["B"] * steps / (gms / 1e3)
+        res["e2e_with_gather_ms_per_step"] = gms / steps
         res["gathered_bytes_per_rank"] = gbuf[0].numel() * gbuf[0].element_size()
     return res
 
 
 def main():
+    sys.dont_write_bytecode = True      # the project modules are imported from here on; the source tree may be read-only
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=100)
@@ -708,7 +711,10 @@ def main():
     ap.add_argument("--streams", type=int, default=0, help="steps in flight (graphs replayed round-robin on as many streams) in the device-resident and e2e loops; 0 = auto: 2, up to 4 when the batch is well below the SM count")
     ap.add_argument("--ncu", type=int, default=0, help="profiling aid: run N eager steps between cudaProfilerStart/Stop and exit (no timing)")
     ap.add_argument("--eager", action="store_true", help="time the Python-dispatched module call instead of the CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     w = dict(WORKLOADS[args.workload])
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,8 +1,9 @@
-"""Import the UNMODIFIED reference tokenizer from /root/reference (build container only).
+"""Import the UNMODIFIED reference tokenizer from a checkout of the original project: oracle/_ref/ (git-ignored,
+not part of this repository) or the directory named by P3TOK_REFERENCE_ROOT.
 
 TEST INFRASTRUCTURE - not product code.  Only `tests/`, `tests/golden/make_golden.py`
-and ad-hoc probes may use this.  `/root/reference` does not exist on the GPU box, so
-nothing that runs there may call `load()`; use `available()` to gate.
+and ad-hoc probes may use this.  Where there is no checkout nothing may call `load()`;
+use `available()` to gate.
 
 The reference package imports `timm` and `h5py` at package-import time
 (src/models/__init__.py:1 -> vit.py:1, src/data/__init__.py:1 -> scanobjectnn.py:2);
@@ -13,7 +14,7 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("P3TOK_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("P3TOK_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 def available() -> bool:

@@ -1,7 +1,7 @@
-"""Generate tests/golden/*.npz from the UNMODIFIED reference (build container only).
+"""Generate tests/golden/*.npz from the UNMODIFIED reference.
 
 Run:  python tests/golden/make_golden.py
-Needs /root/reference (read-only).  The reference's internal `torch.randint` draw for the
+Needs a checkout of the original project (read-only; oracle/ref_loader.py says where).  The reference's internal `torch.randint` draw for the
 first FPS index (src/data/sampler.py:20, src/models/pix4point.py:30) is substituted by the
 synthetic start indices for the duration of each call; nothing else is touched.
 While generating, the script also asserts that oracle/port.py is bit-identical to the

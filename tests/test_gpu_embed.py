@@ -199,7 +199,7 @@ def test_cuda_graph_replay_matches_eager():
     assert torch.equal(g(x0, s0), net(x0, s0))
 
 
-def test_fused_pair_kernel_matches_layerwise(monkeypatch):
+def test_fused_pair_kernel_matches_layerwise(monkeypatch, tmp_path):
     """embed_fused.cu (two layers per kernel, hidden activation kept on-chip; opt-in via P3TOK_FUSED=1) against the
     default layer-by-layer tensor-core path: same bf16 arithmetic, different accumulation grouping."""
     _skip_if_unbuilt("bf16")
@@ -214,7 +214,7 @@ def test_fused_pair_kernel_matches_layerwise(monkeypatch):
         "torch.save(net(x, st).cpu(), sys.argv[1])")
     outs = []
     for flag in ("0", "1"):
-        path = f"/tmp/p3tok_fused_{flag}.pt"
+        path = str(tmp_path / f"fused_{flag}.pt")
         env = dict(os.environ, P3TOK_FUSED=flag)
         subprocess.run([sys.executable, "-c", code, path], check=True, env=env, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
         outs.append(torch.load(path))
@@ -261,7 +261,7 @@ def test_pointvit_tokens_module():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("W,ng", [(128, 8), (128, 4099), (64, 777)])
-def test_stage_kernel_matches_arithmetic_model_and_layerwise(W, ng):
+def test_stage_kernel_matches_arithmetic_model_and_layerwise(W, ng, tmp_path):
     """embed_stage.cu (concat + output layer + pool of a narrow P3Embed stage in one kernel, weights resident in
     shared memory) against a torch model of its arithmetic and against the layer-by-layer tensor-core path
     (P3TOK_STAGE=0 in a subprocess); ragged tile counts (ng not a multiple of 8 patches = 256 rows)."""
@@ -278,7 +278,7 @@ def test_stage_kernel_matches_arithmetic_model_and_layerwise(W, ng):
     model = bf16_emulation(mlp, rows.to(dev()), k)
     err = float((tok - model).abs().max() / model.abs().max())
     assert err < 2e-3, err
-    path_in, path_out = f"/tmp/p3tok_stage_in_{W}_{ng}.pt", f"/tmp/p3tok_stage_out_{W}_{ng}.pt"
+    path_in, path_out = str(tmp_path / "stage_in.pt"), str(tmp_path / "stage_out.pt")
     torch.save(rows, path_in)
     code = (
         "import sys, os; sys.path.insert(0, os.path.join(os.getcwd(), 'adapting-2d-vits-for-3d-point-cloud-understanding_b200'));"

@@ -120,6 +120,26 @@ def test_state_dict_loads_from_reference_modules():
     assert mine2.out_channels == r2.out_channels and mine2.channel_list == r2.channel_list
 
 
+def test_state_dicts_have_the_layouts_the_reference_modules_accepted():
+    """tests/golden/make_golden.py loaded these synthetic state dicts into the reference's own modules with strict=True
+    (apf_height: PointNet encoder E=48 on 8 channels; p4p_2stage / p4p_2stage_k32: P3Embed 1/16 with E=64 / 256;
+    vit_small: APFViTLayer(64, 2) and ClassificationHead(64, 15)), so their key -> shape maps are the reference's.
+    The modules here must have exactly those maps and load them strictly."""
+    from p3tok.apf_model import APFViTLayer, ClassificationHead
+
+    def same_layout(module, sd):
+        shapes = lambda d: {k: tuple(v.shape) or (1,) for k, v in d.items()}     # num_batches_tracked: () here, (1,) stored
+        assert shapes(module.state_dict()) == shapes(sd)
+        module.load_state_dict(sd, strict=True)
+
+    same_layout(PointNet(48, 24, 16, 8).encoder, synth.to_torch_state(synth.apf_encoder_state(48, 8, 12)))
+    for E in (64, 256):
+        same_layout(P3Embed(sample_ratio=1 / 16, k=8, embed_dim=E), synth.to_torch_state(synth.p3embed_state(3, 1 / 16, 4, 4, E, 21)))
+    vit = synth.to_torch_state(synth.apf_vit_state(64, 2, 15, 51))
+    for p, m in (("blocks.0.", APFViTLayer(64, 2)), ("blocks.1.", APFViTLayer(64, 2)), ("head.", ClassificationHead(64, 15))):
+        same_layout(m, {k[len(p):]: v for k, v in vit.items() if k.startswith(p)})
+
+
 def test_no_cpu_fallback():
     from p3tok import functional as F
     x = torch.zeros(1, 16, 3)

@@ -296,3 +296,60 @@ def test_pointvit_block_oracle_matches_golden(golden_dir, name):
     ox, og = oracle.pointvit_blocks(sd, feats, pos, c["depth"], c["heads"])
     assert np.abs(ox - g["feats"]).max() <= 2e-5 * np.abs(g["feats"]).max()
     assert np.abs(og - g["glob"]).max() <= 2e-5 * np.abs(g["glob"]).max()
+
+
+@pytest.mark.parametrize("name", list(cases.INDEX_CASES))
+def test_port_index_ops_match_golden(golden_dir, name):
+    """oracle/port.py's FPS (both update forms) and kNN (both distance forms) against the reference's stored picks; the
+    port's expanded squared distance equals the oracle's arithmetic spec."""
+    import torch
+    from oracle import port
+    c = cases.INDEX_CASES[name]
+    g = _load(golden_dir, name)
+    x = synth.make_cloud(c["kind"], c["B"], c["N"], c["seed"], 3)
+    st = torch.from_numpy(synth.start_indices(c["B"], c["N"], c["seed"]))
+    xt = torch.from_numpy(x)
+    f = torch.from_numpy(g["fps_idx"].astype(np.int64))
+    assert torch.equal(port.fps_indices(xt, c["G"], st), f)
+    assert torch.equal(port.fps_indices(xt, c["G"], st, masked_update=True), f)
+    ctr = port.take(xt, f)
+    d_sq = oracle.pair_dist(x, ctr.numpy(), oracle.KNN_APF_SQ)
+    assert np.array_equal(d_sq, port.sq_dist_expanded(ctr, xt).numpy())
+    ok, msg = oracle.knn_tie_equivalent(port.knn_apf(c["k"], xt, ctr).numpy(), g["knn_apf"].astype(np.int64), d_sq, ulp=0)
+    assert ok, msg
+    d_cd = oracle.pair_dist(x, ctr.numpy(), oracle.KNN_P4P_CDIST)
+    ok, msg = oracle.knn_tie_equivalent(port.knn_p4p(c["k"], xt, ctr).numpy().astype(np.int64),
+                                        g["knn_p4p"].astype(np.int64), d_cd, ulp=1)
+    assert ok, msg
+
+
+@pytest.mark.parametrize("D", cases.FPS_ND_CASES["fps_nd"]["dims"])
+def test_port_fps_nd_matches_golden(golden_dir, D):
+    """oracle/port.py's farthest_point_sampling loop on D-dimensional points against the reference's stored picks."""
+    import torch
+    from oracle import port
+    c = cases.FPS_ND_CASES["fps_nd"]
+    pts = synth.make_points_nd(c["B"], c["N"], D, c["seed"])
+    st = synth.start_indices(c["B"], c["N"], c["seed"])
+    with torch.no_grad():
+        r = port.fps_indices(torch.from_numpy(pts), c["G"], torch.from_numpy(st), masked_update=True)
+    assert np.array_equal(r.numpy(), _load(golden_dir, "fps_nd")[f"idx_D{D}"])
+
+
+@pytest.mark.parametrize("name", ["p4p_2stage", "p4p_2stage_k32"])
+def test_p3embed_port_matches_golden(golden_dir, name):
+    """oracle/port.py's two-stage P3Embed against the reference's stored centres and tokens (both stages chained)."""
+    import torch
+    from oracle import port
+    c = cases.P4P_CASES[name]
+    g = _load(golden_dir, name)
+    B, N = c["B"], c["N"]
+    x = torch.from_numpy(synth.make_cloud(c["kind"], B, N, c["seed"], 3))
+    sd = synth.to_torch_state(synth.p3embed_state(3, c["sample_ratio"], 4, 4, c["embed_dim"], c["seed"]))
+    st = [torch.from_numpy(synth.start_indices(B, N, c["seed"], 0)), torch.from_numpy(synth.start_indices(B, N // 4, c["seed"], 1))]
+    with torch.no_grad():
+        pp, pf = port.p3embed(sd, x, x.transpose(1, 2).contiguous(), c["k"], 2, st)
+    for s in range(2):
+        assert np.array_equal(pp[s + 1].numpy(), g[f"centres{s}"])
+        ref = g[f"tokens{s}"]
+        assert np.abs(pf[s + 1].transpose(1, 2).numpy() - ref).max() <= 1e-6 * np.abs(ref).max()

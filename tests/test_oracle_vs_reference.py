@@ -1,5 +1,6 @@
-"""Build-container only: the port and the oracle against the live reference on fresh random
-shapes (skipped where /root/reference is absent, e.g. the GPU box)."""
+"""The port and the oracle against the live reference on fresh random shapes (skipped where no checkout of the
+original project is present, see oracle/ref_loader.py; tests/test_oracle_vs_golden.py compares both with the
+reference's stored outputs everywhere)."""
 import numpy as np
 import pytest
 import torch
