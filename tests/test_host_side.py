@@ -45,6 +45,64 @@ def test_host_only_size_queries(built):
     assert ws(7, 20011) - ws(6, 20011) == ws(3, 20011) - ws(2, 20011)   # linear in the number of clouds
 
 
+def test_patch_embed_workspace_is_bounded_by_one_chunk(built):
+    """The patch embedding is chunked so any B fits (DESIGN.md §3): p3tok_patch_embed_workspace_bytes (a host computation)
+    never exceeds the workspace of one full chunk, whatever the number of groups.  bf16 / fp32tc chunks hold at most
+    cg_max = ceil8(rows_target / k) groups: chunks are sized equally and rounded up to 8 groups, so the size dips and rises
+    with n and its maximum is reached at n = 2 * (rows_target // k) (two chunks of cg_max groups); fp32 chunks hold 8192.
+    The Python mirror of the policy (tests/test_gpu_chunking.py, which picks the sentinel clouds of the GPU tests) must
+    predict the size: ws(n) == ws(mirror(n)) where mirror(n) is one chunk."""
+    import random
+    from test_gpu_chunking import F32_CHUNK_GROUPS, chunk_size, chunk_wmax, rows_target
+    if os.environ.get("P3TOK_CHUNK_ROWS"):
+        pytest.skip("P3TOK_CHUNK_ROWS overrides the default chunk policy")
+    L = _lib.lib()
+
+    def mlp(meta):
+        m = _lib.MlpStruct()
+        n = meta[1]
+        m.cin, m.n_pre = meta[0], n
+        for i in range(n):
+            m.pre_dim[i], m.pre_relu[i] = meta[2 + i], meta[2 + n + i]
+        m.mid_dim, m.out_dim, m.out_relu = meta[2 + 2 * n:5 + 2 * n]
+        return m
+
+    layouts = {"APF E=384": [6, 3, 256, 512, 384, 1, 1, 0, 768, 384, 0],
+               "P3Embed stage 0": [6, 1, 128, 1, 256, 128, 1], "P3Embed stage 1": [131, 1, 256, 1, 512, 256, 1]}
+    precs = {"bf16": _lib.BF16, "fp32tc": _lib.BF16X3, "fp32": _lib.F32}
+    rnd = random.Random(2026)
+    full_sizes = {}
+    for lname, meta in layouts.items():
+        m = mlp(meta)
+        for pname, prec in precs.items():
+            for k in (1, 5, 24, 32, 64, 128):
+                ws = lambda n: int(L.p3tok_patch_embed_workspace_bytes(ctypes.byref(m), n, k, prec))
+                if pname == "fp32":
+                    cg0 = cg_max = F32_CHUNK_GROUPS
+                else:
+                    cg0 = rows_target(chunk_wmax(meta, pname)) // k
+                    cg_max = (cg0 + 7) // 8 * 8
+                what = f"{lname} {pname} k={k}"
+                n_full = cg0 if pname == "fp32" else 2 * cg0
+                assert chunk_size(n_full, k, meta, pname) == cg_max, what
+                full = ws(n_full)
+                full_sizes[(lname, pname, k)] = full
+                assert ws(cg0) <= full and ws(1) <= full, what
+                # around every change of the chunk count (n = c * cg0 + d) and at random n up to 2^26 groups
+                ns = [c * cg0 + d for c in range(1, 64) for d in range(-9, 10)] + [rnd.randint(1, 1 << 26) for _ in range(300)]
+                worst = max(ws(n) for n in ns if 0 < n <= 1 << 26)
+                assert worst == full, (what, worst, full)          # never above one full chunk, and reached
+                if pname == "fp32":
+                    assert ws(1 << 26) == full and ws(F32_CHUNK_GROUPS + 1) == full, what
+                elif k in (32, 64):                   # rows_target / k is a multiple of 8: mirror(n) is itself one chunk
+                    for n in ns[-200:]:
+                        assert ws(n) == ws(chunk_size(n, k, meta, pname)), f"{what}: n={n}"
+    gb = lambda key: full_sizes[key] / 1e9
+    assert 3.3 < gb(("APF E=384", "bf16", 32)) < 3.5 and 8.8 < gb(("APF E=384", "bf16", 1)) < 9.0
+    assert 8.2 < gb(("APF E=384", "fp32tc", 32)) < 8.4 and 1.6 < gb(("APF E=384", "fp32", 32)) < 1.7
+    assert max(full_sizes.values()) < 16e9                  # fits beside the model on one 180 GB device, any B
+
+
 def test_apf_fold_moves_the_feature_bias_into_the_concat_layer():
     """fold_apf_encoder (p3tok/fold.py): first_conv.6's bias is folded through the max and the concat into second_conv.0 -
     the folded feature layer carries a zero bias and the folded network still equals the oracle (checked above); here: the
