@@ -33,13 +33,14 @@ struct TcExtra {
   float res_mul = 1.f, out_scale = 1.f;
   int64_t ldc = 0;                 // row pitch of out_bf16 in elements (0 = N)
   int x3 = 0;                      // bf16x3 split operands: A [M, 2Kp] = [hi | lo], W [N, 3Kp] = [W_hi | W_hi | W_lo], K = 3Kp
-  int out_split = 0;               // out_bf16 is [M, 2N] = [hi | lo] of the fp32 result
+  int out_split = 0;               // out_bf16 is [M, 2N] = [hi | lo] of the fp32 result ...
+  int split_n = 0;                 // ... or a column slice of a [M, 2 split_n] split matrix: lo at column split_n + c (0 = N)
 };
 int tc_linear_ex(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat16* W, int N, const float* bias, int relu,
                  const TcExtra& ex, __nv_bfloat16* out_bf16, float* out_f32, cudaStream_t s);
 
 // vit.cu
-int64_t apf_vit_workspace(int64_t B, int64_t G, int64_t D, int64_t H, int64_t R);
+int64_t apf_vit_workspace(int64_t B, int64_t G, int64_t D, int64_t H, int64_t R, bool x3);
 
 static inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
 

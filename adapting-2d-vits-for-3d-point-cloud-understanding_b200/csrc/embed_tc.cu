@@ -108,6 +108,7 @@ struct TcParams {
   int x3;                  // bf16x3 split mode (fp32-accurate on the tensor cores): A is [M, 2 Kp] = [hi | lo], W is [N, 3 Kp] =
                            // [W_hi | W_hi | W_lo], K = 3 Kp: k-blocks of the third segment re-read the hi half of A
   int out_split;           // out_bf16 is [M, 2 N] = [hi | lo] of the fp32 result (the next layer's split operand)
+  int split_lo;            // out_split: column of the lo half relative to hi (N, or the full width when out_bf16 is a column slice)
   int prefetch;            // L2-prefetch the next item's activation tile
   int ares;                // A-resident mode (pairs only): a pair walks ALL N tiles of its M group, the group's activation
                            // rows stay in shared memory and only weight boxes stream through the ring
@@ -605,10 +606,10 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                              reinterpret_cast<uint64_t>(&tmC)),
                          "r"(sbox), "r"(n0), "r"(row0)
                          : "memory");
-            if (split)      // the lo half of the split output: columns [N, 2N) of the same row-major matrix
+            if (split)      // the lo half of the split output: split_lo columns right of the hi half, same rows
               asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
                                reinterpret_cast<uint64_t>(&tmC)),
-                           "r"(sbox + (uint32_t)TC_STAGING), "r"(p.N + n0), "r"(row0)
+                           "r"(sbox + (uint32_t)TC_STAGING), "r"(p.split_lo + n0), "r"(row0)
                            : "memory");
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
           }
@@ -705,7 +706,9 @@ static int tc_linear(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat
   p.out_split = ex ? ex->out_split : 0;
   if (p.x3) P3_REQUIRE(K % (3 * TC_BK) == 0, P3TOK_ERR_UNSUPPORTED, "tc_linear(x3): K=%d must be 3 x a multiple of 64", K);
   if (p.out_split) P3_REQUIRE(out_bf16 && N % 64 == 0 && !(ex && ex->epi16), P3TOK_ERR_UNSUPPORTED, "tc_linear(split): N=%d must be a multiple of 64", N);
-  const int64_t ldc = p.out_split ? 2 * (int64_t)N : ((ex && ex->ldc > 0) ? ex->ldc : N);   // row pitch of out_bf16
+  p.split_lo = (p.out_split && ex->split_n > 0) ? ex->split_n : N;
+  P3_REQUIRE(p.split_lo >= N && p.split_lo % 8 == 0, P3TOK_ERR_UNSUPPORTED, "tc_linear(split): split width %d < N=%d", p.split_lo, N);
+  const int64_t ldc = p.out_split ? 2 * (int64_t)p.split_lo : ((ex && ex->ldc > 0) ? ex->ldc : N);   // row pitch of out_bf16
   P3_REQUIRE(ldc == N || (out_bf16 && (!out_f32 || p.out_split) && ldc % 8 == 0), P3TOK_ERR_UNSUPPORTED, "tc_linear: ldc only for bf16 outputs");
   // 16 epilogue warps (lean epilogue: bf16 or TMA-stored / TMA-added fp32 outputs only), asked for by the ViT blocks
   static int epi16_on = -1;
@@ -721,7 +724,7 @@ static int tc_linear(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat
   p.f32_tma = 0;
   p.res_add = 0;
   if (out_bf16) {
-    rc = make_map(&tc, out_bf16, M, p.out_split ? 2 * N : N, 32, ldc);     // store boxes: 64 columns x 32 rows
+    rc = make_map(&tc, out_bf16, M, p.out_split ? p.split_lo + N : N, 32, ldc);     // store boxes: 64 columns x 32 rows
     if (rc) return rc;
   } else if (out_f32 && (TcCfg<TC_EPI_WARPS>::BOXES == 2 || want16) && N % 4 == 0 && (reinterpret_cast<uintptr_t>(out_f32) & 15) == 0) {
     rc = make_map_f32(&tc, out_f32, M, N, 32);  // fp32 store boxes: 32 columns x 32 rows

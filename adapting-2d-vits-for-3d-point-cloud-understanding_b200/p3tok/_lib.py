@@ -98,6 +98,13 @@ _SIGNATURES = {
                                  _i64, _vp, _i64, _vp]),
     "p3tok_layernorm_bf16": (_int, [_vp, _i64, _i64, _f32, _vp, _vp, _vp, _vp]),
     "p3tok_attention_bf16": (_int, [_vp, _i64, _i64, _i64, _i64, _vp, _vp]),
+    "p3tok_vit_x3_workspace_bytes": (_i64, [_i64, _i64, _i64, _i64, _i64]),
+    "p3tok_apf_vit_forward_x3": (_int, [_vp, _i64, _i64, _i64, _i64, _i64, _i64, ctypes.POINTER(VitLayerStruct), _i64, _vp, _vp,
+                                        _f32, _vp, _vp, _i64, _vp]),
+    "p3tok_vit_forward_x3": (_int, [_vp, _i64, _i64, _i64, _i64, _i64, ctypes.POINTER(VitLayerStruct), _i64, _vp, _vp, _vp, _f32, _vp,
+                                    _vp, _i64, _vp, _i64, _vp]),
+    "p3tok_layernorm_split": (_int, [_vp, _i64, _i64, _f32, _vp, _vp, _vp, _vp]),
+    "p3tok_attention_x3": (_int, [_vp, _i64, _i64, _i64, _i64, _vp, _vp]),
     "p3tok_linear_bf16_ex": (_int, [_vp, _i64, _i64, _vp, _i64, _vp, _int, _i64, _vp, _f32, _f32, _vp, _vp, _vp]),
 }
 

@@ -7,7 +7,8 @@ Same constructor arguments, attribute names and state_dict keys (`blocks.{i}.nor
 `.adapter.down_proj`, `encoder_norm`, `point_encoder.encoder.first_conv.0`, `head.mlp_head.0`, ...), so a reference
 checkpoint loads with strict=True.  The torch submodules are parameter containers.  Serving (eval mode, no gradient
 wanted): forward runs `p3tok::apf_vit` - LayerNorm -> tcgen05 GEMMs with GELU / residual epilogues -> attention, fp32
-residual stream, the head's BatchNorms folded.  Training (`.train()`, or a gradient is wanted through eval-mode blocks):
+residual stream, the head's BatchNorms folded - or, with block_precision="fp32tc", `p3tok::apf_vit_x3`, the same kernels on
+bf16x3 split operands (fp32-accurate).  Training (`.train()`, or a gradient is wanted through eval-mode blocks):
 the fp32 autograd path of p3tok/train_vit.py - dropout / DropPath as keep masks, BatchNorm batch statistics, gradients
 for the tokens and for every parameter that requires one (the reference keeps point_encoder / encoder_norm / head
 trainable, apf.py:335-346).  Differences from the reference constructor: no timm / no network here, so
@@ -16,12 +17,12 @@ trainable, apf.py:335-346).  Differences from the reference constructor: no timm
 from __future__ import annotations
 
 import math
-from typing import List, Optional
+from typing import List, Optional, Tuple
 
 import torch
 from torch import nn
 
-from . import ops
+from . import fold, ops
 from .modules import PointNet
 
 
@@ -80,9 +81,9 @@ class APFViTLayer(nn.Module):
         return run_blocks([self], x, None)[0]
 
 
-def fold_vit_layer(layer: "APFViTLayer") -> List[torch.Tensor]:
-    """One APFViTLayer folded into the four GEMMs of struct p3tok_vit_layer (include/p3tok.h), float64 algebra, then bf16
-    matrices / f32 biases in ops.VIT_LAYER_TENSORS order:
+def fold_vit_layer64(layer: "APFViTLayer") -> List[Tuple[torch.Tensor, torch.Tensor]]:
+    """One APFViTLayer folded into the four GEMMs of struct p3tok_vit_layer (include/p3tok.h) in float64: (matrix, bias) for
+    qkv, proj, fc1d, fc2u:
       LayerNorm affines move into the weights that consume the normalised rows (W diag(g), b + W beta);
       norm2 and adapter_norm share their statistics, so [fc1 ; down_proj] is one GEMM on one normalised matrix;
       [fc2 | scale * up_proj] consumes [gelu(fc1) | relu(down)] whole (apf_utils.py:217-233, 284-292)."""
@@ -96,25 +97,65 @@ def fold_vit_layer(layer: "APFViTLayer") -> List[torch.Tensor]:
     dw, db = d(layer.adapter.down_proj.weight), d(layer.adapter.down_proj.bias)
     f2w, f2b = d(layer.mlp.fc2.weight), d(layer.mlp.fc2.bias)
     uw, ub = d(layer.adapter.up_proj.weight), d(layer.adapter.up_proj.bias)
-    mats = [
+    return [
         (qw * g1[None, :], qb + qw @ b1),
         (d(layer.attention.proj.weight), d(layer.attention.proj.bias)),
         (torch.cat([f1w * g2[None, :], dw * ga[None, :]], 0), torch.cat([f1b + f1w @ b2, db + dw @ ba], 0)),
         (torch.cat([f2w, sc * uw], 1), f2b + sc * ub),
     ]
+
+
+def bf16_layer(mats) -> List[torch.Tensor]:
+    """float64 (matrix, bias) pairs -> bf16 matrices / f32 biases in ops.VIT_LAYER_TENSORS order (the bf16 stack)."""
     out: List[torch.Tensor] = []
     for w, b in mats:
         out += [w.to(torch.bfloat16).contiguous(), b.float().contiguous()]
     return out
 
 
-def _layer_params(layer: "APFViTLayer", cache: dict) -> List[torch.Tensor]:
-    """fold_vit_layer, cached per parameter version (no host synchronisation on the steady-state path)."""
+def x3_layer(mats) -> List[torch.Tensor]:
+    """float64 (matrix, bias) pairs -> the x3 form of the fp32-accurate stack (include/p3tok.h p3tok_apf_vit_forward_x3): every
+    matrix fold.split_x3 [W_hi | W_hi | W_lo] over its input padded to a multiple of 64, fc1d's rows and bias padded with zeros
+    to pad64(H + R) (so fc2u's reduction length matches), f32 biases, in ops.VIT_LAYER_TENSORS order."""
+    (qw, qb), (pw, pb), (f1w, f1b), (f2w, f2b) = mats
+    hrp = fold.pad64(f1w.shape[0])
+    f1bp = f1b.new_zeros(hrp)
+    f1bp[:f1b.shape[0]] = f1b
+    out: List[torch.Tensor] = []
+    for w, b, rows in ((qw, qb, None), (pw, pb, None), (f1w, f1bp, hrp), (f2w, f2b, None)):
+        out += [fold.split_x3(w, rows), b.float().contiguous()]
+    return out
+
+
+def fold_vit_layer(layer: "APFViTLayer") -> List[torch.Tensor]:
+    """fold_vit_layer64 as bf16 matrices / f32 biases in ops.VIT_LAYER_TENSORS order (the bf16 stack, ops.apf_vit)."""
+    return bf16_layer(fold_vit_layer64(layer))
+
+
+def fold_vit_layer_x3(layer: "APFViTLayer") -> List[torch.Tensor]:
+    """fold_vit_layer64 in the x3 form of the fp32-accurate stack (ops.apf_vit_x3)."""
+    return x3_layer(fold_vit_layer64(layer))
+
+
+BLOCK_PRECISIONS = ("bf16", "fp32tc")
+
+
+def check_block_precision(p: str) -> bool:
+    """True for the fp32-accurate block stack ("fp32tc": bf16x3 on the tensor cores), False for "bf16"."""
+    if p not in BLOCK_PRECISIONS:
+        raise ValueError(f"block_precision must be 'bf16' or 'fp32tc', got {p!r}")
+    return p == "fp32tc"
+
+
+def _layer_params(layer: "APFViTLayer", cache: dict, precision: str = "bf16") -> List[torch.Tensor]:
+    """fold_vit_layer (fold_vit_layer_x3 for "fp32tc"), cached per parameter version and precision (no host synchronisation
+    on the steady-state path)."""
     ver = tuple((t._version, t.data_ptr()) for t in layer.parameters())
-    hit = cache.get(id(layer))
+    key = (id(layer), precision)
+    hit = cache.get(key)
     if hit is None or hit[0] != ver:
-        hit = (ver, fold_vit_layer(layer))
-        cache[id(layer)] = hit
+        hit = (ver, fold_vit_layer_x3(layer) if precision == "fp32tc" else fold_vit_layer(layer))
+        cache[key] = hit
     return hit[1]
 
 
@@ -127,8 +168,12 @@ def _wants_autograd(layers, x: torch.Tensor, final_norm: Optional[nn.LayerNorm])
     return torch.is_grad_enabled() and x.requires_grad
 
 
-def run_blocks(layers, x: torch.Tensor, final_norm: Optional[nn.LayerNorm], cache: Optional[dict] = None):
-    """(x after the last layer, pooled = max over tokens of final_norm(x) or None)."""
+def run_blocks(layers, x: torch.Tensor, final_norm: Optional[nn.LayerNorm], cache: Optional[dict] = None,
+               precision: str = "bf16"):
+    """(x after the last layer, pooled = max over tokens of final_norm(x) or None).  precision: "bf16" (ops.apf_vit, rtol 1e-2)
+    or "fp32tc" (ops.apf_vit_x3: the same kernels on bf16x3 split operands, rtol 1e-4); train mode and gradient-wanted calls
+    take the fp32 autograd path whatever it says."""
+    x3 = check_block_precision(precision)
     layers = list(layers)
     if _wants_autograd(layers, x, final_norm):
         from . import train_vit
@@ -136,7 +181,7 @@ def run_blocks(layers, x: torch.Tensor, final_norm: Optional[nn.LayerNorm], cach
     cache = {} if cache is None else cache
     params: List[torch.Tensor] = []
     for l in layers:
-        params += _layer_params(l, cache)
+        params += _layer_params(l, cache, precision)
     heads = layers[0].attention.num_heads
     D = x.shape[-1]
     # one eps for every normalisation of the stack (norm2 and adapter_norm share their statistics in the folded layer)
@@ -149,7 +194,7 @@ def run_blocks(layers, x: torch.Tensor, final_norm: Optional[nn.LayerNorm], cach
         fw, fb = torch.ones(D, device=x.device), torch.zeros(D, device=x.device)
     else:
         fw, fb = final_norm.weight.detach().float(), final_norm.bias.detach().float()
-    y, pooled = ops.apf_vit(x.float(), params, heads, layers[0].adapter.down_size, fw, fb, ln_eps)
+    y, pooled = (ops.apf_vit_x3 if x3 else ops.apf_vit)(x.float(), params, heads, layers[0].adapter.down_size, fw, fb, ln_eps)
     return y, (pooled if final_norm is not None else None)
 
 
@@ -186,13 +231,17 @@ class ClassificationHead(nn.Module):
 
 class AdaptPointFormer(nn.Module):
     """apf.py:254-373.  forward(x (B,N,C)) -> (B,num_classes) logits: PointNet tokenizer -> 12 APFViTLayers ->
-    encoder_norm -> max over tokens -> classification head.  `precision` selects the tokenizer's embed path; the block
-    stack always runs bf16 GEMMs on tcgen05 with an fp32 residual stream."""
+    encoder_norm -> max over tokens -> classification head.  `precision` selects the tokenizer's embed path,
+    `block_precision` the block stack's: "bf16" (default) runs bf16 GEMMs on tcgen05 with an fp32 residual stream (rtol
+    1e-2), "fp32tc" the same kernels on bf16x3 split operands (rtol 1e-4, the fp32 contract; about 3x the tensor work)."""
 
     def __init__(self, num_classes: int = 15, embedding_dim: int = 768, vit_name: str = "vit_base_patch16_224",
                  pretrained: bool = False, npoint: int = 196, nsample: int = 32, in_channels: int = 3,
-                 dropout_rate: float = 0.1, dropout_path_rate: float = 0.1, precision: str = "bf16"):
+                 dropout_rate: float = 0.1, dropout_path_rate: float = 0.1, precision: str = "bf16",
+                 block_precision: str = "bf16"):
         super().__init__()
+        check_block_precision(block_precision)
+        self.block_precision = block_precision
         if pretrained:
             raise RuntimeError("AdaptPointFormer: no timm / network in this build - construct with pretrained=False and "
                                "load_state_dict() a reference checkpoint (keys are identical)")
@@ -210,7 +259,7 @@ class AdaptPointFormer(nn.Module):
         """(B,D) pooled features: everything before the classification head (apf.py:358-366)."""
         tok = self.point_encoder(x, start_idx)
         cache = self.__dict__.setdefault("_vit_cache", {})
-        return run_blocks(self.blocks, tok, self.encoder_norm, cache)[1]
+        return run_blocks(self.blocks, tok, self.encoder_norm, cache, self.block_precision)[1]
 
     def _freeze(self) -> None:
         """apf.py:335-346 verbatim in effect: everything frozen except parameters whose name contains 'adaptmlp', 'head',

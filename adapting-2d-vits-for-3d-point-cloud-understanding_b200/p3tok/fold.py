@@ -58,13 +58,7 @@ class PatchMLP:
         key = (str(device), "x3")
         if key not in self._cast:
             def x3(w):
-                w = w.detach().float().cpu()
-                kp = (w.shape[1] + 63) // 64 * 64
-                wp = torch.zeros(w.shape[0], kp)
-                wp[:, :w.shape[1]] = w
-                hi = wp.bfloat16()
-                lo = (wp - hi.float()).bfloat16()
-                return torch.cat([hi, hi, lo], 1).contiguous().to(device)
+                return split_x3(w.cpu()).to(device)
 
             def b(t):
                 return t.to(device=device, dtype=torch.float32).contiguous()
@@ -88,6 +82,24 @@ class PatchMLP:
                 [m(w) for w in self.w_pre], [b(x) for x in self.b_pre], m(self.w_mid_g), m(self.w_mid_f),
                 b(self.b_mid), m(self.w_out), b(self.b_out))
         return self._cast[key]
+
+
+def pad64(n: int) -> int:
+    return (n + 63) // 64 * 64
+
+
+def split_x3(w: torch.Tensor, rows: Optional[int] = None) -> torch.Tensor:
+    """The weight operand of a bf16x3 (fp32-accurate tensor-core) GEMM: W [out, in] -> bfloat16 [rows, 3 * pad64(in)] =
+    [W_hi | W_hi | W_lo] with W_hi = bf16(W), W_lo = bf16(W - W_hi), both taken from W in float64 and zero padded to
+    pad64(in) columns and `rows` (default out) rows, on W's device.  Against activations stored as [hi | lo] one GEMM over
+    the tripled reduction length evaluates a_hi.w_hi + a_lo.w_hi + a_hi.w_lo (csrc/embed_tc.cu tc_linear x3)."""
+    w = w.detach().double()
+    n, k = w.shape
+    wp = w.new_zeros((n if rows is None else rows, pad64(k)))
+    wp[:n, :k] = w
+    hi = wp.bfloat16()
+    lo = (wp - hi.double()).bfloat16()
+    return torch.cat([hi, hi, lo], 1).contiguous()
 
 
 def _mat(sd, name) -> torch.Tensor:

@@ -674,53 +674,115 @@ VIT_LAYER_TENSORS = ("qkv_w", "qkv_b", "proj_w", "proj_b", "fc1d_w", "fc1d_b", "
 _NVT = len(VIT_LAYER_TENSORS)
 
 
+def vit_layer_shapes(D: int, HR: int, x3: bool) -> dict:
+    """Shapes of one p3tok_vit_layer's tensors (include/p3tok.h) for token width D and fc1d width HR (= H + R; x3: the padded
+    width pad64(H + R)): the bf16 layout, or the x3 layout in which every matrix W [out, in] is [W_hi | W_hi | W_lo] over
+    pad64(in) columns (fold.split_x3)."""
+    k = (lambda n: 3 * ((n + 63) // 64 * 64)) if x3 else (lambda n: n)
+    return dict(qkv_w=(3 * D, k(D)), qkv_b=(3 * D,), proj_w=(D, k(D)), proj_b=(D,), fc1d_w=(HR, k(D)), fc1d_b=(HR,),
+                fc2u_w=(D, k(HR)), fc2u_b=(D,))
+
+
+def _vit_layers(name: str, params: Sequence[torch.Tensor], D: int, R: int, x3: bool):
+    """Validate the folded layers against the token width and fill the host array of p3tok_vit_layer descriptors.
+    Returns (descriptors, layer count, H, tensors to keep alive during the call)."""
+    if len(params) % _NVT:
+        raise RuntimeError(f"p3tok::{name}: expected {_NVT} tensors per layer")
+    nl = len(params) // _NVT
+    keep = []
+    layers = (_lib.VitLayerStruct * max(nl, 1))()
+    H = 64
+    for li in range(nl):
+        for j, tname in enumerate(VIT_LAYER_TENSORS):
+            t = params[li * _NVT + j]
+            want = torch.bfloat16 if tname.endswith("_w") else torch.float32
+            if t.dtype != want:
+                raise RuntimeError(f"p3tok::{name}: layer {li} {tname} must be {want}, got {t.dtype}")
+            t = t.contiguous()
+            keep.append(t)
+            setattr(layers[li], tname, t.data_ptr())
+        HR = int(params[li * _NVT + 4].shape[0])
+        want = vit_layer_shapes(D, HR, x3)
+        if any(tuple(params[li * _NVT + j].shape) != want[n] for j, n in enumerate(VIT_LAYER_TENSORS) if n.endswith("_w")):
+            raise RuntimeError(f"p3tok::{name}: weight shapes do not match the token width")
+        if any(params[li * _NVT + j].numel() != want[n][0] for j, n in enumerate(VIT_LAYER_TENSORS) if n.endswith("_b")):
+            raise RuntimeError(f"p3tok::{name}: bias length does not match its matrix")
+        if x3 and (HR % 64 or HR <= R):
+            raise RuntimeError(f"p3tok::{name}: fc1d has {HR} rows, expected pad64(H + R)")
+        H = (HR - R) // 64 * 64 if x3 else HR - R   # x3: H is a multiple of 64 and H + R <= HR < H + R + 64
+    return layers, nl, H, keep
+
+
+def _apf_vit(name: str, x3: bool, tokens, params, heads, bottleneck, final_w, final_b, ln_eps):
+    _need_cuda(name, tokens, final_w, final_b, *params)
+    x = _f32c(name, tokens).clone()                        # the residual stream is updated in place
+    B, G, D = (int(v) for v in x.shape)
+    fw, fb = _f32c(name, final_w), _f32c(name, final_b)
+    R = int(bottleneck)
+    layers, nl, H, keep = _vit_layers(name, params, D, R, x3)
+    pooled = torch.empty((B, D), dtype=torch.float32, device=x.device)
+    L = _L()
+    ws_bytes, forward = ((L.p3tok_vit_x3_workspace_bytes, L.p3tok_apf_vit_forward_x3) if x3
+                         else (L.p3tok_apf_vit_workspace_bytes, L.p3tok_apf_vit_forward))
+    with torch.cuda.device(x.device):
+        nbytes = int(ws_bytes(B, G, D, H, R))
+        ws = torch.empty((max(nbytes, 1024),), dtype=torch.uint8, device=x.device)
+        with _timed(name):
+            check(forward(x.data_ptr(), B, G, D, int(heads), H, R, layers, nl, fw.data_ptr(), fb.data_ptr(), float(ln_eps),
+                          pooled.data_ptr(), ws.data_ptr(), nbytes, _stream()), name)
+    del keep
+    return x, pooled
+
+
 @torch.library.custom_op("p3tok::apf_vit", mutates_args=(), device_types="cuda")
 def apf_vit(tokens: torch.Tensor, params: Sequence[torch.Tensor], heads: int, bottleneck: int, final_w: torch.Tensor,
             final_b: torch.Tensor, ln_eps: float = 1e-5) -> Tuple[torch.Tensor, torch.Tensor]:
     """tokens (B,G,D) f32 -> (x (B,G,D) f32 after the last block, pooled (B,D) f32 = max_G encoder_norm(x)).
     params: 8 tensors per layer in VIT_LAYER_TENSORS order - the layer as folded by apf_model.fold_vit_layer
     (matrices bf16 [out,in], biases f32)."""
-    if len(params) % _NVT:
-        raise RuntimeError(f"p3tok::apf_vit: expected {_NVT} tensors per layer")
-    nl = len(params) // _NVT
-    _need_cuda("apf_vit", tokens, final_w, final_b, *params)
-    x = _f32c("apf_vit", tokens).clone()                  # the residual stream is updated in place
-    B, G, D = (int(v) for v in x.shape)
-    fw, fb = _f32c("apf_vit", final_w), _f32c("apf_vit", final_b)
-    keep = []
-    layers = (_lib.VitLayerStruct * max(nl, 1))()
-    R = int(bottleneck)
-    H = 64
-    for li in range(nl):
-        for j, name in enumerate(VIT_LAYER_TENSORS):
-            t = params[li * _NVT + j]
-            want = torch.bfloat16 if name.endswith("_w") else torch.float32
-            if t.dtype != want:
-                raise RuntimeError(f"p3tok::apf_vit: layer {li} {name} must be {want}, got {t.dtype}")
-            t = t.contiguous()
-            keep.append(t)
-            setattr(layers[li], name, t.data_ptr())
-        qkv, proj, fc1d, fc2u = (params[li * _NVT + j] for j in (0, 2, 4, 6))
-        HR = int(fc1d.shape[0])
-        if tuple(qkv.shape) != (3 * D, D) or tuple(proj.shape) != (D, D) or fc1d.shape[1] != D or tuple(fc2u.shape) != (D, HR):
-            raise RuntimeError("p3tok::apf_vit: weight shapes do not match the token width")
-        H = HR - R                                        # [fc1 ; down_proj]: the adapter bottleneck is the tail
-        for j in (1, 3, 5, 7):
-            if params[li * _NVT + j].numel() != params[li * _NVT + j - 1].shape[0]:
-                raise RuntimeError("p3tok::apf_vit: bias length does not match its matrix")
-    pooled = torch.empty((B, D), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        nbytes = int(_L().p3tok_apf_vit_workspace_bytes(B, G, D, H, R))
-        ws = torch.empty((max(nbytes, 1024),), dtype=torch.uint8, device=x.device)
-        with _timed("apf_vit"):
-            check(_L().p3tok_apf_vit_forward(x.data_ptr(), B, G, D, int(heads), H, R, layers, nl, fw.data_ptr(), fb.data_ptr(),
-                                             float(ln_eps), pooled.data_ptr(), ws.data_ptr(), nbytes, _stream()), "apf_vit")
-    return x, pooled
+    return _apf_vit("apf_vit", False, tokens, params, heads, bottleneck, final_w, final_b, ln_eps)
 
 
 @apf_vit.register_fake
 def _(tokens, params, heads, bottleneck, final_w, final_b, ln_eps=1e-5):
     return tokens.new_empty(tokens.shape), tokens.new_empty((tokens.shape[0], tokens.shape[2]))
+
+
+@torch.library.custom_op("p3tok::apf_vit_x3", mutates_args=(), device_types="cuda")
+def apf_vit_x3(tokens: torch.Tensor, params: Sequence[torch.Tensor], heads: int, bottleneck: int, final_w: torch.Tensor,
+               final_b: torch.Tensor, ln_eps: float = 1e-5) -> Tuple[torch.Tensor, torch.Tensor]:
+    """apf_vit, fp32-accurate (bf16x3 split operands on the same kernels, rtol 1e-4): params are the layers as folded by
+    apf_model.fold_vit_layer_x3 (vit_layer_shapes(D, pad64(H + R), True)); D must be a multiple of 64."""
+    return _apf_vit("apf_vit_x3", True, tokens, params, heads, bottleneck, final_w, final_b, ln_eps)
+
+
+@apf_vit_x3.register_fake
+def _(tokens, params, heads, bottleneck, final_w, final_b, ln_eps=1e-5):
+    return tokens.new_empty(tokens.shape), tokens.new_empty((tokens.shape[0], tokens.shape[2]))
+
+
+def _vit_blocks(name: str, x3: bool, feats, pos, params, heads, final_w, final_b, ln_eps, pool_skip):
+    _need_cuda(name, feats, pos, final_w, final_b, *params)
+    x = _f32c(name, feats).clone()
+    B, S, D = (int(v) for v in x.shape)
+    p = _f32c(name, pos) if pos is not None else None
+    if p is not None and tuple(p.shape) != (B, S, D):
+        raise RuntimeError(f"p3tok::{name}: pos must have the shape of feats")
+    fw, fb = _f32c(name, final_w), _f32c(name, final_b)
+    layers, nl, H, keep = _vit_layers(name, params, D, 0, x3)
+    out = torch.empty((B, S, D), dtype=torch.float32, device=x.device)
+    pooled = torch.empty((B, D), dtype=torch.float32, device=x.device)
+    L = _L()
+    ws_bytes, forward = ((L.p3tok_vit_x3_workspace_bytes, L.p3tok_vit_forward_x3) if x3
+                         else (L.p3tok_apf_vit_workspace_bytes, L.p3tok_vit_forward))
+    with torch.cuda.device(x.device):
+        nbytes = int(ws_bytes(B, S, D, H, 0))
+        ws = torch.empty((max(nbytes, 1024),), dtype=torch.uint8, device=x.device)
+        with _timed(name):
+            check(forward(x.data_ptr(), B, S, D, int(heads), H, layers, nl, _ptr(p), fw.data_ptr(), fb.data_ptr(), float(ln_eps),
+                          out.data_ptr(), pooled.data_ptr(), int(pool_skip), ws.data_ptr(), nbytes, _stream()), name)
+    del keep
+    return out, pooled
 
 
 @torch.library.custom_op("p3tok::vit_blocks", mutates_args=(), device_types="cuda")
@@ -729,46 +791,23 @@ def vit_blocks(feats: torch.Tensor, pos: Optional[torch.Tensor], params: Sequenc
     """Plain pre-norm ViT blocks (timm `Block`, what Pix4Point runs): feats (B,S,D) f32 = [cls ; tokens], pos (B,S,D) or None
     re-added in front of every block -> (LayerNorm(x) (B,S,D) f32, max over rows >= pool_skip (B,D) f32).  params: 8 tensors
     per layer in VIT_LAYER_TENSORS order, folded by p4p_model.fold_timm_block (no adapter columns)."""
-    if len(params) % _NVT:
-        raise RuntimeError(f"p3tok::vit_blocks: expected {_NVT} tensors per layer")
-    nl = len(params) // _NVT
-    _need_cuda("vit_blocks", feats, pos, final_w, final_b, *params)
-    x = _f32c("vit_blocks", feats).clone()
-    B, S, D = (int(v) for v in x.shape)
-    p = _f32c("vit_blocks", pos) if pos is not None else None
-    if p is not None and tuple(p.shape) != (B, S, D):
-        raise RuntimeError("p3tok::vit_blocks: pos must have the shape of feats")
-    fw, fb = _f32c("vit_blocks", final_w), _f32c("vit_blocks", final_b)
-    keep = []
-    layers = (_lib.VitLayerStruct * max(nl, 1))()
-    H = 64
-    for li in range(nl):
-        for j, name in enumerate(VIT_LAYER_TENSORS):
-            t = params[li * _NVT + j]
-            want = torch.bfloat16 if name.endswith("_w") else torch.float32
-            if t.dtype != want:
-                raise RuntimeError(f"p3tok::vit_blocks: layer {li} {name} must be {want}, got {t.dtype}")
-            t = t.contiguous()
-            keep.append(t)
-            setattr(layers[li], name, t.data_ptr())
-        qkv, proj, fc1, fc2 = (params[li * _NVT + j] for j in (0, 2, 4, 6))
-        H = int(fc1.shape[0])
-        if tuple(qkv.shape) != (3 * D, D) or tuple(proj.shape) != (D, D) or fc1.shape[1] != D or tuple(fc2.shape) != (D, H):
-            raise RuntimeError("p3tok::vit_blocks: weight shapes do not match the token width")
-    out = torch.empty((B, S, D), dtype=torch.float32, device=x.device)
-    pooled = torch.empty((B, D), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        nbytes = int(_L().p3tok_apf_vit_workspace_bytes(B, S, D, H, 0))
-        ws = torch.empty((max(nbytes, 1024),), dtype=torch.uint8, device=x.device)
-        with _timed("vit_blocks"):
-            check(_L().p3tok_vit_forward(x.data_ptr(), B, S, D, int(heads), H, layers, nl, _ptr(p), fw.data_ptr(), fb.data_ptr(),
-                                         float(ln_eps), out.data_ptr(), pooled.data_ptr(), int(pool_skip), ws.data_ptr(), nbytes,
-                                         _stream()), "vit_blocks")
-    del keep
-    return out, pooled
+    return _vit_blocks("vit_blocks", False, feats, pos, params, heads, final_w, final_b, ln_eps, pool_skip)
 
 
 @vit_blocks.register_fake
+def _(feats, pos, params, heads, final_w, final_b, ln_eps, pool_skip):
+    return feats.new_empty(feats.shape), feats.new_empty((feats.shape[0], feats.shape[2]))
+
+
+@torch.library.custom_op("p3tok::vit_blocks_x3", mutates_args=(), device_types="cuda")
+def vit_blocks_x3(feats: torch.Tensor, pos: Optional[torch.Tensor], params: Sequence[torch.Tensor], heads: int,
+                  final_w: torch.Tensor, final_b: torch.Tensor, ln_eps: float, pool_skip: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """vit_blocks, fp32-accurate (bf16x3 split operands, rtol 1e-4): params folded by p4p_model.fold_timm_block_x3
+    (vit_layer_shapes(D, pad64(H), True)); D must be a multiple of 64."""
+    return _vit_blocks("vit_blocks_x3", True, feats, pos, params, heads, final_w, final_b, ln_eps, pool_skip)
+
+
+@vit_blocks_x3.register_fake
 def _(feats, pos, params, heads, final_w, final_b, ln_eps, pool_skip):
     return feats.new_empty(feats.shape), feats.new_empty((feats.shape[0], feats.shape[2]))
 
@@ -808,6 +847,47 @@ def attention_bf16(qkv: torch.Tensor, B: int, G: int, heads: int) -> torch.Tenso
 
 
 @attention_bf16.register_fake
+def _(qkv, B, G, heads):
+    return qkv.new_empty((qkv.shape[0], qkv.shape[1] // 3))
+
+
+@torch.library.custom_op("p3tok::layernorm_split", mutates_args=(), device_types="cuda")
+def layernorm_split(x: torch.Tensor, w: Optional[torch.Tensor], b: Optional[torch.Tensor], eps: float) -> torch.Tensor:
+    """LayerNorm(x) of x (M,D) f32 as the split operand of the x3 stack: (M, 2D) bf16 = [hi | lo], hi + lo = the fp32 value
+    to 16 mantissa bits."""
+    _need_cuda("layernorm_split", x, w, b)
+    x = _f32c("layernorm_split", x)
+    w = None if w is None else _f32c("layernorm_split", w)
+    b = None if b is None else _f32c("layernorm_split", b)
+    M, D = int(x.shape[0]), int(x.shape[1])
+    out = torch.empty((M, 2 * D), dtype=torch.bfloat16, device=x.device)
+    with torch.cuda.device(x.device), _timed("layernorm_split"):
+        check(_L().p3tok_layernorm_split(x.data_ptr(), M, D, float(eps), _ptr(w), _ptr(b), out.data_ptr(), _stream()),
+              "layernorm_split")
+    return out
+
+
+@layernorm_split.register_fake
+def _(x, w, b, eps):
+    return x.new_empty((x.shape[0], 2 * x.shape[1]), dtype=torch.bfloat16)
+
+
+@torch.library.custom_op("p3tok::attention_x3", mutates_args=(), device_types="cuda")
+def attention_x3(qkv: torch.Tensor, B: int, G: int, heads: int) -> torch.Tensor:
+    """qkv (B*G, 6D) bf16 = [hi | lo] of the qkv matrix of attention_bf16 -> [hi | lo] of softmax(q k^T / sqrt(hd)) v as
+    (B*G, 2D) bf16, fp32-accurate (bf16x3 products, fp32 softmax)."""
+    _need_cuda("attention_x3", qkv)
+    if qkv.dtype != torch.bfloat16 or qkv.dim() != 2 or qkv.shape[0] != B * G or qkv.shape[1] % 6:
+        raise RuntimeError("p3tok::attention_x3: expected (B*G, 6D) bf16")
+    qkv = qkv.contiguous()
+    D = int(qkv.shape[1]) // 6
+    out = torch.empty((B * G, 2 * D), dtype=torch.bfloat16, device=qkv.device)
+    with torch.cuda.device(qkv.device), _timed("attention_x3"):
+        check(_L().p3tok_attention_x3(qkv.data_ptr(), B, G, D, int(heads), out.data_ptr(), _stream()), "attention_x3")
+    return out
+
+
+@attention_x3.register_fake
 def _(qkv, B, G, heads):
     return qkv.new_empty((qkv.shape[0], qkv.shape[1] // 3))
 

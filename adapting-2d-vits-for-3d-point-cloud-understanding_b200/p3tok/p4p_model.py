@@ -6,7 +6,8 @@ The reference takes its blocks from `timm.create_model(...)` (pix4point.py:221-2
 parameter layout (`vit.blocks.{i}.norm1 / attn.qkv / attn.proj / norm2 / mlp.fc1 / mlp.fc2`, `vit.norm`, `vit.cls_token`,
 `vit.pos_embed`) - a PointViT checkpoint loads with strict=False (timm's own unused patch embedding / head are skipped).
 forward runs the sm_100a kernels (`p3tok::vit_blocks`: the APF block-stack kernels without the adapter columns, the
-positional add fused into each block's first normalisation pass) in eval mode; `.train()` - or a gradient wanted through
+positional add fused into each block's first normalisation pass; `p3tok::vit_blocks_x3` with block_precision="fp32tc") in
+eval mode; `.train()` - or a gradient wanted through
 eval-mode blocks - takes the fp32 autograd path of p3tok/train_vit.py (Pix4Point trains everything, or everything but `vit.*`
 with frozen=True, pix4point.py:229-233).
 """
@@ -18,6 +19,7 @@ import torch
 from torch import nn
 
 from . import ops
+from .apf_model import bf16_layer, check_block_precision, x3_layer
 from .modules import PointViTTokens
 
 
@@ -47,19 +49,25 @@ class TimmBlock(nn.Module):
         self.mlp = _Mlp(dim, int(dim * mlp_ratio))
 
 
-def fold_timm_block(blk: TimmBlock) -> List[torch.Tensor]:
-    """A block folded into the four GEMMs of struct p3tok_vit_layer (LayerNorm affines moved into the consuming weights),
-    float64 algebra, bf16 matrices / f32 biases in ops.VIT_LAYER_TENSORS order."""
+def fold_timm_block64(blk: TimmBlock) -> List[Tuple[torch.Tensor, torch.Tensor]]:
+    """A block folded into the four GEMMs of struct p3tok_vit_layer (LayerNorm affines moved into the consuming weights) in
+    float64: (matrix, bias) for qkv, proj, fc1, fc2."""
     d = lambda t: t.detach().double()
     g1, b1, g2, b2 = d(blk.norm1.weight), d(blk.norm1.bias), d(blk.norm2.weight), d(blk.norm2.bias)
     qw, qb = d(blk.attn.qkv.weight), d(blk.attn.qkv.bias)
     f1w, f1b = d(blk.mlp.fc1.weight), d(blk.mlp.fc1.bias)
-    mats = [(qw * g1[None, :], qb + qw @ b1), (d(blk.attn.proj.weight), d(blk.attn.proj.bias)),
+    return [(qw * g1[None, :], qb + qw @ b1), (d(blk.attn.proj.weight), d(blk.attn.proj.bias)),
             (f1w * g2[None, :], f1b + f1w @ b2), (d(blk.mlp.fc2.weight), d(blk.mlp.fc2.bias))]
-    out: List[torch.Tensor] = []
-    for w, b in mats:
-        out += [w.to(torch.bfloat16).contiguous(), b.float().contiguous()]
-    return out
+
+
+def fold_timm_block(blk: TimmBlock) -> List[torch.Tensor]:
+    """fold_timm_block64 as bf16 matrices / f32 biases in ops.VIT_LAYER_TENSORS order (ops.vit_blocks)."""
+    return bf16_layer(fold_timm_block64(blk))
+
+
+def fold_timm_block_x3(blk: TimmBlock) -> List[torch.Tensor]:
+    """fold_timm_block64 in the x3 form of the fp32-accurate stack (ops.vit_blocks_x3, apf_model.x3_layer)."""
+    return x3_layer(fold_timm_block64(blk))
 
 
 class _Vit(nn.Module):
@@ -75,12 +83,17 @@ class _Vit(nn.Module):
 
 class PointViT(nn.Module):
     """pix4point.py:194-271.  forward(p, x=None) -> (p_list, x_list, feats (B,1+G,E) after the final norm);
-    forward_cls_feat(p, x=None) -> (B, E * len(global_features)).  Defaults = vit_small_patch16_384 (E 384, depth 12, 6 heads)."""
+    forward_cls_feat(p, x=None) -> (B, E * len(global_features)).  Defaults = vit_small_patch16_384 (E 384, depth 12, 6 heads).
+    `precision` selects the tokenizer's embed path, `block_precision` the block stack's: "bf16" (default, rtol 1e-2) or
+    "fp32tc" (bf16x3 split operands on the same kernels, rtol 1e-4)."""
 
     def __init__(self, in_channels: int = 3, embed_dim: int = 384, pretrained_model: str = "vit_small_patch16_384.augreg_in21k_ft_in1k",
                  pretrained: bool = False, frozen: bool = False, k_neighbors: int = 16, global_features: str = "max,cls",
-                 depth: int = 12, num_heads: int = 6, mlp_ratio: float = 4.0, precision: str = "bf16", **p3embed_kwargs):
+                 depth: int = 12, num_heads: int = 6, mlp_ratio: float = 4.0, precision: str = "bf16", block_precision: str = "bf16",
+                 **p3embed_kwargs):
         super().__init__()
+        check_block_precision(block_precision)
+        self.block_precision = block_precision
         if pretrained:
             raise RuntimeError("PointViT: no timm / network in this build - construct with pretrained=False and load_state_dict() "
                                "a reference checkpoint (strict=False: timm's unused patch embedding / head keys are skipped)")
@@ -103,10 +116,12 @@ class PointViT(nn.Module):
     def _folded(self) -> List[torch.Tensor]:
         ver = tuple((t._version, t.data_ptr()) for t in self.vit.blocks.parameters())
         cache = self.__dict__.setdefault("_fold_cache", {})
-        if cache.get("ver") != ver:
-            cache["ver"] = ver
-            cache["params"] = [t for blk in self.vit.blocks for t in fold_timm_block(blk)]
-        return cache["params"]
+        hit = cache.get(self.block_precision)
+        if hit is None or hit[0] != ver:
+            fold_block = fold_timm_block_x3 if self.block_precision == "fp32tc" else fold_timm_block
+            hit = (ver, [t for blk in self.vit.blocks for t in fold_block(blk)])
+            cache[self.block_precision] = hit
+        return hit[1]
 
     def _run(self, p: torch.Tensor, x: Optional[torch.Tensor], start_idx=None):
         tok = self.__dict__["_tok"]
@@ -120,8 +135,9 @@ class PointViT(nn.Module):
         if len(eps) != 1:
             raise RuntimeError(f"PointViT: all LayerNorms must share one eps, got {sorted(eps)}")
         heads = self.vit.blocks[0].attn.num_heads
-        out, pooled = ops.vit_blocks(feats, pos, self._folded(), heads, self.norm.weight.detach().float(), self.norm.bias.detach().float(),
-                                     eps.pop(), 1)
+        blocks = ops.vit_blocks_x3 if self.block_precision == "fp32tc" else ops.vit_blocks
+        out, pooled = blocks(feats, pos, self._folded(), heads, self.norm.weight.detach().float(), self.norm.bias.detach().float(),
+                             eps.pop(), 1)
         return p_list, x_list, out, pooled
 
     def forward(self, p: torch.Tensor, x: Optional[torch.Tensor] = None, start_idx=None) -> Tuple[list, list, torch.Tensor]:
@@ -172,7 +188,8 @@ class ClsHead(nn.Module):
 class Pix4Point(nn.Module):
     """pix4point.py:328-437: PointViT encoder (`model`) + ClsHead on its 'max,cls' global features (`cls_head`, 2 * embed_dim
     inputs).  Same constructor arguments (plus the PointViT geometry, since timm cannot supply it here), same initialisation
-    (xavier linears, zero biases, unit BatchNorm; cls token / position ~ N(0, 0.02) when not pretrained), same helpers."""
+    (xavier linears, zero biases, unit BatchNorm; cls token / position ~ N(0, 0.02) when not pretrained), same helpers.
+    pointvit_kwargs go to PointViT (precision, block_precision, depth, num_heads, ...)."""
 
     def __init__(self, num_classes: int = 15, embed_dim: int = 768, pretrained_model: str = "vit_small_patch16_384.augreg_in21k_ft_in1k",
                  pretrained: bool = False, frozen: bool = False, k_neighbors: int = 16, **pointvit_kwargs):

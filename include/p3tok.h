@@ -295,12 +295,39 @@ P3TOK_API int p3tok_vit_forward(float* x, int64_t B, int64_t S, int64_t D, int64
                       const float* final_norm_b, float ln_eps, float* out_norm, float* pooled_out, int64_t pool_skip,
                       void* workspace, int64_t workspace_bytes, void* stream);
 
+/* The fp32-accurate forms of the two stacks above (bf16x3 on the tensor cores, the rtol 1e-4 contract of the fp32 tokenizer):
+ * every GEMM operand is a split pair v = hi + lo with hi = bf16(v), lo = bf16(v - hi), and a product is evaluated as
+ * a_hi.b_hi + a_lo.b_hi + a_hi.b_lo on tcgen05 (GEMMs) or mma.sync (attention: scores and P V; softmax in fp32).  Same
+ * arguments and the same p3tok_vit_layer descriptor, whose matrices then hold the x3 form, with Dp = D (D must be a multiple
+ * of 64) and HRp = pad64(H + R) (p3tok_vit_forward_x3: R = 0):
+ *   qkv_w  [3D, 3D]     proj_w [D, 3D]     fc1d_w [HRp, 3D]     fc2u_w [D, 3 HRp]       (bf16)
+ *   each W [out, in] of the bf16 layout above stored as [W_hi | W_hi | W_lo], in padded to a multiple of 64 with zeros
+ *   (p3tok/fold.py split_x3, from the float64 folded matrix); fc1d_w's rows H + R .. HRp - 1 are zero and fc1d_b has HRp
+ *   entries (zero past H + R): GELU(0) = ReLU(0) = 0, so the padding adds nothing.  Biases f32.
+ * Workspace: p3tok_vit_x3_workspace_bytes(B, G, D, H, R) (p3tok_vit_forward_x3: R = 0). */
+P3TOK_API int64_t p3tok_vit_x3_workspace_bytes(int64_t B, int64_t G, int64_t D, int64_t H, int64_t R);
+P3TOK_API int p3tok_apf_vit_forward_x3(float* x, int64_t B, int64_t G, int64_t D, int64_t heads, int64_t H, int64_t R,
+                             const p3tok_vit_layer* layers, int64_t n_layers, const float* final_norm_w,
+                             const float* final_norm_b, float ln_eps, float* pooled_out, void* workspace,
+                             int64_t workspace_bytes, void* stream);
+P3TOK_API int p3tok_vit_forward_x3(float* x, int64_t B, int64_t S, int64_t D, int64_t heads, int64_t H,
+                         const p3tok_vit_layer* layers, int64_t n_layers, const float* pos, const float* final_norm_w,
+                         const float* final_norm_b, float ln_eps, float* out_norm, float* pooled_out, int64_t pool_skip,
+                         void* workspace, int64_t workspace_bytes, void* stream);
+
 /* Building blocks of the above, exported for tests.
  * p3tok_layernorm_bf16: out = bf16(LN(x; w, b)) over the rows of x (M,D) f32; w = b = NULL: normalisation only.
  * p3tok_attention_bf16: qkv (B*G, 3D) bf16 laid out as AttentionLayer's reshape(B,N,3,heads,hd) -> out (B*G, D) bf16. */
 P3TOK_API int p3tok_layernorm_bf16(const float* x, int64_t M, int64_t D, float eps, const float* w, const float* b,
                          void* out, void* stream);
 P3TOK_API int p3tok_attention_bf16(const void* qkv, int64_t B, int64_t G, int64_t D, int64_t heads, void* out, void* stream);
+/* Their split forms (the building blocks of the _x3 stacks), exported for tests:
+ * p3tok_layernorm_split: out (M, 2D) bf16 = [hi | lo] of LN(x; w, b);
+ * p3tok_attention_x3: qkv (B*G, 6D) bf16 = [hi | lo] of the qkv matrix above (lo of column c at column 3D + c) -> out
+ * (B*G, 2D) bf16 = [hi | lo] of softmax(q k^T / sqrt(hd)) v. */
+P3TOK_API int p3tok_layernorm_split(const float* x, int64_t M, int64_t D, float eps, const float* w, const float* b,
+                          void* out, void* stream);
+P3TOK_API int p3tok_attention_x3(const void* qkv, int64_t B, int64_t G, int64_t D, int64_t heads, void* out, void* stream);
 /* p3tok_linear_bf16 with the ViT epilogues: act 0 none / 1 ReLU / 2 exact GELU / 3 GELU on columns < gelu_cols and ReLU on
  * the rest; then, if residual != NULL, out_f32 = res_mul * residual + out_scale * act(A W^T + bias) (residual may alias
  * out_f32).  N <= 2048 per call. */
