@@ -55,8 +55,6 @@ struct FusedParams {
   int nch;                          // chunk operand buffers in shared memory: 2, or 1 when the weight rings need the room
   int nacc;                         // chunk accumulators in TMEM: 2 when N2 <= 256, else 1 (384 output + 128 chunk columns = 512)
   int nq, nq_rows;                  // output columns per B-MMA: N2 (nq = 1) or N2/2 (nq = 2, N2 > 256)
-  int xtile;                        // A-GEMM of the next tile's first chunk issued before this tile's last B-GEMM (P3TOK_FUSED_XTILE)
-  int a_reuse;                      // nq = 2: second MMA of a K step re-uses the A operand from the collector (P3TOK_FUSED_AREUSE)
   const float* bias_a;              // [N1] or null
   const float* gbias;               // [M / rows_per_group, N1] or null; rows_per_group % 32 == 0
   int rows_per_group;
@@ -263,11 +261,10 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         __syncwarp();
         ++gc;
       };
-      // P3TOK_FUSED_XTILE=1: the A-GEMM runs one chunk ahead of the B-GEMM ACROSS tiles (chunk 0 of the next tile issued
+      // Measured and dropped: the A-GEMM running one chunk ahead of the B-GEMM ACROSS tiles (chunk 0 of the next tile issued
       // before the last B-GEMM of this tile) to give the tensor pipe work while the tile epilogue drains the output
       // accumulator (~4600 of 24700 cycles per tile at E = 384).  Measured on the same box: c2 0.977 vs 0.947 ms per step
       // WITHOUT it - the early A(0) delays the last B-GEMM and with it the tile epilogue that the next B(0) waits for.
-      // Off by default.
       // Also measured and dropped (round 2, last session): the issuing thread POLLING the A and B streams' barriers
       // (mbarrier.test_wait) and issuing whichever k-block / K step has its operands, instead of parking inside A(j+1) on
       // the weight box the 5-slot A ring cannot hold yet while B(j) is ready (the "Anext" stamps of
@@ -275,20 +272,15 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       // stream has priority: one thread walking a state machine with 4-6 barrier probes (a shared-memory round trip each)
       // per step needs longer per k-block than the 260 cycles its four MMAs take, so the tensor pipe starves on ISSUE.
       // The blocking walk costs ~15 instructions per k-block.
-      auto first_A = [&](int tile_it) {
-        if (issuer) fu_trace(p, tile_it, 0, 4, clock64());        // tile start
-        mbar_wait(a0_full, (uint32_t)(tile_it & 1));
-        if (issuer) fu_trace(p, tile_it, 0, 5, clock64());        // A0 present
+      for (int tp = pair_id; tp < p.num_pairs; tp += pair_stride, ++it) {
+        if (issuer) fu_trace(p, it, 0, 4, clock64());        // tile start
+        mbar_wait(a0_full, (uint32_t)(it & 1));
+        if (issuer) fu_trace(p, it, 0, 5, clock64());        // A0 present
         tc_fence_after();
         issue_A(NC == 1);
-        if (issuer) fu_trace(p, tile_it, 0, 6, clock64());        // A(0) issued
-      };
-      if (p.xtile && pair_id < p.num_pairs) first_A(0);
-      for (int tp = pair_id; tp < p.num_pairs; tp += pair_stride, ++it) {
-        if (!p.xtile) first_A(it);
+        if (issuer) fu_trace(p, it, 0, 6, clock64());        // A(0) issued
         for (int j = 0; j < NC; ++j) {
           if (j + 1 < NC) issue_A(j + 1 == NC - 1);
-          else if (p.xtile && tp + pair_stride < p.num_pairs) first_A(it + 1);
           // B(j): output accumulator += chunk(j) . W_b[:, chunk j]^T, one MMA group per quarter of the output columns
           const uint32_t b = p.nch == 2 ? (gcb & 1) : 0u;          // chunk operand buffer and how often it was used
           const uint32_t cuse = p.nch == 2 ? (gcb >> 1) : gcb;
@@ -297,7 +289,7 @@ tc_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           if (issuer) fu_trace(p, it, j, 1, clock64());           // chunk j operand ready
           if (j == 0) mbar_wait(acc3_empty, (uint32_t)(it & 1) ^ 1);
           tc_fence_after();
-          if (NQ == 2 && p.a_reuse) {
+          if (NQ == 2) {
             // two output column groups: both MMAs of a K step read the same chunk operand - the second one takes it from
             // the A collector instead of shared memory (this kernel is bound by shared-memory bandwidth)
             for (int kb2 = 0; kb2 < 2; ++kb2) {
@@ -718,12 +710,6 @@ int tc_fused(const __nv_bfloat16* A0, int64_t M, int K0, const __nv_bfloat16* Wa
   p.nacc = N2 <= 256 ? 2 : 1;
   p.nq = N2 > 256 ? 2 : 1;
   p.nq_rows = N2 / p.nq;
-  static int areuse_on = -1;
-  if (areuse_on < 0) { const char* e = getenv("P3TOK_FUSED_AREUSE"); areuse_on = e ? atoi(e) : 1; }
-  p.a_reuse = areuse_on && p.nq == 2;
-  static int xtile_on = -1;
-  if (xtile_on < 0) { const char* e = getenv("P3TOK_FUSED_XTILE"); xtile_on = e ? atoi(e) : 0; }
-  p.xtile = xtile_on;
   p.rb_box = (p.nq_rows / 2) * 128;
   P3_REQUIRE(fused_rings(K0, N1, N2, p.store_out != 0, l1 != nullptr, p.nch, p.ra_slots, p.rb_slots, p.rb_box), P3TOK_ERR_UNSUPPORTED,
              "tc_fused: shapes do not fit shared memory");

@@ -53,10 +53,7 @@ namespace p3tok {
 
 // ------------------------------------------------------------------------------------------------ GEMM
 constexpr int TC_MAX_STAGES = 8;
-#ifndef P3TOK_EPI_WARPS
-#define P3TOK_EPI_WARPS 8
-#endif
-constexpr int TC_EPI_WARPS = P3TOK_EPI_WARPS;        // default epilogue-warp count: 2 warps per TMEM lane quarter (see TcCfg below)
+constexpr int TC_EPI_WARPS = 8;                      // default epilogue-warp count: 2 warps per TMEM lane quarter (see TcCfg below)
 constexpr int TC_MAX_KB = 8;                         // A-resident mode: K <= 512
 constexpr int TC_A_STAGE = TC_BM * TC_BK * 2;        // 16 KB
 constexpr int TC_STAGING = 32 * 128;                 // one 32-row x 64-column bf16 store box (4 KB, 128B-swizzled)
@@ -65,10 +62,7 @@ constexpr int TC_MAX_N = 2048;                       // bias vector staged in sh
 // is sized at launch to fill what is left: a stage round trip (TMA latency ~1500 cycles + MMA drain) needs
 // >= ingest_rate x latency bytes in flight, so the pair mode (32 KB stages) runs 5-6 stages deep.
 constexpr int TC_SMEM = 227 * 1024;
-#ifndef P3TOK_EPI_BOXES
-#define P3TOK_EPI_BOXES (P3TOK_EPI_WARPS > 8 ? 1 : 2)
-#endif
-constexpr int TC_EPI_BOXES = P3TOK_EPI_BOXES;        // TMA-store boxes per epilogue warp (2 = double-buffered)
+constexpr int TC_EPI_BOXES = 2;                      // TMA-store boxes per epilogue warp (2 = double-buffered)
 constexpr int TC_SGB_BYTES = 256;                    // per-warp 64-float group-bias slice
 // The epilogue-warp count is a template parameter of the kernel: EW = TC_EPI_WARPS (8) for the tokenizer's layers, whose
 // tiles are MMA-bound (16 warps measured -12 % there: registers), EW = 16 for the small-M bf16-output GEMMs of the ViT
@@ -86,8 +80,6 @@ struct TcCfg {
 struct TcParams {
   int M, N, K, BN;
   int num_m_tiles, num_n_tiles;
-  int CL;                  // cluster size (1, 2 or 4): CTAs of a cluster take consecutive M tiles of the same
-                           // N tile and share the weight tile by TMA multicast (each loads BN/CL rows of it)
   const float* bias;       // [N] or null
   const float* gbias;      // [ceil(M/rows_per_group), N] or null
   int rows_per_group;
@@ -109,7 +101,6 @@ struct TcParams {
                            // [W_hi | W_hi | W_lo], K = 3 Kp: k-blocks of the third segment re-read the hi half of A
   int out_split;           // out_bf16 is [M, 2 N] = [hi | lo] of the fp32 result (the next layer's split operand)
   int split_lo;            // out_split: column of the lo half relative to hi (N, or the full width when out_bf16 is a column slice)
-  int prefetch;            // L2-prefetch the next item's activation tile
   int ares;                // A-resident mode (pairs only): a pair walks ALL N tiles of its M group, the group's activation
                            // rows stay in shared memory and only weight boxes stream through the ring
   unsigned long long* trace;  // debug (P3TOK_TC_TRACE=1): per-CTA clock stamps, 16 words per tile per role
@@ -333,7 +324,7 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);   // provably warp-uniform role index
   const int lane = threadIdx.x & 31;
-  const int CL = p.CL;
+  constexpr int CL = PAIR ? 2 : 1;                    // a pair's CTAs take consecutive M tiles and half the weight tile each
   const int rank = CL > 1 ? (int)cluster_ctarank() : 0;
   const int cluster_id = blockIdx.x / CL, num_clusters = gridDim.x / CL;
   const int num_mg = (p.num_m_tiles + CL - 1) / CL;
@@ -352,14 +343,13 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     nt = item - mg * p.num_n_tiles;
     return item < num_items;
   };
-  const uint16_t mc_mask = (uint16_t)((1u << CL) - 1);
 
   if (threadIdx.x == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmB)) : "memory");
     for (int s = 0; s < TC_STAGES; ++s) {
       mbar_init(&full[s], 1);
-      mbar_init(&empty[s], PAIR ? 1 : CL);   // multicast: every CTA of the cluster must have consumed the slot
+      mbar_init(&empty[s], 1);
     }
     for (int b = 0; b < 2; ++b) {
       mbar_init(&tfull[b], 1);
@@ -383,7 +373,7 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();   // peers' barriers are initialised before any multicast / remote arrive
+  if (CL > 1) cluster_sync_all();   // peers' barriers are initialised before any pair load / remote arrive
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
@@ -396,14 +386,14 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     // bytes landing on this CTA's (pair: the leader's) full barrier per stage
     const uint32_t tx = PAIR ? 2u * ((ARES ? 0u : (uint32_t)TC_A_STAGE) + (uint32_t)(p.BN / 2) * TC_BK * 2)
                              : TC_A_STAGE + (uint32_t)p.BN * TC_BK * 2;
-    const int brows = p.BN / CL;     // rows of the weight tile this CTA fetches (and multicasts)
+    const int brows = p.BN / CL;     // rows of the weight tile this CTA fetches
     // A column of k-block kb: plain, or (bf16x3) [hi | lo | hi again] over the [hi | lo] operand
     const int kb_seg = p.x3 ? num_kb / 3 : num_kb;
     auto acol = [&](int kb) { return (p.x3 && kb >= 2 * kb_seg ? kb - 2 * kb_seg : kb) * TC_BK; };
     int mg, nt;
     for (int li = 0; decode(li, mg, nt); ++li) {
       const int mt = mg * CL + rank;   // may be a dummy tile past the end: TMA zero-fills, stores are clipped
-      if (p.prefetch && issuer && !ARES && !p.x3) {
+      if (issuer && !ARES && !p.x3) {
         // pull the NEXT item's activation tile (streamed from HBM exactly once) into L2 ahead of its loads
         int nmg, nnt;
         if (decode(li + 1, nmg, nnt)) {
@@ -426,8 +416,7 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           } else {
             mbar_expect_tx(&full[stage], tx);
             tma_load_2d(a_dst, &tmA, &full[stage], acol(kb), mt * TC_BM);
-            if (CL == 1) tma_load_2d(b_dst, &tmB, &full[stage], kb * TC_BK, nt * p.BN);
-            else tma_load_2d_mc(b_dst + rank * brows * 128, &tmB, &full[stage], kb * TC_BK, nt * p.BN + rank * brows, mc_mask);
+            tma_load_2d(b_dst, &tmB, &full[stage], kb * TC_BK, nt * p.BN);
           }
         }
         __syncwarp();
@@ -486,8 +475,7 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
               else tc_mma(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (uint32_t)((kb | k) != 0));
             }
             if (PAIR) tc_commit_pair(&empty[stage]);      // frees the stage in both CTAs of the pair
-            else if (CL == 1) tc_commit(&empty[stage]);   // frees the smem stage once these MMAs have read it
-            else tc_commit_mc(&empty[stage], mc_mask);    // ... in every CTA that multicasts into it
+            else tc_commit(&empty[stage]);                // frees the smem stage once these MMAs have read it
             if (PAIR && ARES && nt == p.num_n_tiles - 1) tc_commit_pair(&a_empty[kb]);   // last reader of this group's K block
           }
           __syncwarp();
@@ -681,19 +669,11 @@ static int tc_linear(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat
     P3_REQUIRE(ex->bn % 64 == 0 && ex->bn <= 256, P3TOK_ERR_INVALID, "tc_linear: tile width %d", ex->bn);
     p.BN = ex->bn;
   }
-  // P3TOK_TC_CLUSTER: 1 = one CTA per tile; 2/4 = TMA multicast of the weight tile across a cluster;
-  // P3TOK_TC_PAIR=1 (default): CTA pairs with cta_group::2 MMAs (M = 256 per pair, weight tile split)
-  static int want_cl = 0, want_pair = -1;
-  if (!want_cl) {
-    const char* e = getenv("P3TOK_TC_CLUSTER");
-    want_cl = e ? atoi(e) : 1;
-    if (want_cl != 1 && want_cl != 2 && want_cl != 4) want_cl = 1;
-    const char* e2 = getenv("P3TOK_TC_PAIR");
-    want_pair = e2 ? atoi(e2) : 1;
-  }
-  const bool pair = want_pair && ((M + TC_BM - 1) / TC_BM) >= 2;
   p.num_m_tiles = (int)((M + TC_BM - 1) / TC_BM);
   p.num_n_tiles = (N + p.BN - 1) / p.BN;
+  // CTA pairs with cta_group::2 MMAs (M = 256 per pair, weight tile split) wherever there are two M tiles
+  const bool pair = p.num_m_tiles >= 2;
+  const int CL = pair ? 2 : 1;
   p.bias = bias; p.gbias = gbias; p.rows_per_group = rows_per_group > 0 ? rows_per_group : 1; p.relu = relu;
   p.out_bf16 = out_bf16; p.out_f32 = out_f32; p.out_max = out_max; p.out_max_bf16 = out_max_bf16; p.max_relu = max_relu;
   p.gelu = ex ? ex->gelu : 0;
@@ -711,22 +691,18 @@ static int tc_linear(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat
   const int64_t ldc = p.out_split ? 2 * (int64_t)p.split_lo : ((ex && ex->ldc > 0) ? ex->ldc : N);   // row pitch of out_bf16
   P3_REQUIRE(ldc == N || (out_bf16 && (!out_f32 || p.out_split) && ldc % 8 == 0), P3TOK_ERR_UNSUPPORTED, "tc_linear: ldc only for bf16 outputs");
   // 16 epilogue warps (lean epilogue: bf16 or TMA-stored / TMA-added fp32 outputs only), asked for by the ViT blocks
-  static int epi16_on = -1;
-  if (epi16_on < 0) { const char* e = getenv("P3TOK_TC_EPI16"); epi16_on = e ? atoi(e) : 1; }
-  const bool want16 = epi16_on && ex && ex->epi16 && !out_max && !out_max_bf16 && !gbias && !(out_bf16 && out_f32);
+  const bool want16 = ex && ex->epi16 && !out_max && !out_max_bf16 && !gbias && !(out_bf16 && out_f32);
   CUtensorMap ta, tb, tc;
   int rc = make_map(&ta, A, M, p.x3 ? K / 3 * 2 : K, TC_BM);    // x3: the operand holds [hi | lo], 2/3 of the reduction length
   if (rc) return rc;
-  p.CL = pair ? 2 : want_cl;
-  while (p.CL > 1 && p.num_m_tiles < p.CL) p.CL /= 2;
-  rc = make_map(&tb, W, N, K, p.BN / p.CL);     // each CTA of a cluster fetches BN/CL rows of the weight tile
+  rc = make_map(&tb, W, N, K, p.BN / CL);       // each CTA of a pair fetches half the rows of the weight tile
   if (rc) return rc;
   p.f32_tma = 0;
   p.res_add = 0;
   if (out_bf16) {
     rc = make_map(&tc, out_bf16, M, p.out_split ? p.split_lo + N : N, 32, ldc);     // store boxes: 64 columns x 32 rows
     if (rc) return rc;
-  } else if (out_f32 && (TcCfg<TC_EPI_WARPS>::BOXES == 2 || want16) && N % 4 == 0 && (reinterpret_cast<uintptr_t>(out_f32) & 15) == 0) {
+  } else if (out_f32 && N % 4 == 0 && (reinterpret_cast<uintptr_t>(out_f32) & 15) == 0) {
     rc = make_map_f32(&tc, out_f32, M, N, 32);  // fp32 store boxes: 32 columns x 32 rows
     if (rc) return rc;
     p.f32_tma = 1;
@@ -752,28 +728,20 @@ static int tc_linear(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat
   const int smem_fixed = ew16 ? TcCfg<16>::SMEM_FIXED : TcCfg<TC_EPI_WARPS>::SMEM_FIXED;
   {
     const int wrows = pair ? p.BN / 2 : p.BN;
-    // A-resident mode (P3TOK_TC_ARES=0 disables): with several N tiles per M group the default walk re-fetches the same
+    // A-resident mode: with several N tiles per M group the default walk re-fetches the same
     // activation tile once per N tile, and at 128 rows per CTA the L2 -> shared-memory fill (activation tile + half a
     // weight tile per MMA group, ~62 B/cycle/SM at BN = 256) outruns what TMA delivers (~42 B/cycle/SM) before the
     // tensor pipe is busy.  Keeping the M group's rows resident halves the fill.
-    static int ares_on = -1;
-    if (ares_on < 0) { const char* e = getenv("P3TOK_TC_ARES"); ares_on = e ? atoi(e) : 1; }
     const int num_kb = (K + TC_BK - 1) / TC_BK;
     p.ares = 0;
-    if (ares_on && pair && !p.x3 && p.num_n_tiles >= 2 && num_kb <= TC_MAX_KB) {
+    if (pair && !p.x3 && p.num_n_tiles >= 2 && num_kb <= TC_MAX_KB) {
       const int ring = TC_SMEM - smem_fixed - num_kb * TC_A_STAGE;
       if (ring / (wrows * TC_BK * 2) >= 3) p.ares = 1;
     }
     p.stage_bytes = (p.ares ? 0 : TC_A_STAGE) + wrows * TC_BK * 2;
     p.stages = (TC_SMEM - smem_fixed - (p.ares ? num_kb * TC_A_STAGE : 0)) / p.stage_bytes;
     if (p.stages > TC_MAX_STAGES) p.stages = TC_MAX_STAGES;
-    static int cap = -1;
-    if (cap < 0) { const char* e = getenv("P3TOK_TC_STAGES"); cap = e ? atoi(e) : 0; }
-    if (cap > 1 && p.stages > cap) p.stages = cap;
   }
-  static int prefetch_on = -1;
-  if (prefetch_on < 0) { const char* e = getenv("P3TOK_TC_PREFETCH"); prefetch_on = e ? atoi(e) : 1; }
-  p.prefetch = prefetch_on;
   static int trace_on = -1;
   if (trace_on < 0) trace_on = getenv("P3TOK_TC_TRACE") ? 1 : 0;
   p.trace = nullptr;
@@ -785,21 +753,21 @@ static int tc_linear(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat
     P3_CUDA(cudaMalloc(&p.trace2, 8 * 4 * 8 * 8));
     P3_CUDA(cudaMemsetAsync(p.trace2, 0, 8 * 4 * 8 * 8, s));
   }
-  const int items = p.ares ? (p.num_m_tiles + p.CL - 1) / p.CL : ((p.num_m_tiles + p.CL - 1) / p.CL) * p.num_n_tiles;
-  const int max_clusters = num_sms() / p.CL;
+  const int items = p.ares ? (p.num_m_tiles + CL - 1) / CL : ((p.num_m_tiles + CL - 1) / CL) * p.num_n_tiles;
+  const int max_clusters = num_sms() / CL;
   const int clusters = items < max_clusters ? items : max_clusters;
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(clusters * p.CL));
+  cfg.gridDim = dim3((unsigned)(clusters * CL));
   cfg.blockDim = dim3(ew16 ? TcCfg<16>::THREADS : TcCfg<TC_EPI_WARPS>::THREADS);
   cfg.dynamicSmemBytes = TC_SMEM;
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)p.CL;
+  attr[0].val.clusterDim.x = (unsigned)CL;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = p.CL > 1 ? 1 : 0;
+  cfg.numAttrs = CL > 1 ? 1 : 0;
   if (ew16) {
     if (pair) P3_CUDA(cudaLaunchKernelEx(&cfg, tc_linear_kernel<true, 16>, ta, tb, tc, p));
     else P3_CUDA(cudaLaunchKernelEx(&cfg, tc_linear_kernel<false, 16>, ta, tb, tc, p));
@@ -823,7 +791,7 @@ static int tc_linear(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat
                 (long long)(q[1] - q[0]), (long long)(q[2] - q[1]), (long long)(q[3] - q[2]), (long long)(q[4] - q[3]),
                 (long long)(q[5] - q[4]), (long long)(q[6] - q[5]));
       }
-    fprintf(stderr, "[tc_trace] M=%d N=%d K=%d BN=%d CL=%d grid=%d ares=%d stages=%d\n", p.M, p.N, p.K, p.BN, p.CL, clusters * p.CL, p.ares, p.stages);
+    fprintf(stderr, "[tc_trace] M=%d N=%d K=%d BN=%d CL=%d grid=%d ares=%d stages=%d\n", p.M, p.N, p.K, p.BN, CL, clusters * CL, p.ares, p.stages);
     for (int cta = 0; cta < 2; ++cta) {
       const unsigned long long t0 = h[(((size_t)cta * 64 + 0) * 3 + 1) * 4 + 0];
       for (int it = 0; it < 8; ++it) {
@@ -1433,10 +1401,8 @@ int patch_embed_bf16(const p3tok_rows* R, const p3tok_mlp* m, void* ws, int64_t 
   const bool rot_rows = L.kpad0 && R->kind == 1 && R->D % 4 == 0 && R->D >= 4 &&
                         (reinterpret_cast<uintptr_t>(R->feats) & 15) == 0;
   // P3Embed stage >= 1 (a single wide per-point layer): the gather runs inside the GEMM's producer (embed_gather.cu) and the
-  // row matrix never exists.  P3TOK_GATHER_FUSED=0 selects the round-1 path (gather kernel + tc_linear).
-  static int gfuse_on = -1;
-  if (gfuse_on < 0) { const char* e = getenv("P3TOK_GATHER_FUSED"); gfuse_on = e ? atoi(e) : 1; }
-  const bool gather_fused = gfuse_on && rot_rows && m->n_pre == 1 && m->pre_relu[0] == 1 && tc_gather_linear_supported(R, m->pre_dim[0], k);
+  // row matrix never exists; other shapes gather to bf16 rows for tc_linear.
+  const bool gather_fused = rot_rows && m->n_pre == 1 && m->pre_relu[0] == 1 && tc_gather_linear_supported(R, m->pre_dim[0], k);
   const int64_t kpadw = gather_fused ? align_up(L.kpad0, 64) : L.kpad0;
   if (L.kpad0) {
     pad_weight_kernel<<<grid_1d((int64_t)m->pre_dim[0] * kpadw, 256), 256, 0, s>>>(
@@ -1454,12 +1420,10 @@ int patch_embed_bf16(const p3tok_rows* R, const p3tok_mlp* m, void* ws, int64_t 
     int kin;
     // APF blocks: the first layer runs inside the "pre" pair kernel (embed_fused.cu, FusedL1) - its 512-byte bf16 rows are
     // never written; what the pair kernel reads instead is 16 bytes per row (neighbour - centre) + one centre per 32 rows.
-    // P3TOK_L1_FUSED=0 selects the separate first-layer kernel.
-    static int l1f_on = -1, fuse_on0 = -1;
-    if (l1f_on < 0) { const char* e = getenv("P3TOK_L1_FUSED"); l1f_on = e ? atoi(e) : 1; }
+    static int fuse_on0 = -1;
     if (fuse_on0 < 0) { const char* e = getenv("P3TOK_FUSED"); fuse_on0 = e ? atoi(e) : 1; }
     FusedL1 l1;
-    const bool l1_fused = l1f_on && fuse_on0 && L.l1_rows_pad && !L.kpad0 && R->kind == 0 && (R->C == 3 || R->C == 4) && fused_max &&
+    const bool l1_fused = fuse_on0 && L.l1_rows_pad && !L.kpad0 && R->kind == 0 && (R->C == 3 || R->C == 4) && fused_max &&
                           m->pre_relu[1] == 1 && m->pre_relu[2] == 0 && tc_fused_l1_supported(m->pre_dim[1], m->pre_dim[2]);
     if (l1_fused) {
       char* l1b = base + L.off_l1;
@@ -1484,9 +1448,7 @@ int patch_embed_bf16(const p3tok_rows* R, const p3tok_mlp* m, void* ws, int64_t 
 #define P3_L1(IDX, CPV)                                                                                        \
   rows_first_layer_kernel<IDX, CPV><<<blocks, 128, 0, s>>>(*R, g0, rows, (const __nv_bfloat16*)m->w_pre[0],    \
                                                            m->b_pre[0], m->cin, m->pre_dim[0], m->pre_relu[0], act[cur], l1_gmax)
-      static int apf_split = -1;
-      if (apf_split < 0) { const char* e = getenv("P3TOK_L1_SPLIT"); apf_split = e ? atoi(e) : 1; }
-      if (apf_split && R->kind == 0 && k % 32 == 0 && (R->C == 3 || R->C == 4) &&
+      if (R->kind == 0 && k % 32 == 0 && (R->C == 3 || R->C == 4) &&
           (m->pre_dim[0] == 64 || m->pre_dim[0] == 128 || m->pre_dim[0] == 256)) {
         const unsigned nb = (unsigned)std::min<int64_t>((blocks + 3) / 4, (int64_t)num_sms() * 10);
 #define P3_L1A(IDX, NPL)                                                                                              \
@@ -1496,7 +1458,7 @@ int patch_embed_bf16(const p3tok_rows* R, const p3tok_mlp* m, void* ws, int64_t 
         if (i64) { if (npl == 2) P3_L1A(int64_t, 2); else if (npl == 4) P3_L1A(int64_t, 4); else P3_L1A(int64_t, 8); }
         else     { if (npl == 2) P3_L1A(int32_t, 2); else if (npl == 4) P3_L1A(int32_t, 4); else P3_L1A(int32_t, 8); }
 #undef P3_L1A
-      } else if (apf_split && R->kind == 0 && k % 32 == 0 && (R->C == 3 || R->C == 4) && m->pre_dim[0] % 2 == 0) {
+      } else if (R->kind == 0 && k % 32 == 0 && (R->C == 3 || R->C == 4) && m->pre_dim[0] % 2 == 0) {
         if (i64) rows_first_layer_apf_kernel<int64_t><<<blocks, 128, 0, s>>>(*R, g0, rows, (const __nv_bfloat16*)m->w_pre[0],
                                                                           m->b_pre[0], m->pre_dim[0], m->pre_relu[0], act[cur]);
         else rows_first_layer_apf_kernel<int32_t><<<blocks, 128, 0, s>>>(*R, g0, rows, (const __nv_bfloat16*)m->w_pre[0],

@@ -20,8 +20,6 @@
 // fps_cluster_trace.cu: a B200 seats only 15 clusters of 8 (or 7) CTAs - a cluster must sit inside one
 // GPC - so the 16 clouds of BASELINE configs[3] ran as TWO waves (3.9 ms); as clusters of 6 (10923
 // points per CTA; 22 seats) they are one (2.3 ms).
-#include <stdlib.h>
-
 #include <cooperative_groups.h>
 #include <cuda/ptx>
 
@@ -395,12 +393,9 @@ extern "C" int p3tok_fps(const float* x, int64_t B, int64_t N, int64_t pt_stride
   cudaStream_t s = as_stream(stream);
   const int Bi = (int)B, Ni = (int)N, Gi = (int)G, ps = (int)pt_stride;
   if (N <= FPS_SLICE) {           // one CTA per cloud, every point in registers
-    static int ppt_env = -1;      // P3TOK_FPS_PPT=8|16|32 forces the points per thread (experiments)
-    if (ppt_env < 0) { const char* e = getenv("P3TOK_FPS_PPT"); ppt_env = e ? atoi(e) : 0; }
-    const int ppt = ppt_env ? ppt_env : (Ni >= 1024 ? 16 : 8);   // measured: 16 beats 8 by 9-12 % from N = 1024 up, 32 is no better
+    const int ppt = Ni >= 1024 ? 16 : 8;   // measured: 16 beats 8 by 9-12 % from N = 1024 up, 32 is no better
     int threads = ((Ni + ppt - 1) / ppt + 31) / 32 * 32;
     if (threads < 32) threads = 32;
-    if (ppt == 32) return fps_launch<1, 32>(x, Bi, Ni, ps, start_idx, Gi, out_idx, Ni, threads, 1, s);
     if (ppt == 16) return fps_launch<1, 16>(x, Bi, Ni, ps, start_idx, Gi, out_idx, Ni, threads, 1, s);
     return fps_launch<1, 8>(x, Bi, Ni, ps, start_idx, Gi, out_idx, Ni, threads, 1, s);
   }
@@ -414,12 +409,9 @@ extern "C" int p3tok_fps(const float* x, int64_t B, int64_t N, int64_t pt_stride
   static thread_local int seats[32][17][33];  // [device][cluster size][warps per CTA]: 0 = not asked yet
   int dev = 0;
   P3_CUDA(cudaGetDevice(&dev));
-  static int cl_env = -1;                     // P3TOK_FPS_CLUSTER=n forces the cluster size (experiments)
-  if (cl_env < 0) { const char* e = getenv("P3TOK_FPS_CLUSTER"); cl_env = e ? atoi(e) : 0; }
   int best_cl = 0, best_threads = 0, best_slice = 0;
   double best_cost = 0;
   for (int cl = hi; cl >= lo && cl >= 1; --cl) {
-    if (cl_env >= lo && cl_env <= hi && cl != cl_env) continue;
     const int slice = (Ni + cl - 1) / cl;
     const bool wide = slice > FPS_SLICE;
     if (wide && cl > 8) continue;             // the 16-CTA instantiation holds regular slices only

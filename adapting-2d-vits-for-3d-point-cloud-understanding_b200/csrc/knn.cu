@@ -442,7 +442,7 @@ template <int KPL, int MODE>
 __global__ void __launch_bounds__(KNN_WARPS * 32, KPL == 1 ? KNS_MIN_BLOCKS : 4)
 knn_sorted_kernel(const float4* __restrict__ pts, const int* __restrict__ ids, const float* __restrict__ bb,
                   const int* __restrict__ lut, const float* __restrict__ meta_all, int S, int nblk, const float* __restrict__ centres,
-                  int G, int64_t total, int k, void* __restrict__ idx_out, int idx_is_i64, float* __restrict__ dist_out, int best_first) {
+                  int G, int64_t total, int k, void* __restrict__ idx_out, int idx_is_i64, float* __restrict__ dist_out) {
   __shared__ uint64_t queue[KNN_WARPS][64];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t cw = (int64_t)blockIdx.x * KNN_WARPS + warp;      // this warp's centre
@@ -535,8 +535,8 @@ knn_sorted_kernel(const float4* __restrict__ pts, const int* __restrict__ ids, c
   // is tight after the first 2-3 blocks (the genuinely nearest ~96 points), so far fewer candidates pass the filter and
   // reach the queue merges that bound this kernel than in curve order (round 1: seed from the curve position, then all
   // blocks in index order - ~10 merges per centre at N = 8192, k = 32).
-  if (best_first && nblk >= 128) {     // (measured: neutral on uniform clouds, +6 % on clustered ones at N = 8192; below
-                                       //  4096 points the 8-keys-per-lane bookkeeping costs more than it saves)
+  if (nblk >= 128) {     // (measured: neutral on uniform clouds, +6 % on clustered ones at N = 8192; below
+                         //  4096 points the 8-keys-per-lane bookkeeping costs more than it saves)
     for (int r0 = 0; r0 < nblk; r0 += 256) {
       uint32_t key[8];
 #pragma unroll
@@ -637,12 +637,10 @@ static int knn_sorted_launch(const float4* pts, const int* ids, const float* bb,
                              const float* centres, int G, int64_t total, int k, int mode, void* idx_out, int i64, float* dist_out,
                              cudaStream_t s) {
   const unsigned grid = (unsigned)((total + KNN_WARPS - 1) / KNN_WARPS);
-  static int bf = -1;          // P3TOK_KNN_BEST_FIRST=0: the round-1 traversal (seed from the curve position, then index order)
-  if (bf < 0) { const char* e = getenv("P3TOK_KNN_BEST_FIRST"); bf = e ? atoi(e) : 1; }
   if (mode == P3TOK_KNN_APF_SQ)
-    knn_sorted_kernel<KPL, P3TOK_KNN_APF_SQ><<<grid, KNN_WARPS * 32, 0, s>>>(pts, ids, bb, lut, meta, S, nblk, centres, G, total, k, idx_out, i64, dist_out, bf);
+    knn_sorted_kernel<KPL, P3TOK_KNN_APF_SQ><<<grid, KNN_WARPS * 32, 0, s>>>(pts, ids, bb, lut, meta, S, nblk, centres, G, total, k, idx_out, i64, dist_out);
   else
-    knn_sorted_kernel<KPL, P3TOK_KNN_P4P_CDIST><<<grid, KNN_WARPS * 32, 0, s>>>(pts, ids, bb, lut, meta, S, nblk, centres, G, total, k, idx_out, i64, dist_out, bf);
+    knn_sorted_kernel<KPL, P3TOK_KNN_P4P_CDIST><<<grid, KNN_WARPS * 32, 0, s>>>(pts, ids, bb, lut, meta, S, nblk, centres, G, total, k, idx_out, i64, dist_out);
   P3_LAUNCH_CHECK("knn_sorted_kernel");
   return P3TOK_OK;
 }
@@ -690,19 +688,6 @@ static KnsPtrs kns_ptrs(void* workspace, int64_t B, int64_t N) {
   p.meta = reinterpret_cast<float*>(base + L.off_meta);
   return p;
 }
-
-namespace p3tok {
-// views into a prepared workspace for the block-culled FPS (fps_culled.cu)
-int kns_workspace_views(const void* workspace, int64_t workspace_bytes, int64_t B, int64_t N, const float4** pts, const int** ids,
-                        const float** bb) {
-  P3_REQUIRE(N > 0 && N <= KNS_MAX_N && B >= 0, P3TOK_ERR_UNSUPPORTED, "sorted workspace: N=%lld outside (0, %d]", (long long)N, KNS_MAX_N);
-  P3_REQUIRE(workspace_bytes >= kns_layout(B, N).total, P3TOK_ERR_WORKSPACE, "sorted workspace %lld < %lld bytes",
-             (long long)workspace_bytes, (long long)kns_layout(B, N).total);
-  const KnsPtrs w = kns_ptrs(const_cast<void*>(workspace), B, N);
-  *pts = w.pts; *ids = w.ids; *bb = w.bb;
-  return P3TOK_OK;
-}
-}  // namespace p3tok
 
 // The preparation half (depends on the clouds only, not on the centres) ...
 extern "C" int p3tok_knn_prepare(const float* x, int64_t B, int64_t N, int64_t pt_stride, void* workspace, int64_t workspace_bytes,

@@ -55,24 +55,9 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, u
       "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
-// multicast variant: the box lands at the same smem offset in every CTA of `mask`, and each destination's
-// mbarrier (same offset) receives the complete_tx
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(
-          smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
 // L2 prefetch of a tensor box (no shared memory, no barrier): turns the later TMA load into an L2 hit
 __device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* map, int c0, int c1) {
   asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void tc_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(mask)
                : "memory");
 }
 // ---- CTA-pair (cta_group::2) forms: one MMA spans both SMs of the pair (M = 256), each CTA holds its 128

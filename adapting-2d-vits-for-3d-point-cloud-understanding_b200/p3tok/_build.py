@@ -15,7 +15,7 @@ INCLUDE = os.path.join(_ROOT, "include")
 LIB_PATH = os.path.join(_PKG, "libp3tok.so")
 OBJ_DIR = os.path.join(CSRC, "_obj")
 
-SOURCES = ["capi.cu", "fps.cu", "fps_culled.cu", "fps_nd.cu", "sqdist.cu", "knn.cu", "group.cu", "mlp_f32.cu", "embed_tc.cu", "embed_fused.cu", "embed_stage.cu", "embed_gather.cu", "vit.cu", "train.cu", "train_vit.cu"]
+SOURCES = ["capi.cu", "fps.cu", "fps_nd.cu", "sqdist.cu", "knn.cu", "group.cu", "mlp_f32.cu", "embed_tc.cu", "embed_fused.cu", "embed_stage.cu", "embed_gather.cu", "vit.cu", "train.cu", "train_vit.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "--expt-extended-lambda", "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC",
@@ -39,10 +39,6 @@ def _newer(target: str, deps: List[str]) -> bool:
 
 def build_library(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(OBJ_DIR, exist_ok=True)
-    extra = []
-    if os.environ.get("P3TOK_EPI_WARPS"):          # experiment knob: epilogue warps of tc_linear_kernel (8 or 16)
-        extra = ["-DP3TOK_EPI_WARPS=" + os.environ["P3TOK_EPI_WARPS"]]
-        force = True
     headers = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))]
     headers += [os.path.join(INCLUDE, f) for f in os.listdir(INCLUDE)]
     nvcc = _nvcc()
@@ -53,7 +49,7 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
         o = os.path.join(OBJ_DIR, src.replace(".cu", ".o"))
         objs.append(o)
         if force or _newer(o, [s] + headers):
-            jobs.append([nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", s, "-o", o])
+            jobs.append([nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", s, "-o", o])
 
     def run(cmd):
         r = subprocess.run(cmd, capture_output=True, text=True)

@@ -55,7 +55,6 @@ _SIGNATURES = {
     "p3tok_last_error": (ctypes.c_char_p, []),
     "p3tok_kernel_launches": (_i64, []),
     "p3tok_fps": (_int, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _vp]),
-    "p3tok_fps_sorted": (_int, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _vp]),
     "p3tok_fps_nd": (_int, [_vp, _i64, _i64, _i64, _i64, _vp, _i64, _vp, _vp, _vp]),
     "p3tok_square_distance": (_int, [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _vp]),
     "p3tok_gather_points": (_int, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _vp]),
@@ -130,7 +129,7 @@ def lib() -> ctypes.CDLL:
             fn = getattr(L, name)
             fn.restype = res
             fn.argtypes = args
-        if L.p3tok_abi_version() != 2:
+        if L.p3tok_abi_version() != 3:
             raise RuntimeError("libp3tok.so ABI version mismatch; rebuild")
         _lib = L
     return _lib

@@ -9,7 +9,6 @@ implementation for any device but CUDA.
 from __future__ import annotations
 
 import ctypes
-import os
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -102,38 +101,10 @@ def _point_stride(x: torch.Tensor) -> Tuple[torch.Tensor, int]:
 
 
 # --------------------------------------------------------------------------------------------- fps
-# Block-culled FPS on the sorted workspace (N <= 8192, csrc/fps_culled.cu): exact and parity-green, but MEASURED no faster
-# than the sweep kernel on B200 (c3: 3.07 vs 2.95 ms; c2 / c5: 2-3x slower) - an FPS iteration is bound by the latency of
-# its reduction chain (redux.sync, barrier, broadcast), not by the distance pass the culling removes - so it is opt-in.
-_FPS_CULLED = os.environ.get("P3TOK_FPS_CULLED", "0") != "0"
-_FPS_CULLED_MIN_N = int(os.environ.get("P3TOK_FPS_CULLED_MIN_N", "4096"))
-
-
-def _use_culled_fps(B: int, N: int, npoint: int) -> bool:
-    return (_FPS_CULLED and _KNN_SORTED and B > 0 and npoint >= 8 and _FPS_CULLED_MIN_N <= N <= 8192
-            and int(_L().p3tok_knn_workspace_bytes(B, N)) > 0)
-
-
 @torch.library.custom_op("p3tok::fps", mutates_args=(), device_types="cuda")
 def fps(x: torch.Tensor, start_idx: torch.Tensor, npoint: int) -> torch.Tensor:
-    """(B,npoint) int64 FPS indices.  Clouds of at most 8192 points are first sorted into the kNN workspace
-    (p3tok_knn_prepare) and sampled by the block-culled kernel (p3tok_fps_sorted); larger ones (or P3TOK_FPS_CULLED=0)
-    by the sweep kernel (p3tok_fps, a thread-block cluster per cloud beyond 8192 points).  Same picks either way."""
-    _need_cuda("fps", x, start_idx)
-    B, N = int(x.shape[0]), int(x.shape[1])
-    if _use_culled_fps(B, N, npoint):
-        return fps_sorted(x, knn_prepare(x), start_idx, npoint)
-    return fps_sweep(x, start_idx, npoint)
-
-
-@fps.register_fake
-def _(x, start_idx, npoint):
-    return x.new_empty((x.shape[0], npoint), dtype=torch.int64)
-
-
-@torch.library.custom_op("p3tok::fps_sweep", mutates_args=(), device_types="cuda")
-def fps_sweep(x: torch.Tensor, start_idx: torch.Tensor, npoint: int) -> torch.Tensor:
-    """The sweep kernel (p3tok_fps): every iteration updates every point; one CTA per cloud, a cluster beyond 8192 points."""
+    """(B,npoint) int64 FPS indices (p3tok_fps): every iteration updates every point; one CTA per cloud, a
+    thread-block cluster per cloud beyond 8192 points."""
     _need_cuda("fps", x, start_idx)
     B, N = int(x.shape[0]), int(x.shape[1])
     x = x if x.dtype == torch.float32 else x.float()
@@ -147,7 +118,7 @@ def fps_sweep(x: torch.Tensor, start_idx: torch.Tensor, npoint: int) -> torch.Te
     return out
 
 
-@fps_sweep.register_fake
+@fps.register_fake
 def _(x, start_idx, npoint):
     return x.new_empty((x.shape[0], npoint), dtype=torch.int64)
 
@@ -221,10 +192,6 @@ def _(x, idx):
 
 
 # --------------------------------------------------------------------------------------------- knn
-_KNN_SORTED = os.environ.get("P3TOK_KNN_SORTED", "1") != "0"
-_OVERLAP = os.environ.get("P3TOK_OVERLAP", "auto")         # FPS and the kNN preparation on two streams: 0 / 1 / auto
-
-
 @torch.library.custom_op("p3tok::knn", mutates_args=(), device_types="cuda")
 def knn(x: torch.Tensor, centres: torch.Tensor, k: int, mode: int, int32_out: bool,
         return_dist: bool) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -242,9 +209,8 @@ def knn(x: torch.Tensor, centres: torch.Tensor, k: int, mode: int, int32_out: bo
     idx = torch.empty((B, G, k), dtype=torch.int32 if int32_out else torch.int64, device=x.device)
     dist = torch.empty((B, G, k) if return_dist else (0,), dtype=torch.float32, device=x.device)
     # Z-order sorted blocks + bounding-box culling (same results bit for bit; clouds beyond 8192 points as segments of
-    # 8192, up to 131072);
-    # P3TOK_KNN_SORTED=0 forces the plain sweep
-    ws_bytes = int(_L().p3tok_knn_workspace_bytes(B, N)) if _KNN_SORTED and B * G > 0 else 0
+    # 8192, up to 131072); the plain sweep beyond that
+    ws_bytes = int(_L().p3tok_knn_workspace_bytes(B, N)) if B * G > 0 else 0
     with torch.cuda.device(x.device), _timed("knn"):
         if ws_bytes > 0:
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
@@ -268,14 +234,14 @@ def _(x, centres, k, mode, int32_out, return_dist):
 @torch.library.custom_op("p3tok::knn_prepare", mutates_args=(), device_types="cuda")
 def knn_prepare(x: torch.Tensor) -> torch.Tensor:
     """The centre-independent half of the sorted kNN (Z-order sort + block boxes of every cloud) -> workspace bytes;
-    empty when the sorted variant does not apply (N > 131072 or P3TOK_KNN_SORTED=0).  Enqueued on the CURRENT stream:
+    empty when the sorted variant does not apply (N > 131072).  Enqueued on the CURRENT stream:
     modules run it on a side stream next to FPS."""
     _need_cuda("knn_prepare", x)
     x_in = x
     x = x if x.dtype == torch.float32 else x.float()
     x, stride = _point_stride(x)
     B, N = int(x.shape[0]), int(x.shape[1])
-    ws_bytes = int(_L().p3tok_knn_workspace_bytes(B, N)) if _KNN_SORTED and B > 0 else 0
+    ws_bytes = int(_L().p3tok_knn_workspace_bytes(B, N)) if B > 0 else 0
     ws = torch.empty(max(ws_bytes, 0), dtype=torch.uint8, device=x.device)
     if ws_bytes > 0:
         with torch.cuda.device(x.device), _timed("knn"):
@@ -337,41 +303,15 @@ def _ws_check(ws: torch.Tensor, x: torch.Tensor) -> None:
                            "call knn_prepare(x) again")
 
 
-@torch.library.custom_op("p3tok::fps_sorted", mutates_args=(), device_types="cuda")
-def fps_sorted(x: torch.Tensor, ws: torch.Tensor, start_idx: torch.Tensor, npoint: int) -> torch.Tensor:
-    """FPS indices (B,npoint) int64 of the clouds `x` from the workspace knn_prepare(x) filled (block-culled kernel)."""
-    _need_cuda("fps_sorted", x, ws, start_idx)
-    _ws_check(ws, x)
-    B, N = int(x.shape[0]), int(x.shape[1])
-    start = start_idx.to(torch.int64).contiguous()
-    if start.shape != (B,):
-        raise RuntimeError(f"p3tok::fps: start_idx must have shape ({B},)")
-    out = torch.empty((B, npoint), dtype=torch.int64, device=x.device)
-    with torch.cuda.device(x.device), _timed("fps"):
-        check(_L().p3tok_fps_sorted(ws.data_ptr(), int(ws.numel()), B, N, start.data_ptr(), npoint, out.data_ptr(), _stream()),
-              "fps_sorted")
-    return out
-
-
-@fps_sorted.register_fake
-def _(x, ws, start_idx, npoint):
-    return x.new_empty((x.shape[0], npoint), dtype=torch.int64)
-
-
 def fps_with_knn_prepare(x: torch.Tensor, start_idx: torch.Tensor, npoint: int) -> Tuple[torch.Tensor, torch.Tensor]:
     """(fps_idx, knn workspace): FPS on the current stream with the kNN preparation of the same clouds on a side stream
     (both are one-CTA-per-cloud kernels that leave most of every SM idle; the preparation does not need the centres).
     Fork / join by events, so the pair is capturable into a CUDA graph.  Measured (B200, same box): with one CTA per cloud
     in each kernel the pair helps only while the two grids fit side by side - c1 (B = 32) 0.319 -> 0.293 ms per step; at
     c2 (B = 128) the preparation's 1024-thread sort shares SMs with FPS, whose dependent iterations are the critical
-    path, and the step gets slower (0.972 -> 1.012 ms; c5 2.34 -> 2.38) - so "auto" overlaps only when 2 B <= #SMs.
-    P3TOK_OVERLAP=0 / 1 forces back-to-back / overlapped."""
+    path, and the step gets slower (0.972 -> 1.012 ms; c5 2.34 -> 2.38) - so the pair overlaps only when 2 B <= #SMs."""
     _need_cuda("fps_with_knn_prepare", x)         # before the stream calls below, which reject CPU devices
-    if _use_culled_fps(int(x.shape[0]), int(x.shape[1]), npoint):
-        # round 2: the preparation comes FIRST - FPS itself runs on the sorted blocks (p3tok_fps_sorted), then the kNN query
-        ws = knn_prepare(x)
-        return fps_sorted(x, ws, start_idx, npoint), ws
-    if _OVERLAP == "0" or (_OVERLAP != "1" and 2 * int(x.shape[0]) > _sm_count(x.device)):
+    if 2 * int(x.shape[0]) > _sm_count(x.device):
         return fps(x, start_idx, npoint), knn_prepare(x)
     cur = torch.cuda.current_stream(x.device)
     side = _side_stream(x.device)

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define P3TOK_ABI_VERSION 2
+#define P3TOK_ABI_VERSION 3
 
 #if defined(__GNUC__)
 #define P3TOK_API __attribute__((visibility("default")))
@@ -67,14 +67,6 @@ P3TOK_API int64_t p3tok_kernel_launches(void);
  * CTA) is chosen per launch so that all B clouds are resident at once (cudaOccupancyMaxActiveClusters). */
 P3TOK_API int p3tok_fps(const float* x, int64_t B, int64_t N, int64_t pt_stride, const int64_t* start_idx,
               int64_t G, int64_t* out_idx, void* stream);
-
-/* The same sampling for clouds of at most 8192 points on a workspace p3tok_knn_prepare has filled for these clouds
- * (below): the cloud is visited in 32-point blocks of a Z-order curve and a block is touched only when its running
- * distances can change (bounding-box lower bound of the computed distance vs the block's maximum), so an iteration costs
- * a box test per block instead of a pass over the cloud.  Same picks as p3tok_fps bit for bit (same distance arithmetic,
- * same lowest-original-index tie-break).  The modules prepare once and run FPS, then the kNN query, on the same workspace. */
-P3TOK_API int p3tok_fps_sorted(const void* workspace, int64_t workspace_bytes, int64_t B, int64_t N,
-                     const int64_t* start_idx, int64_t G, int64_t* out_idx, void* stream);
 
 /* farthest_point_sampling (src/models/pix4point.py:8-53) on D-dimensional points, 1 <= D <= 16: the reference sums the
  * squared differences over ALL D coordinates (line 44, torch.sum(..., dim=2)).  x: point p of cloud b at

@@ -1,4 +1,4 @@
-"""Scratch driver (not a test): device time of p3tok_fps alone.  usage: [P3TOK_FPS_PPT=n] python tests/_fps_time.py"""
+"""Scratch driver (not a test): device time of p3tok_fps alone.  usage: python tests/_fps_time.py"""
 import os
 import sys
 
@@ -19,8 +19,8 @@ for (B, N, G) in ((256, 8192, 2048), (148, 8192, 2048), (256, 4096, 1024), (128,
     for rep in range(4):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        out = ops.fps_sweep(x, st, G)
+        out = ops.fps(x, st, G)
         e1.record()
         torch.cuda.synchronize()
         ts.append(e0.elapsed_time(e1))
-    print(f"PPT={os.environ.get('P3TOK_FPS_PPT', 'auto'):>4s}  B={B:5d} N={N:6d} G={G:5d}: {min(ts):8.3f} ms  ({1e3 * min(ts) / G:.3f} us/iter)  checksum {int(out.sum())}")
+    print(f"B={B:5d} N={N:6d} G={G:5d}: {min(ts):8.3f} ms  ({1e3 * min(ts) / G:.3f} us/iter)  checksum {int(out.sum())}")

@@ -42,7 +42,7 @@ for B, N, D, G in ((32, 1024, 4, 256), (128, 2048, 6, 128), (32, 8192, 8, 512), 
     ms = timed(lambda: ops.fps_nd(x, st, G), reps=20)
     line = f"fps_nd B={B} N={N} D={D} G={G}: {ms:.3f} ms ({ms * 1e3 / G:.2f} us/iteration)"
     if D == 3:
-        line += f"; fps_kernel (xyz path) {timed(lambda: ops.fps_sweep(x, st, G), reps=20):.3f} ms"
+        line += f"; fps_kernel (xyz path) {timed(lambda: ops.fps(x, st, G), reps=20):.3f} ms"
     print(line)
 for B, S, N in ((128, 128, 2048), (16, 2048, 65536)):
     x = torch.from_numpy(synth.make_cloud("uniform", B, N, 2, 3)).to(dev)

@@ -200,8 +200,8 @@ def test_cuda_graph_replay_matches_eager():
 
 
 def test_fused_pair_kernel_matches_layerwise(monkeypatch, tmp_path):
-    """embed_fused.cu (two layers per kernel, hidden activation kept on-chip; opt-in via P3TOK_FUSED=1) against the
-    default layer-by-layer tensor-core path: same bf16 arithmetic, different accumulation grouping."""
+    """embed_fused.cu (two layers per kernel, hidden activation kept on-chip; the default) against the layer-by-layer
+    tensor-core path (P3TOK_FUSED=0): same bf16 arithmetic, different accumulation grouping."""
     _skip_if_unbuilt("bf16")
     import subprocess, sys, os
     code = (

@@ -401,16 +401,15 @@ def test_fps_many_iterations_bit_exact_near_ties():
         x = synth.make_cloud("uniform", B, N, 777, 3)
         st = synth.start_indices(B, N, 777)
         ref = oracle.fps(x, st, G)
-        for name, fn in (("fps", ops.fps), ("fps_sweep", ops.fps_sweep)):     # block-culled (N <= 8192) and sweep kernels
-            got = fn(to_dev(x), to_dev(st), G).cpu().numpy()
-            bad = np.argwhere(got != ref)
-            assert bad.size == 0, f"{name}: {len(bad)} picks differ; first at cloud {bad[0][0]} iteration {bad[0][1]}"
+        got = ops.fps(to_dev(x), to_dev(st), G).cpu().numpy()
+        bad = np.argwhere(got != ref)
+        assert bad.size == 0, f"{len(bad)} picks differ; first at cloud {bad[0][0]} iteration {bad[0][1]}"
 
 
-def test_culled_fps_equals_the_sweep_kernel_and_the_oracle():
-    """p3tok_fps_sorted (block-culled, on the Z-order sorted workspace) against p3tok_fps (every point, every iteration) and
-    the oracle: ragged N (partial last block, 1..8 warps, 8 / 16 / 32 slots per warp), G up to N and beyond, 3- and
-    4-channel rows, all cloud kinds incl. exact duplicates (ties resolved by the lowest ORIGINAL index)."""
+def test_fps_ragged_shapes_equal_the_oracle():
+    """p3tok_fps against the oracle: ragged N (partial last warp, 8 and 16 points per thread, up to the largest
+    single-CTA cloud), G up to N and beyond, 3- and 4-channel rows, all cloud kinds incl. exact duplicates (ties resolved
+    by the lowest index)."""
     rng = np.random.RandomState(7)
     kinds = ["uniform", "clustered", "duplicates"]
     shapes = [(3, 33, 33), (2, 100, 40), (4, 256, 64), (2, 257, 257), (3, 1000, 999), (2, 1024, 256), (2, 2048, 128), (2, 2049, 300),
@@ -421,11 +420,6 @@ def test_culled_fps_equals_the_sweep_kernel_and_the_oracle():
         if C == 4:
             x = np.concatenate([x, x[..., 1:2] - x[..., 1:2].min(1, keepdims=True)], -1).astype(np.float32)
         st = rng.randint(0, N, size=B).astype(np.int64)
-        xt, stt = to_dev(x), to_dev(st)
-        ws = ops.knn_prepare(xt)
-        a = ops.fps_sorted(xt, ws, stt, G).cpu().numpy()
-        b = ops.fps_sweep(xt, stt, G).cpu().numpy()
-        c = oracle.fps(x, st, G)
-        assert np.array_equal(a, c), (B, N, G, "culled vs oracle", np.argwhere(a != c)[:3])
-        assert np.array_equal(b, c), (B, N, G, "sweep vs oracle")
-        assert np.array_equal(ops.fps(xt, stt, G).cpu().numpy(), c)       # the dispatching op
+        got = ops.fps(to_dev(x), to_dev(st), G).cpu().numpy()
+        ref = oracle.fps(x, st, G)
+        assert np.array_equal(got, ref), (B, N, G, np.argwhere(got != ref)[:3])

@@ -66,7 +66,7 @@ def test_fps_nd_on_xyz_equals_the_tokenizers_fps_kernel():
         x = synth.make_cloud(kind, B, N, 17, 3)
         st = synth.start_indices(B, N, 17)
         a = ops.fps_nd(to_dev(x), to_dev(st), G).cpu().numpy()
-        b = ops.fps_sweep(to_dev(x), to_dev(st), G).cpu().numpy()
+        b = ops.fps(to_dev(x), to_dev(st), G).cpu().numpy()
         assert np.array_equal(a, b) and np.array_equal(a, oracle.fps(x, st, G))
 
 

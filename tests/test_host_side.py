@@ -27,7 +27,7 @@ def test_library_exports_every_declared_symbol(built):
         assert hasattr(L, n), n
     assert sorted(_lib._SIGNATURES) == names      # the Python binding covers the whole header
     L.p3tok_abi_version.restype = ctypes.c_int
-    assert L.p3tok_abi_version() == 2             # host-only call, no GPU needed
+    assert L.p3tok_abi_version() == 3             # host-only call, no GPU needed
 
 
 def test_host_only_size_queries(built):
