@@ -20,6 +20,8 @@
 //   p3tok_group_sum_f32             sum over the k rows of a group          gradient of the expanded global feature
 //   p3tok_scatter_rows_add_f32      gradient of the kNN gather: every point collects the gradients of all its rows
 //   p3tok_build_rows_f32            the gathered row matrix of p3tok_rows    (forward input of the training path)
+//   p3tok_apf_rows_bwd_f32          adjoint of the APF rows: gradient to the input points (neighbour and centre terms)
+//   p3tok_gather_points_bwd_f32     adjoint of p3tok_gather_points (index_points, fps, the centres)
 #include "embed.cuh"
 
 namespace p3tok {
@@ -231,6 +233,42 @@ __global__ void scatter_rows_add_kernel(const float* __restrict__ dRows, const i
   }
 }
 
+// adjoint of the APF rows (build_rows kind 0): output group bj reads input group g = perm[bj]; its row n is
+// [x[nbr] - x[ctr] || x[ctr]].  One thread per (output group, channel): d rel goes to the neighbour (one atomic per element),
+// sum_n (d ctr - d rel) is reduced over the group's k rows in a register and added to the centre with one atomic.
+template <typename IdxT>
+__global__ void apf_rows_bwd_kernel(const float* __restrict__ dRows, const int64_t* __restrict__ ctr_idx,
+                                    const IdxT* __restrict__ knn_idx, const int64_t* __restrict__ perm, int64_t N, int64_t G,
+                                    int k, int C, int64_t BG, float* __restrict__ dX) {
+  const int64_t total = BG * C;
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int c = (int)(e % C);
+    const int64_t bj = e / C;
+    const int64_t b = bj / G;
+    const int64_t g = perm ? perm[bj] : (bj - b * G);
+    const IdxT* nbr = knn_idx + (b * G + g) * k;
+    const float* d = dRows + bj * k * 2 * C + c;
+    float acc = 0.f;
+    for (int n = 0; n < k; ++n) {
+      const float drel = d[(int64_t)n * 2 * C], dctr = d[(int64_t)n * 2 * C + C];
+      atomicAdd(&dX[(b * N + (int64_t)nbr[n]) * C + c], drel);
+      acc += dctr - drel;
+    }
+    atomicAdd(&dX[(b * N + ctr_idx[b * G + g]) * C + c], acc);
+  }
+}
+
+// adjoint of gather_points: dX[b, idx[b,s], c] += dOut[b, s, c]
+__global__ void gather_points_bwd_kernel(const float* __restrict__ dOut, int64_t N, int C, const int64_t* __restrict__ idx,
+                                         int64_t S, int64_t total, float* __restrict__ dX) {
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int c = (int)(e % C);
+    const int64_t bs = e / C;
+    const int64_t b = bs / S;
+    atomicAdd(&dX[(b * N + idx[bs]) * C + c], dOut[e]);
+  }
+}
+
 }  // namespace p3tok
 
 using namespace p3tok;
@@ -362,4 +400,34 @@ extern "C" int p3tok_build_rows_f32(const p3tok_rows* rows, float* X, void* stre
   P3_REQUIRE(rows->kind != 0 || rows->ctr_idx, P3TOK_ERR_INVALID, "build_rows_f32: APF rows need ctr_idx");
   P3_REQUIRE(rows->kind != 1 || rows->feats, P3TOK_ERR_INVALID, "build_rows_f32: P4P rows need feats");
   return build_rows_f32(rows, 0, rows->B * rows->G, X, as_stream(stream));
+}
+
+extern "C" int p3tok_apf_rows_bwd_f32(const p3tok_rows* rows, const float* dRows, float* dX, void* stream) {
+  P3_REQUIRE(rows && rows->kind == 0, P3TOK_ERR_INVALID, "apf_rows_bwd_f32: APF (kind 0) rows expected");
+  P3_REQUIRE(rows->B >= 0 && rows->N > 0 && rows->G >= 0 && rows->k > 0 && rows->k < (1 << 30) && rows->C > 0,
+             P3TOK_ERR_INVALID, "apf_rows_bwd_f32: bad shape");
+  P3_REQUIRE(rows->idx_dtype == P3TOK_I64 || rows->idx_dtype == P3TOK_I32, P3TOK_ERR_INVALID, "apf_rows_bwd_f32: bad idx_dtype");
+  const int64_t BG = rows->B * rows->G;
+  if (BG == 0) return P3TOK_OK;
+  P3_REQUIRE(dRows && dX && rows->ctr_idx && rows->knn_idx, P3TOK_ERR_INVALID, "apf_rows_bwd_f32: null pointer");
+  cudaStream_t s = as_stream(stream);
+  if (rows->idx_dtype == P3TOK_I64)
+    apf_rows_bwd_kernel<int64_t><<<tr_grid(BG * rows->C, 256), 256, 0, s>>>(
+        dRows, rows->ctr_idx, static_cast<const int64_t*>(rows->knn_idx), rows->perm, rows->N, rows->G, (int)rows->k, rows->C, BG, dX);
+  else
+    apf_rows_bwd_kernel<int32_t><<<tr_grid(BG * rows->C, 256), 256, 0, s>>>(
+        dRows, rows->ctr_idx, static_cast<const int32_t*>(rows->knn_idx), rows->perm, rows->N, rows->G, (int)rows->k, rows->C, BG, dX);
+  P3_LAUNCH_CHECK("apf_rows_bwd_kernel");
+  return P3TOK_OK;
+}
+
+extern "C" int p3tok_gather_points_bwd_f32(const float* dOut, int64_t B, int64_t N, int64_t C, const int64_t* idx, int64_t S, float* dX,
+                                           void* stream) {
+  P3_REQUIRE(B >= 0 && N > 0 && C > 0 && S >= 0, P3TOK_ERR_INVALID, "gather_points_bwd_f32: bad shape");
+  const int64_t total = B * S * C;
+  if (total == 0) return P3TOK_OK;
+  P3_REQUIRE(dOut && idx && dX, P3TOK_ERR_INVALID, "gather_points_bwd_f32: null pointer");
+  gather_points_bwd_kernel<<<tr_grid(total, 256), 256, 0, as_stream(stream)>>>(dOut, N, (int)C, idx, S, total, dX);
+  P3_LAUNCH_CHECK("gather_points_bwd_kernel");
+  return P3TOK_OK;
 }

@@ -84,6 +84,8 @@ _SIGNATURES = {
     "p3tok_group_sum_f32": (_int, [_vp, _i64, _i64, _i64, _vp, _vp]),
     "p3tok_scatter_rows_add_f32": (_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _vp, _vp, _vp]),
     "p3tok_build_rows_f32": (_int, [ctypes.POINTER(RowsStruct), _vp, _vp]),
+    "p3tok_apf_rows_bwd_f32": (_int, [ctypes.POINTER(RowsStruct), _vp, _vp, _vp]),
+    "p3tok_gather_points_bwd_f32": (_int, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _vp]),
     "p3tok_ln_fwd_f32": (_int, [_vp, _i64, _i64, _vp, _vp, _f32, _vp, _vp, _vp, _vp]),
     "p3tok_ln_bwd_f32": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _int, _vp, _vp]),
     "p3tok_ln_param_grad_f32": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),

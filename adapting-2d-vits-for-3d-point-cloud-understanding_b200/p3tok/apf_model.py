@@ -23,7 +23,7 @@ import torch
 from torch import nn
 
 from . import fold, ops
-from .modules import PointNet
+from .modules import PointNet, wants_input_grad
 
 
 class _Mlp(nn.Module):
@@ -218,9 +218,9 @@ class ClassificationHead(nn.Module):
         return w.float().contiguous(), b.float().contiguous()
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
-        if self.training:
+        if self.training or wants_input_grad(x):         # eval mode + gradient wanted: running statistics, dropout off
             from . import train_vit
-            return train_vit.head_train(self, x, sync=bool(getattr(self, "sync_bn", False)))
+            return train_vit.head_train(self, x, sync=bool(getattr(self, "sync_bn", False)), running=not self.training)
         m = self.mlp_head
         x = x.float().contiguous()
         for lin, bn, relu in ((m[0], m[1], True), (m[4], m[5], True), (m[8], None, False)):

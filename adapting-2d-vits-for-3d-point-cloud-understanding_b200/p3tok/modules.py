@@ -8,9 +8,13 @@ The parameter containers (Conv1d/BatchNorm1d/... inside nn.Sequential at the ref
 indices) exist so reference checkpoints load with strict=True; forward never calls them.
 eval():  BatchNorm uses the running statistics, folded into the weights (p3tok/fold.py); `precision` selects
          "fp32" (CUDA-core FFMA, rtol 1e-4 contract) or "bf16" (tcgen05 tensor cores, rtol 1e-2 contract).
+eval() with a gradient wanted for the input (grad mode on and the input requires grad, `wants_input_grad`): the fp32
+         autograd path of train() with running-statistics BatchNorm - buffers untouched, nothing all-reduced - so x.grad
+         (and the gradient of every parameter that requires one) is filled as with the reference; fp32 tokens whatever
+         `precision` / `token_dtype` say.  Every other eval-mode call runs the serving kernels above.
 train(): batch-statistics BatchNorm (running estimates updated like nn.BatchNorm) and autograd through both
-         max-pools, the concat and the gather - p3tok/train.py over csrc/train.cu, fp32 (SURVEY.md 8f "next" #4);
-         `sync_bn=True` all-reduces the BatchNorm sums when the batch is sharded over ranks.
+         max-pools, the concat and the gather to the input points - p3tok/train.py over csrc/train.cu, fp32 (SURVEY.md 8f
+         "next" #4); `sync_bn=True` all-reduces the BatchNorm sums when the batch is sharded over ranks.
 """
 from __future__ import annotations
 
@@ -41,6 +45,13 @@ def _check_token_dtype(token_dtype, precision: str) -> bool:
     if precision != "bf16":
         raise ValueError("token_dtype=torch.bfloat16 needs precision='bf16'")
     return True
+
+
+def wants_input_grad(*inputs: Optional[torch.Tensor]) -> bool:
+    """An eval-mode module takes the fp32 autograd path (running-statistics BatchNorm) only when a gradient is wanted for one of
+    its inputs - grad mode on and the input requires grad (the rule of apf_model._wants_autograd).  Any other eval-mode call,
+    whatever `requires_grad` the parameters carry, runs the serving kernels."""
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs)
 
 
 def _bn_eps(module: nn.Module):
@@ -136,9 +147,9 @@ class Encoder(nn.Module, _FoldedMixin):
 
     def forward(self, point_groups: torch.Tensor) -> torch.Tensor:
         B, G, k, cin = point_groups.shape
-        if self.training:                       # batch-statistics BatchNorm + autograd (p3tok/train.py), fp32
+        if self.training or wants_input_grad(point_groups):   # autograd (p3tok/train.py), fp32; eval: running statistics
             rows = point_groups.float().reshape(B * G * k, cin)
-            return train.encoder_train(self, rows, k, self.sync_bn).view(B, G, self.encoder_channel)
+            return train.encoder_train(self, rows, k, self.sync_bn, not self.training).view(B, G, self.encoder_channel)
         m = self.folded(point_groups.device)
         rows = point_groups.float().reshape(B * G * k, cin)
         tok = ops.patch_embed(_lib.ROWS_DIRECT, rows, None, None, None, None, B * G, k, m.tensors(), m.meta(),
@@ -166,9 +177,11 @@ class PointNet(nn.Module):
         G, k = self.group.num_group, self.group.group_size
         with torch.no_grad():
             fps_idx, _, knn_idx, perm = self.group.indices(x, start_idx)
-        if self.encoder.training:               # train mode: the gathered rows feed the batch-statistics Encoder (p3tok/train.py)
+        if self.encoder.training or wants_input_grad(x):
+            # autograd: the gathered rows (differentiable with respect to x) feed the Encoder - batch statistics in train mode,
+            # running statistics in eval mode (p3tok/train.py)
             rows = train.apf_rows(x, fps_idx, knn_idx, perm)
-            return train.encoder_train(self.encoder, rows, k, self.encoder.sync_bn).view(B, G, -1)
+            return train.encoder_train(self.encoder, rows, k, self.encoder.sync_bn, not self.encoder.training).view(B, G, -1)
         m = self.encoder.folded(x.device)
         if m.cin != 2 * C:
             raise RuntimeError(f"PointNet: in_channel={m.cin} but input has C={C} (expects in_channel == 2*C)")
@@ -225,8 +238,8 @@ class P3Embed(nn.Module, _FoldedMixin):
 
     def forward(self, p: torch.Tensor, f: torch.Tensor, start_idx: Optional[List[torch.Tensor]] = None
                 ) -> Tuple[List[torch.Tensor], List[torch.Tensor]]:
-        if self.training:
-            return self._forward_train(p, f, start_idx)
+        if self.training or wants_input_grad(p, f):
+            return self._forward_train(p, f, start_idx, running=not self.training)
         bf16 = _check_precision(self.precision)
         B, N = int(p.shape[0]), int(p.shape[1])
         out_p, out_f = [p], [f]
@@ -250,9 +263,10 @@ class P3Embed(nn.Module, _FoldedMixin):
         return out_p, out_f
 
 
-def _p3embed_forward_train(self, p, f, start_idx=None):
-    """P3Embed.forward in train mode (pix4point.py:166-191): index ops without gradient, differentiable gather of the rows
-    (points and features collect the gradients of every neighbourhood they appear in), batch-statistics stage MLP."""
+def _p3embed_forward_train(self, p, f, start_idx=None, running=False):
+    """P3Embed.forward under autograd (pix4point.py:166-191): index ops without gradient, differentiable gather of the rows
+    (points and features collect the gradients of every neighbourhood they appear in), stage MLP with batch-statistics
+    BatchNorm (train mode) or, running=True, the running estimates (eval mode with a gradient wanted for p or f)."""
     B, N = int(p.shape[0]), int(p.shape[1])
     out_p, out_f = [p], [f]
     pts = p.float()
@@ -268,7 +282,7 @@ def _p3embed_forward_train(self, p, f, start_idx=None):
             kidx = ops.knn_query(pd, ws, ctr_nd, self.k, _lib.KNN_P4P_CDIST, True)
         ctr = torch.gather(pts, 1, cidx.unsqueeze(-1).expand(-1, -1, 3))     # pix4point.py:176 (differentiable like the reference)
         rows = train.GatherRowsFn.apply(pts.contiguous(), feat.contiguous(), kidx)
-        tok = train.p3stage_train(conv1, conv2, rows, self.k, self.sync_bn)
+        tok = train.p3stage_train(conv1, conv2, rows, self.k, self.sync_bn, running)
         feat = tok.view(B, G, -1)
         pts = ctr
         out_p.append(ctr)

@@ -2,9 +2,10 @@
 
 Each op validates its tensors (CUDA, dtype, contiguity), allocates the outputs with torch (the
 library owns no memory), and enqueues the kernels on torch's current stream.  Shape-only "fake"
-implementations are registered so the ops trace under torch.export / FakeTensor; there is no
-autograd registration (forward / inference path; indices are not differentiable) and no
-implementation for any device but CUDA.
+implementations are registered so the ops trace under torch.export / FakeTensor.  The three gathers
+(gather_points, apf_group, group_gather) are differentiable with respect to their point / feature
+inputs through adjoint ops of their own; every other op is a forward / inference op (indices are not
+differentiable).  There is no implementation for any device but CUDA.
 """
 from __future__ import annotations
 
@@ -409,6 +410,151 @@ def group_gather(pnts: torch.Tensor, feats: torch.Tensor, idx: torch.Tensor) -> 
 def _(pnts, feats, idx):
     B, G, k = idx.shape
     return pnts.new_empty((B, G, k, 3)), pnts.new_empty((B, G, k, feats.shape[-1]))
+
+
+# ------------------------------------------------------------------------------- gradients of the gathers
+# gather_points, apf_group and group_gather are differentiable with respect to their point / feature inputs, as the
+# reference's index_points and advanced-index gathers are (sampler.py:77-94, apf.py:70-95, pix4point.py:92-102); index inputs
+# get no gradient.  Each adjoint is an op of its own over csrc/train.cu; it scatters with fp32 atomic adds, so the gradient
+# is reproducible to rounding, not bit for bit.
+@torch.library.custom_op("p3tok::gather_points_bwd", mutates_args=(), device_types="cuda")
+def gather_points_bwd(grad: torch.Tensor, idx: torch.Tensor, N: int) -> torch.Tensor:
+    """grad (*idx.shape, C) -> dX (B,N,C): the adjoint of gather_points (p3tok_gather_points_bwd_f32)."""
+    _need_cuda("gather_points_bwd", grad, idx)
+    g = grad.float().contiguous()
+    B, C = int(idx.shape[0]), int(g.shape[-1])
+    flat = idx.to(torch.int64).reshape(B, -1).contiguous()
+    dx = torch.zeros((B, N, C), dtype=torch.float32, device=g.device)
+    with torch.cuda.device(g.device), _timed("gather_bwd"):
+        check(_L().p3tok_gather_points_bwd_f32(g.data_ptr(), B, N, C, flat.data_ptr(), int(flat.shape[1]), dx.data_ptr(), _stream()),
+              "gather_points_bwd")
+    return dx
+
+
+@gather_points_bwd.register_fake
+def _(grad, idx, N):
+    return grad.new_empty((idx.shape[0], N, grad.shape[-1]), dtype=torch.float32)
+
+
+def _gather_points_setup(ctx, inputs, output):
+    x, idx = inputs
+    ctx.save_for_backward(idx)
+    ctx.N = int(x.shape[1])
+
+
+def _gather_points_backward(ctx, grad):
+    (idx,) = ctx.saved_tensors
+    return gather_points_bwd(grad, idx, ctx.N), None
+
+
+gather_points.register_autograd(_gather_points_backward, setup_context=_gather_points_setup)
+
+
+def apf_rows_descriptor(B: int, N: int, C: int, fps_idx: torch.Tensor, knn_idx: torch.Tensor, perm: Optional[torch.Tensor]):
+    """(p3tok_rows of kind 0 over these indices, the index tensors it points into).  knn_idx stays int32 or int64."""
+    ci = fps_idx.to(torch.int64).contiguous()
+    kn = (knn_idx if knn_idx.dtype in (torch.int32, torch.int64) else knn_idx.to(torch.int64)).contiguous()
+    pm = perm.to(torch.int64).contiguous() if perm is not None else None
+    r = _lib.RowsStruct()
+    r.kind, r.C, r.D, r.idx_dtype = _lib.ROWS_APF, C, 0, _lib.I32 if kn.dtype == torch.int32 else _lib.I64
+    r.B, r.N, r.G, r.k = B, N, int(kn.shape[1]), int(kn.shape[2])
+    r.ctr_idx, r.knn_idx, r.perm = ci.data_ptr(), kn.data_ptr(), _ptr(pm)
+    return r, (ci, kn, pm)
+
+
+@torch.library.custom_op("p3tok::apf_group_bwd", mutates_args=(), device_types="cuda")
+def apf_group_bwd(grad_neigh: Optional[torch.Tensor], grad_center: Optional[torch.Tensor], fps_idx: torch.Tensor,
+                  knn_idx: torch.Tensor, perm: Optional[torch.Tensor], N: int, C: int) -> torch.Tensor:
+    """The adjoint of apf_group -> dX (B,N,C): the neighbourhood rows through p3tok_apf_rows_bwd_f32, the centres (xyz of
+    x[b, fps_idx[b, perm[b,j]]]) through p3tok_gather_points_bwd_f32.  Either gradient may be None."""
+    _need_cuda("apf_group_bwd", grad_neigh, grad_center, fps_idx, knn_idx, perm)
+    B, G = int(knn_idx.shape[0]), int(knn_idx.shape[1])
+    dx = torch.zeros((B, N, C), dtype=torch.float32, device=fps_idx.device)
+    L = _L()
+    with torch.cuda.device(dx.device), _timed("apf_group_bwd"):
+        if grad_neigh is not None:
+            g = grad_neigh.float().contiguous()
+            r, keep = apf_rows_descriptor(B, N, C, fps_idx, knn_idx, perm)
+            check(L.p3tok_apf_rows_bwd_f32(ctypes.byref(r), g.data_ptr(), dx.data_ptr(), _stream()), "apf_rows_bwd_f32")
+            del keep
+        if grad_center is not None:
+            src = fps_idx.to(torch.int64)
+            src = (torch.gather(src, 1, perm.to(torch.int64)) if perm is not None else src).contiguous()
+            gc = grad_center.float()
+            if C != 3:                                     # the centres are channels 0..2 of the gathered rows
+                gc = torch.nn.functional.pad(gc, (0, C - 3))
+            gc = gc.contiguous()
+            check(L.p3tok_gather_points_bwd_f32(gc.data_ptr(), B, N, C, src.data_ptr(), G, dx.data_ptr(), _stream()),
+                  "gather_points_bwd")
+    return dx
+
+
+@apf_group_bwd.register_fake
+def _(grad_neigh, grad_center, fps_idx, knn_idx, perm, N, C):
+    return fps_idx.new_empty((knn_idx.shape[0], N, C), dtype=torch.float32)
+
+
+def _apf_group_setup(ctx, inputs, output):
+    x, fps_idx, knn_idx, perm = inputs
+    ctx.set_materialize_grads(False)                       # an unused output (often `center`) costs no scatter
+    ctx.save_for_backward(fps_idx, knn_idx, perm)
+    ctx.N, ctx.C = int(x.shape[1]), int(x.shape[2])
+
+
+def _apf_group_backward(ctx, grad_neigh, grad_center):
+    fps_idx, knn_idx, perm = ctx.saved_tensors
+    if grad_neigh is None and grad_center is None:
+        return None, None, None, None
+    return apf_group_bwd(grad_neigh, grad_center, fps_idx, knn_idx, perm, ctx.N, ctx.C), None, None, None
+
+
+apf_group.register_autograd(_apf_group_backward, setup_context=_apf_group_setup)
+
+
+@torch.library.custom_op("p3tok::group_gather_bwd", mutates_args=(), device_types="cuda")
+def group_gather_bwd(grad_p: Optional[torch.Tensor], grad_f: Optional[torch.Tensor], idx: torch.Tensor, N: int, D: int,
+                     need_p: bool, need_f: bool) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The adjoint of group_gather through p3tok_scatter_rows_add_f32 -> (dP (B,N,3), dF (B,N,D)); an output not asked for
+    (need_p / need_f False) is returned empty."""
+    _need_cuda("group_gather_bwd", grad_p, grad_f, idx)
+    B, G, k = (int(v) for v in idx.shape)
+    dev = idx.device
+    gp = grad_p.float() if grad_p is not None else torch.zeros((B, G, k, 3), dtype=torch.float32, device=dev)
+    gf = grad_f.float() if grad_f is not None else torch.zeros((B, G, k, D), dtype=torch.float32, device=dev)
+    drows = torch.cat([gp, gf], -1).contiguous()           # the (B,G,k,3+D) row layout of the scatter
+    i32 = idx.to(torch.int32).contiguous()
+    dp = torch.zeros((B, N, 3) if need_p else (0,), dtype=torch.float32, device=dev)
+    df = torch.zeros((B, N, D) if need_f else (0,), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev), _timed("group_gather_bwd"):
+        check(_L().p3tok_scatter_rows_add_f32(drows.data_ptr(), i32.data_ptr(), B, N, G, k, D, dp.data_ptr() if need_p else None,
+                                              df.data_ptr() if need_f else None, _stream()), "scatter_rows_add_f32")
+    return dp, df
+
+
+@group_gather_bwd.register_fake
+def _(grad_p, grad_f, idx, N, D, need_p, need_f):
+    B = idx.shape[0]
+    return (idx.new_empty((B, N, 3) if need_p else (0,), dtype=torch.float32),
+            idx.new_empty((B, N, D) if need_f else (0,), dtype=torch.float32))
+
+
+def _group_gather_setup(ctx, inputs, output):
+    pnts, feats, idx = inputs
+    ctx.set_materialize_grads(False)
+    ctx.save_for_backward(idx)
+    ctx.N, ctx.D = int(pnts.shape[1]), int(feats.shape[-1])
+
+
+def _group_gather_backward(ctx, grad_p, grad_f):
+    (idx,) = ctx.saved_tensors
+    need_p, need_f = bool(ctx.needs_input_grad[0]), bool(ctx.needs_input_grad[1])
+    if (grad_p is None and grad_f is None) or not (need_p or need_f):
+        return None, None, None
+    dp, df = group_gather_bwd(grad_p, grad_f, idx, ctx.N, ctx.D, need_p, need_f)
+    return (dp if need_p else None), (df if need_f else None), None
+
+
+group_gather.register_autograd(_group_gather_backward, setup_context=_group_gather_setup)
 
 
 # ------------------------------------------------------------------------------------- patch embed

@@ -20,7 +20,7 @@ from torch import nn
 
 from . import ops
 from .apf_model import bf16_layer, check_block_precision, x3_layer
-from .modules import PointViTTokens
+from .modules import PointViTTokens, wants_input_grad
 
 
 class _Attn(nn.Module):
@@ -173,8 +173,8 @@ class ClsHead(nn.Module):
 
     def forward(self, end_points: torch.Tensor) -> torch.Tensor:
         from . import train_vit
-        if self.training:
-            return train_vit.head_train(self, end_points)
+        if self.training or wants_input_grad(end_points):   # eval mode + gradient wanted: running statistics, dropout off
+            return train_vit.head_train(self, end_points, running=not self.training)
         blocks, last = train_vit.mlp_head_blocks(self.head)
         x = end_points.float().contiguous()
         for lin, bn, _ in blocks:

@@ -12,9 +12,14 @@ Sharded batches: BatchNorm couples the clouds of a batch, so with the batch spli
 sum x, sum x^2, row count; backward: sum dy, sum dy*xhat) are all-reduced - the ONE collective the path has (`sync_bn=True`
 on the module, torch.distributed initialised).  Weight gradients are per-rank partial sums, reduced by the caller (DDP).
 
+Running-statistics mode (`running` on the Functions, `running=True` on encoder_train / p3stage_train): the same Functions for
+eval-mode modules whose input wants a gradient (adversarial attacks, saliency) - nn.BatchNorm's eval semantics (running mean /
+variance, no update, no all-reduce), and the weight-gradient products of parameters that do not require grad are skipped.
+ApfRowsFn builds the APF rows and sends their gradient back to the input points.
+
 fp32 on CUDA cores; per-channel sums in fp64.  The eval-mode (serving) path is the tensor-core one; this path exists so that
-the kernels can replace the reference inside its trainers.  Opt-in: P3TOK_TRAIN_TC=1 (or `set_tensor_core_gemms(1)`) sends the
-forward and dX products through the fp32-accurate bf16x3 tensor-core GEMM (`p3tok_linear_x3_f32`: operands split into bf16
+the kernels can replace the reference inside its trainers and wherever the reference is differentiated.  Opt-in:
+P3TOK_TRAIN_TC=1 (or `set_tensor_core_gemms(1)`) sends the forward and dX products through the fp32-accurate bf16x3 tensor-core GEMM (`p3tok_linear_x3_f32`: operands split into bf16
 hi + lo, three partial products in one tcgen05 GEMM, fp32 accumulate, ~1e-5 of max); the weight-gradient products stay on CUDA
 cores.  The fp32 CUDA-core SGEMMs stay the default: they are what the 1e-4 parity tests pin.
 """
@@ -26,7 +31,7 @@ from typing import List, Optional, Tuple
 
 import torch
 
-from . import _lib
+from . import _lib, ops
 from ._lib import check
 
 
@@ -145,10 +150,15 @@ def group_sum(x: torch.Tensor, k: int) -> torch.Tensor:
 
 
 class BNState:
-    """Batch statistics of one BatchNorm application: what forward normalised with and what backward needs."""
+    """Statistics of one BatchNorm application: what forward normalised with and what backward needs.  count is None in the
+    running-statistics mode (eval-mode BatchNorm: the statistics are constants, not functions of the batch)."""
 
     def __init__(self, mean, rstd, count, var_unbiased, mean64):
         self.mean, self.rstd, self.count, self.var_unbiased, self.mean64 = mean, rstd, count, var_unbiased, mean64
+
+    @property
+    def running(self) -> bool:
+        return self.count is None
 
 
 def _all_reduce(t: torch.Tensor, sync: bool) -> torch.Tensor:
@@ -167,37 +177,55 @@ def combine_stats(s: torch.Tensor, q: torch.Tensor, count: float, eps: float):
     return mean, rstd, var * (count / max(count - 1.0, 1.0))
 
 
-def bn_forward(z: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, relu: bool, sync: bool) -> Tuple[torch.Tensor, BNState]:
-    s, q = colstats(z)
+def bn_forward(z: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, relu: bool, sync: bool,
+               running: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> Tuple[torch.Tensor, BNState]:
+    """act(BatchNorm(z)) on rows.  running=None: batch statistics (train mode, all-reduced with sync); running=(running_mean,
+    running_var): eval-mode BatchNorm - normalise with the module's running estimates, no reduction, nothing all-reduced."""
     M, N = z.shape
-    packed = _all_reduce(torch.cat([s, q, torch.tensor([float(M)], dtype=torch.float64, device=z.device)]), sync)
-    s, q = packed[:N], packed[N:2 * N]
-    count = float(packed[2 * N].item()) if sync else float(M)
-    mean64, rstd64, var_unb = combine_stats(s, q, count, eps)
-    mean, rstd = mean64.float(), rstd64.float()
+    if running is not None:
+        mean64 = _f32(running[0]).double()
+        mean, rstd = mean64.float(), (1.0 / torch.sqrt(_f32(running[1]).double() + eps)).float()
+        st = BNState(mean, rstd, None, None, mean64)
+    else:
+        s, q = colstats(z)
+        packed = _all_reduce(torch.cat([s, q, torch.tensor([float(M)], dtype=torch.float64, device=z.device)]), sync)
+        s, q = packed[:N], packed[N:2 * N]
+        count = float(packed[2 * N].item()) if sync else float(M)
+        mean64, rstd64, var_unb = combine_stats(s, q, count, eps)
+        st = BNState(mean64.float(), rstd64.float(), count, var_unb, mean64)
     y = torch.empty_like(z)
     g, b = _f32(gamma), _f32(beta)
     with torch.cuda.device(z.device):
-        check(_L().p3tok_bn_act_f32(z.data_ptr(), M, N, mean.data_ptr(), rstd.data_ptr(), g.data_ptr(), b.data_ptr(), int(relu),
+        check(_L().p3tok_bn_act_f32(z.data_ptr(), M, N, st.mean.data_ptr(), st.rstd.data_ptr(), g.data_ptr(), b.data_ptr(), int(relu),
                                     y.data_ptr(), _s()), "bn_act_f32")
-    return y, BNState(mean, rstd, count, var_unb, mean64)
+    return y, st
 
 
-def bn_backward(dy: torch.Tensor, z: torch.Tensor, st: BNState, gamma: torch.Tensor, beta: torch.Tensor, relu: bool, sync: bool):
-    """-> (dz, dgamma, dbeta) for dy = dL/d(act(BN(z)))."""
+def bn_backward(dy: torch.Tensor, z: torch.Tensor, st: BNState, gamma: torch.Tensor, beta: torch.Tensor, relu: bool, sync: bool,
+                want_params: bool = True):
+    """-> (dz, dgamma, dbeta) for dy = dL/d(act(BN(z))).  In the running-statistics mode dz = gamma rstd dy' (the apply kernel
+    with both sums zero), and dgamma / dbeta (the sums of dy' xhat and dy') are computed only when want_params."""
     dy = _f32(dy)
     M, N = z.shape
     g, b = _f32(gamma), _f32(beta)
-    s12 = torch.empty(2 * N, dtype=torch.float64, device=z.device)
+    stats = not st.running or want_params
+    s12 = (torch.empty if stats else torch.zeros)(2 * N, dtype=torch.float64, device=z.device)
+    local = None
     with torch.cuda.device(z.device):
-        check(_L().p3tok_bn_bwd_stats_f32(dy.data_ptr(), z.data_ptr(), M, N, st.mean.data_ptr(), st.rstd.data_ptr(), g.data_ptr(),
-                                          b.data_ptr(), int(relu), s12.data_ptr(), s12.data_ptr() + 8 * N, _s()), "bn_bwd_stats_f32")
-        local = s12.clone()
-        _all_reduce(s12, sync)
+        if stats:
+            check(_L().p3tok_bn_bwd_stats_f32(dy.data_ptr(), z.data_ptr(), M, N, st.mean.data_ptr(), st.rstd.data_ptr(), g.data_ptr(),
+                                              b.data_ptr(), int(relu), s12.data_ptr(), s12.data_ptr() + 8 * N, _s()), "bn_bwd_stats_f32")
+            local = s12.clone()
+            if st.running:
+                s12.zero_()
+        if not st.running:
+            _all_reduce(s12, sync)
         dz = torch.empty_like(z)
-        check(_L().p3tok_bn_bwd_apply_f32(dy.data_ptr(), z.data_ptr(), M, N, int(round(st.count)), st.mean.data_ptr(), st.rstd.data_ptr(),
-                                          g.data_ptr(), b.data_ptr(), int(relu), s12.data_ptr(), s12.data_ptr() + 8 * N, dz.data_ptr(),
-                                          _s()), "bn_bwd_apply_f32")
+        check(_L().p3tok_bn_bwd_apply_f32(dy.data_ptr(), z.data_ptr(), M, N, 1 if st.running else int(round(st.count)), st.mean.data_ptr(),
+                                          st.rstd.data_ptr(), g.data_ptr(), b.data_ptr(), int(relu), s12.data_ptr(), s12.data_ptr() + 8 * N,
+                                          dz.data_ptr(), _s()), "bn_bwd_apply_f32")
+    if local is None:
+        return dz, None, None
     # parameter gradients stay per-rank partial sums (the caller's gradient all-reduce, e.g. DDP, sums them)
     return dz, local[N:].float(), local[:N].float()
 
@@ -211,114 +239,136 @@ def _t(w: torch.Tensor) -> torch.Tensor:
 
 
 # ------------------------------------------------------------------------------------------------ APF Encoder
+def _running(i: int, running):
+    return None if running is None else running[i]
+
+
+def _with_stats(ctx, out: torch.Tensor, stats) -> tuple:
+    """(out, mean, unbiased variance per BatchNorm) in train mode; (out,) in the running-statistics mode."""
+    outs = [out]
+    for st in stats:
+        if not st.running:
+            outs += [st.mean64.float(), st.var_unbiased.float()]
+    ctx.mark_non_differentiable(*outs[1:])
+    return tuple(outs)
+
+
+def running_stats(bns) -> tuple:
+    """((running_mean, running_var), ...) of eval-mode BatchNorm modules (the running-statistics mode of the Functions)."""
+    return tuple((bn.running_mean, bn.running_var) for bn in bns)
+
+
+def _grad_if(need: bool, fn):
+    """fn() when the gradient is wanted: the weight-gradient products of frozen parameters are never computed."""
+    return fn() if need else None
+
+
 class EncoderTrainFn(torch.autograd.Function):
-    """Encoder.get_features in train mode (apf.py:145-169).  inputs: rows (M, cin) with M = groups * k, then the 16
-    parameter tensors in state_dict order of first_conv.{0,1,3,4,6}, second_conv.{0,1,3} (running buffers excluded).
-    Returns (tokens (groups, E), batch mean / unbiased variance of the three BatchNorms for the running-estimate update)."""
+    """Encoder.get_features under autograd (apf.py:145-169).  inputs: rows (M, cin) with M = groups * k, k, the three BatchNorm
+    eps, sync, running, then the 16 parameter tensors in state_dict order of first_conv.{0,1,3,4,6}, second_conv.{0,1,3}.
+    running=None: train mode (batch statistics); running = ((running_mean, running_var) x 3): eval-mode BatchNorm.
+    Returns (tokens (groups, E), batch mean / unbiased variance of the three BatchNorms for the running-estimate update); in the
+    running mode, where nothing is updated, (tokens,)."""
 
     @staticmethod
-    def forward(ctx, rows, k, eps, sync, W1, b1, g1, be1, W2, b2, g2, be2, W3, b3, W4, b4, g4, be4, W5, b5):
+    def forward(ctx, rows, k, eps, sync, running, W1, b1, g1, be1, W2, b2, g2, be2, W3, b3, W4, b4, g4, be4, W5, b5):
         rows = _f32(rows)
         W1m, W2m, W3m, W4m, W5m = (_w2(w) for w in (W1, W2, W3, W4, W5))
         E = W3m.shape[0]
         z1 = linear(rows, W1m, b1)
-        h1, s1 = bn_forward(z1, g1, be1, eps[0], True, sync)
+        h1, s1 = bn_forward(z1, g1, be1, eps[0], True, sync, _running(0, running))
         z2 = linear(h1, W2m, b2)
-        h2, s2 = bn_forward(z2, g2, be2, eps[1], True, sync)
+        h2, s2 = bn_forward(z2, g2, be2, eps[1], True, sync, _running(1, running))
         ft = linear(h2, W3m, b3)
         gl, arg_g = group_max_arg(ft, k)                           # apf.py:160
         W4g, W4f = W4m[:, :E].contiguous(), W4m[:, E:].contiguous()
         gb = linear(gl, W4g, b4)                                   # the expanded global half of the concat, once per group
         z4 = linear(ft, W4f, None, gb, k)                          # apf.py:162-163 without the (M, 2E) concat tensor
-        h4, s4 = bn_forward(z4, g4, be4, eps[2], True, sync)
+        h4, s4 = bn_forward(z4, g4, be4, eps[2], True, sync, _running(2, running))
         o = linear(h4, W5m, b5)
         tok, arg_o = group_max_arg(o, k)                           # apf.py:167
         ctx.k, ctx.sync, ctx.E = k, sync, E
         ctx.stats = (s1, s2, s4)
-        ctx.need_input = rows.requires_grad if isinstance(rows, torch.Tensor) else False
         ctx.save_for_backward(rows, z1, h1, z2, h2, ft, gl, z4, h4, arg_g, arg_o, W1m, W2m, W3m, W4g, W4f, W5m, g1, be1, g2, be2, g4, be4)
         ctx.shapes = [w.shape for w in (W1, W2, W3, W4, W5)]
-        outs = [tok]
-        for st in (s1, s2, s4):
-            outs += [st.mean64.float(), st.var_unbiased.float()]
-        ctx.mark_non_differentiable(*outs[1:])
-        return tuple(outs)
+        return _with_stats(ctx, tok, (s1, s2, s4))
 
     @staticmethod
     def backward(ctx, gtok, *_unused):
         (rows, z1, h1, z2, h2, ft, gl, z4, h4, arg_g, arg_o, W1m, W2m, W3m, W4g, W4f, W5m, g1, be1, g2, be2, g4, be4) = ctx.saved_tensors
         k, sync, E = ctx.k, ctx.sync, ctx.E
         s1, s2, s4 = ctx.stats
+        need = ctx.needs_input_grad[5:]        # W1 b1 g1 be1 W2 b2 g2 be2 W3 b3 W4 b4 g4 be4 W5 b5
         do = group_max_bwd(gtok, arg_o, k)
-        dW5, db5 = linear_tn(do, h4), colsum(do)
-        dz4, dg4, dbe4 = bn_backward(linear(do, _t(W5m)), z4, s4, g4, be4, True, sync)
+        dW5, db5 = _grad_if(need[14], lambda: linear_tn(do, h4)), _grad_if(need[15], lambda: colsum(do))
+        dz4, dg4, dbe4 = bn_backward(linear(do, _t(W5m)), z4, s4, g4, be4, True, sync, need[12] or need[13])
         dzg = group_sum(dz4, k)                                    # the global feature collects its k copies
-        dW4 = torch.cat([linear_tn(dzg, gl), linear_tn(dz4, ft)], 1)
-        db4 = colsum(dz4)
+        dW4 = _grad_if(need[10], lambda: torch.cat([linear_tn(dzg, gl), linear_tn(dz4, ft)], 1))
+        db4 = _grad_if(need[11], lambda: colsum(dz4))
         dft = linear(dz4, _t(W4f))
         group_max_bwd(linear(dzg, _t(W4g)), arg_g, k, into=dft)
-        dW3, db3 = linear_tn(dft, h2), colsum(dft)
-        dz2, dg2, dbe2 = bn_backward(linear(dft, _t(W3m)), z2, s2, g2, be2, True, sync)
-        dW2, db2 = linear_tn(dz2, h1), colsum(dz2)
-        dz1, dg1, dbe1 = bn_backward(linear(dz2, _t(W2m)), z1, s1, g1, be1, True, sync)
-        dW1, db1 = linear_tn(dz1, rows), colsum(dz1)
+        dW3, db3 = _grad_if(need[8], lambda: linear_tn(dft, h2)), _grad_if(need[9], lambda: colsum(dft))
+        dz2, dg2, dbe2 = bn_backward(linear(dft, _t(W3m)), z2, s2, g2, be2, True, sync, need[6] or need[7])
+        dW2, db2 = _grad_if(need[4], lambda: linear_tn(dz2, h1)), _grad_if(need[5], lambda: colsum(dz2))
+        dz1, dg1, dbe1 = bn_backward(linear(dz2, _t(W2m)), z1, s1, g1, be1, True, sync, need[2] or need[3])
+        dW1, db1 = _grad_if(need[0], lambda: linear_tn(dz1, rows)), _grad_if(need[1], lambda: colsum(dz1))
         drows = linear(dz1, _t(W1m)) if ctx.needs_input_grad[0] else None
         sh = ctx.shapes
-        return (drows, None, None, None, dW1.reshape(sh[0]), db1, dg1, dbe1, dW2.reshape(sh[1]), db2, dg2, dbe2, dW3.reshape(sh[2]), db3,
-                dW4.reshape(sh[3]), db4, dg4, dbe4, dW5.reshape(sh[4]), db5)
+        rs = lambda t, s: None if t is None else t.reshape(s)
+        return (drows, None, None, None, None, rs(dW1, sh[0]), db1, dg1, dbe1, rs(dW2, sh[1]), db2, dg2, dbe2, rs(dW3, sh[2]), db3,
+                rs(dW4, sh[3]), db4, dg4, dbe4, rs(dW5, sh[4]), db5)
 
 
 # ------------------------------------------------------------------------------------------------ P3Embed stage
 class P3StageTrainFn(torch.autograd.Function):
-    """One P3Embed stage in train mode on its gathered rows (pix4point.py:179-188): rows (M, 3+D), parameters of
-    convs.s.{0.0, 0.1, 0.2, 1.0, 1.1, 1.3, 1.4}.  Returns (out (groups, W), batch statistics of the three BatchNorms)."""
+    """One P3Embed stage under autograd on its gathered rows (pix4point.py:179-188): rows (M, 3+D), k, eps, sync, running (None:
+    train mode; three (running_mean, running_var) pairs: eval-mode BatchNorm), parameters of convs.s.{0.0, 0.1, 0.2, 1.0, 1.1,
+    1.3, 1.4}.  Returns (out (groups, W), batch statistics of the three BatchNorms), or (out,) in the running mode."""
 
     @staticmethod
-    def forward(ctx, rows, k, eps, sync, Wa, Wb, bb, g1, be1, Wc, g2, be2, Wd, g3, be3):
+    def forward(ctx, rows, k, eps, sync, running, Wa, Wb, bb, g1, be1, Wc, g2, be2, Wd, g3, be3):
         rows = _f32(rows)
         Wam, Wbm, Wcm, Wdm = (_w2(w) for w in (Wa, Wb, Wc, Wd))
         W = Wbm.shape[0]
         a = linear(rows, Wam)                                      # no bias, no activation (pix4point.py:139)
         z1 = linear(a, Wbm, bb)
-        f1, s1 = bn_forward(z1, g1, be1, eps[0], True, sync)
+        f1, s1 = bn_forward(z1, g1, be1, eps[0], True, sync, _running(0, running))
         gl, arg_g = group_max_arg(f1, k)                           # pix4point.py:185
         Wcg, Wcf = Wcm[:, :W].contiguous(), Wcm[:, W:].contiguous()
         z2 = linear(f1, Wcf, None, linear(gl, Wcg), k)             # [pooled || local] concat, pooled half once per group
-        h2, s2 = bn_forward(z2, g2, be2, eps[1], True, sync)
+        h2, s2 = bn_forward(z2, g2, be2, eps[1], True, sync, _running(1, running))
         z3 = linear(h2, Wdm)
-        h3, s3 = bn_forward(z3, g3, be3, eps[2], True, sync)
+        h3, s3 = bn_forward(z3, g3, be3, eps[2], True, sync, _running(2, running))
         out, arg_o = group_max_arg(h3, k)                          # pix4point.py:188
         ctx.k, ctx.sync = k, sync
         ctx.stats = (s1, s2, s3)
         ctx.save_for_backward(rows, a, z1, f1, gl, z2, h2, z3, arg_g, arg_o, Wam, Wbm, Wcg, Wcf, Wdm, g1, be1, g2, be2, g3, be3)
         ctx.shapes = [w.shape for w in (Wa, Wb, Wc, Wd)]
-        outs = [out]
-        for st in (s1, s2, s3):
-            outs += [st.mean64.float(), st.var_unbiased.float()]
-        ctx.mark_non_differentiable(*outs[1:])
-        return tuple(outs)
+        return _with_stats(ctx, out, (s1, s2, s3))
 
     @staticmethod
     def backward(ctx, gout, *_unused):
         (rows, a, z1, f1, gl, z2, h2, z3, arg_g, arg_o, Wam, Wbm, Wcg, Wcf, Wdm, g1, be1, g2, be2, g3, be3) = ctx.saved_tensors
         k, sync = ctx.k, ctx.sync
         s1, s2, s3 = ctx.stats
+        need = ctx.needs_input_grad[5:]        # Wa Wb bb g1 be1 Wc g2 be2 Wd g3 be3
         dh3 = group_max_bwd(gout, arg_o, k)
-        dz3, dg3, dbe3 = bn_backward(dh3, z3, s3, g3, be3, True, sync)
-        dWd = linear_tn(dz3, h2)
-        dz2, dg2, dbe2 = bn_backward(linear(dz3, _t(Wdm)), z2, s2, g2, be2, True, sync)
+        dz3, dg3, dbe3 = bn_backward(dh3, z3, s3, g3, be3, True, sync, need[9] or need[10])
+        dWd = _grad_if(need[8], lambda: linear_tn(dz3, h2))
+        dz2, dg2, dbe2 = bn_backward(linear(dz3, _t(Wdm)), z2, s2, g2, be2, True, sync, need[6] or need[7])
         dzg = group_sum(dz2, k)
-        dWc = torch.cat([linear_tn(dzg, gl), linear_tn(dz2, f1)], 1)
+        dWc = _grad_if(need[5], lambda: torch.cat([linear_tn(dzg, gl), linear_tn(dz2, f1)], 1))
         df1 = linear(dz2, _t(Wcf))
         group_max_bwd(linear(dzg, _t(Wcg)), arg_g, k, into=df1)
-        dz1, dg1, dbe1 = bn_backward(df1, z1, s1, g1, be1, True, sync)
-        dWb, dbb = linear_tn(dz1, a), colsum(dz1)
+        dz1, dg1, dbe1 = bn_backward(df1, z1, s1, g1, be1, True, sync, need[3] or need[4])
+        dWb, dbb = _grad_if(need[1], lambda: linear_tn(dz1, a)), _grad_if(need[2], lambda: colsum(dz1))
         da = linear(dz1, _t(Wbm))
-        dWa = linear_tn(da, rows)
+        dWa = _grad_if(need[0], lambda: linear_tn(da, rows))
         drows = linear(da, _t(Wam)) if ctx.needs_input_grad[0] else None
         sh = ctx.shapes
-        return (drows, None, None, None, dWa.reshape(sh[0]), dWb.reshape(sh[1]), dbb, dg1, dbe1, dWc.reshape(sh[2]), dg2, dbe2,
-                dWd.reshape(sh[3]), dg3, dbe3)
+        rs = lambda t, s: None if t is None else t.reshape(s)
+        return (drows, None, None, None, None, rs(dWa, sh[0]), rs(dWb, sh[1]), dbb, dg1, dbe1, rs(dWc, sh[2]), dg2, dbe2,
+                rs(dWd, sh[3]), dg3, dbe3)
 
 
 class GatherRowsFn(torch.autograd.Function):
@@ -358,22 +408,34 @@ class GatherRowsFn(torch.autograd.Function):
         return dp, df, None
 
 
+class ApfRowsFn(torch.autograd.Function):
+    """The (B*G*k, 2C) rows [x[nbr] - x[ctr] || x[ctr]] of Group.forward (apf.py:74-110) in Morton group order; backward sends
+    the row gradients to the points (p3tok_apf_rows_bwd_f32): every neighbour collects d rel, every centre sum_k (d ctr - d rel)."""
+
+    @staticmethod
+    def forward(ctx, x, fps_idx, knn_idx, perm):
+        x = _f32(x)
+        B, N, C = x.shape
+        r, keep = ops.apf_rows_descriptor(B, N, C, fps_idx, knn_idx.to(torch.int64), perm)
+        r.x = x.data_ptr()
+        rows = torch.empty((B * r.G * r.k, 2 * C), dtype=torch.float32, device=x.device)
+        with torch.cuda.device(x.device):
+            check(_L().p3tok_build_rows_f32(ctypes.byref(r), rows.data_ptr(), _s()), "build_rows_f32")
+        ctx.save_for_backward(*keep[:2], perm)
+        ctx.dims = (N, C)
+        return rows
+
+    @staticmethod
+    def backward(ctx, drows):
+        fps_idx, knn_idx, perm = ctx.saved_tensors
+        N, C = ctx.dims
+        dx = ops.apf_group_bwd(drows, None, fps_idx, knn_idx, perm, N, C) if ctx.needs_input_grad[0] else None
+        return dx, None, None, None
+
+
 def apf_rows(x: torch.Tensor, fps_idx: torch.Tensor, knn_idx: torch.Tensor, perm: Optional[torch.Tensor]) -> torch.Tensor:
-    """The (B*G*k, 2C) rows of Group.forward (apf.py:74-110) for the training path (inputs are data: no gradient)."""
-    x = _f32(x)
-    B, N, C = x.shape
-    G, k = knn_idx.shape[1], knn_idx.shape[2]
-    ci, kn = fps_idx.to(torch.int64).contiguous(), knn_idx.to(torch.int64).contiguous()
-    pm = perm.to(torch.int64).contiguous() if perm is not None else None
-    r = _lib.RowsStruct()
-    r.kind, r.C, r.D, r.idx_dtype = _lib.ROWS_APF, C, 0, _lib.I64
-    r.B, r.N, r.G, r.k = B, N, G, k
-    r.x, r.ctr_idx, r.knn_idx = x.data_ptr(), ci.data_ptr(), kn.data_ptr()
-    r.perm = pm.data_ptr() if pm is not None else None
-    rows = torch.empty((B * G * k, 2 * C), dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        check(_L().p3tok_build_rows_f32(ctypes.byref(r), rows.data_ptr(), _s()), "build_rows_f32")
-    return rows
+    """The APF rows of x under autograd (ApfRowsFn): the gradient reaches x when x requires one."""
+    return ApfRowsFn.apply(x, fps_idx, knn_idx, perm)
 
 
 @torch.no_grad()
@@ -387,23 +449,29 @@ def update_running(bn: torch.nn.modules.batchnorm._BatchNorm, mean: torch.Tensor
     bn.running_var.mul_(1.0 - m).add_(var_unbiased.to(bn.running_var.dtype), alpha=m)
 
 
-def encoder_train(enc, rows: torch.Tensor, k: int, sync: bool) -> torch.Tensor:
-    """Train-mode Encoder.forward on rows (M, cin) -> tokens (groups, E); updates the module's BatchNorm buffers."""
+def encoder_train(enc, rows: torch.Tensor, k: int, sync: bool, running: bool = False) -> torch.Tensor:
+    """Encoder.forward under autograd on rows (M, cin) -> tokens (groups, E).  running=False: train mode, updates the module's
+    BatchNorm buffers; running=True: eval-mode BatchNorm on the running estimates, buffers untouched, nothing all-reduced."""
     fc, sc = enc.first_conv, enc.second_conv
-    eps = (float(fc[1].eps), float(fc[4].eps), float(sc[1].eps))
-    outs = EncoderTrainFn.apply(rows, int(k), eps, bool(sync), fc[0].weight, fc[0].bias, fc[1].weight, fc[1].bias, fc[3].weight,
-                                fc[3].bias, fc[4].weight, fc[4].bias, fc[6].weight, fc[6].bias, sc[0].weight, sc[0].bias,
-                                sc[1].weight, sc[1].bias, sc[3].weight, sc[3].bias)
-    for bn, i in ((fc[1], 1), (fc[4], 3), (sc[1], 5)):
-        update_running(bn, outs[i], outs[i + 1])
+    bns = (fc[1], fc[4], sc[1])
+    eps = tuple(float(bn.eps) for bn in bns)
+    outs = EncoderTrainFn.apply(rows, int(k), eps, bool(sync) and not running, running_stats(bns) if running else None,
+                                fc[0].weight, fc[0].bias, fc[1].weight, fc[1].bias, fc[3].weight, fc[3].bias, fc[4].weight, fc[4].bias,
+                                fc[6].weight, fc[6].bias, sc[0].weight, sc[0].bias, sc[1].weight, sc[1].bias, sc[3].weight, sc[3].bias)
+    if not running:
+        for bn, i in zip(bns, (1, 3, 5)):
+            update_running(bn, outs[i], outs[i + 1])
     return outs[0]
 
 
-def p3stage_train(conv1, conv2, rows: torch.Tensor, k: int, sync: bool) -> torch.Tensor:
-    eps = (float(conv1[2].eps), float(conv2[1].eps), float(conv2[4].eps))
-    outs = P3StageTrainFn.apply(rows, int(k), eps, bool(sync), conv1[0].weight, conv1[1].weight, conv1[1].bias, conv1[2].weight,
-                                conv1[2].bias, conv2[0].weight, conv2[1].weight, conv2[1].bias, conv2[3].weight, conv2[4].weight,
-                                conv2[4].bias)
-    for bn, i in ((conv1[2], 1), (conv2[1], 3), (conv2[4], 5)):
-        update_running(bn, outs[i], outs[i + 1])
+def p3stage_train(conv1, conv2, rows: torch.Tensor, k: int, sync: bool, running: bool = False) -> torch.Tensor:
+    """One P3Embed stage under autograd on its rows; running as in encoder_train."""
+    bns = (conv1[2], conv2[1], conv2[4])
+    eps = tuple(float(bn.eps) for bn in bns)
+    outs = P3StageTrainFn.apply(rows, int(k), eps, bool(sync) and not running, running_stats(bns) if running else None,
+                                conv1[0].weight, conv1[1].weight, conv1[1].bias, conv1[2].weight, conv1[2].bias, conv2[0].weight,
+                                conv2[1].weight, conv2[1].bias, conv2[3].weight, conv2[4].weight, conv2[4].bias)
+    if not running:
+        for bn, i in zip(bns, (1, 3, 5)):
+            update_running(bn, outs[i], outs[i + 1])
     return outs[0]

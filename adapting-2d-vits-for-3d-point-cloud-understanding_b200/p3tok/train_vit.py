@@ -328,11 +328,12 @@ def dropout(x: torch.Tensor, p: float, training: bool, mask: Optional[torch.Tens
 class HeadTrainFn(torch.autograd.Function):
     """An MLP head in train mode: (Linear -> BatchNorm1d (batch statistics) -> ReLU -> Dropout) x n -> Linear - the reference's
     ClassificationHead (apf.py:230-252, n = 2) and ClsHead (pix4point.py:295-325).
-    apply(x (B,E), eps (n), sync, masks (n entries or None), W1, b1, g1, be1, ..., Wn, bn, gn, ben, Wout, bout) ->
-    (logits, batch mean / unbiased variance of every BatchNorm for the running-estimate update)."""
+    apply(x (B,E), eps (n), sync, masks (n entries or None), running (None, or n (running_mean, running_var) pairs: eval-mode
+    BatchNorm), W1, b1, g1, be1, ..., Wn, bn, gn, ben, Wout, bout) -> (logits, batch mean / unbiased variance of every BatchNorm
+    for the running-estimate update), or (logits,) in the running mode."""
 
     @staticmethod
-    def forward(ctx, x, eps, sync, masks, *params):
+    def forward(ctx, x, eps, sync, masks, running, *params):
         n = (len(params) - 2) // 4
         h = _f32(x)
         masks = tuple(masks) if masks is not None else (None,) * n
@@ -340,7 +341,7 @@ class HeadTrainFn(torch.autograd.Function):
         for i in range(n):
             W, b, g, be = params[4 * i:4 * i + 4]
             z = linear(h, W, b)
-            y, st = bn_forward(z, g, be, eps[i], True, sync)
+            y, st = bn_forward(z, g, be, eps[i], True, sync, None if running is None else running[i])
             saved += [h, z]
             stats.append(st)
             h = mask_mul(y, masks[i])
@@ -349,7 +350,8 @@ class HeadTrainFn(torch.autograd.Function):
         ctx.save_for_backward(*saved, h, *params)
         outs = [out]
         for st in stats:
-            outs += [st.mean64.float(), st.var_unbiased.float()]
+            if not st.running:
+                outs += [st.mean64.float(), st.var_unbiased.float()]
         ctx.mark_non_differentiable(*outs[1:])
         return tuple(outs)
 
@@ -357,18 +359,21 @@ class HeadTrainFn(torch.autograd.Function):
     def backward(ctx, g, *_unused):
         n = ctx.n
         saved, params = ctx.saved_tensors[:2 * n + 1], ctx.saved_tensors[2 * n + 1:]
+        need = ctx.needs_input_grad[5:]
         grads = [None] * len(params)
         g = _f32(g)
-        grads[-2], grads[-1] = linear_tn(g, saved[2 * n]), colsum(g)
+        grads[-2] = linear_tn(g, saved[2 * n]) if need[-2] else None
+        grads[-1] = colsum(g) if need[-1] else None
         d = linear(g, _t(_f32(params[-2])))
         for i in reversed(range(n)):
             W, b, gam, be = params[4 * i:4 * i + 4]
             hin, z = saved[2 * i], saved[2 * i + 1]
-            dz, dgam, dbe = bn_backward(mask_mul(d, ctx.masks[i]), z, ctx.stats[i], gam, be, True, ctx.sync)
-            grads[4 * i:4 * i + 4] = [linear_tn(dz, hin), colsum(dz), dgam, dbe]
+            nd = need[4 * i:4 * i + 4]
+            dz, dgam, dbe = bn_backward(mask_mul(d, ctx.masks[i]), z, ctx.stats[i], gam, be, True, ctx.sync, nd[2] or nd[3])
+            grads[4 * i:4 * i + 4] = [linear_tn(dz, hin) if nd[0] else None, colsum(dz) if nd[1] else None, dgam, dbe]
             if i > 0 or ctx.needs_input_grad[0]:
                 d = linear(dz, _t(_f32(W)))
-        return (d if ctx.needs_input_grad[0] else None, None, None, None, *grads)
+        return (d if ctx.needs_input_grad[0] else None, None, None, None, None, *grads)
 
 
 def mlp_head_blocks(seq):
@@ -378,21 +383,25 @@ def mlp_head_blocks(seq):
     return [(mods[4 * i], mods[4 * i + 1], mods[4 * i + 3]) for i in range(n)], mods[-1]
 
 
-def head_train(head, x: torch.Tensor, masks=None, sync: bool = False, generator: Optional[torch.Generator] = None) -> torch.Tensor:
-    """Train-mode forward of an MLP head module (attribute `mlp_head` or `head`) on x (B,E); updates the BatchNorm buffers like
-    nn.BatchNorm1d does."""
-    from .train import update_running
+def head_train(head, x: torch.Tensor, masks=None, sync: bool = False, generator: Optional[torch.Generator] = None,
+               running: bool = False) -> torch.Tensor:
+    """Forward of an MLP head module (attribute `mlp_head` or `head`) on x (B,E) under autograd.  Train mode: dropout keep masks,
+    batch statistics, the BatchNorm buffers updated like nn.BatchNorm1d does.  running=True: the module in eval mode - dropout
+    is the identity, BatchNorm uses the running estimates, no buffer changes, nothing all-reduced."""
+    from .train import running_stats, update_running
     blocks, last = mlp_head_blocks(head.mlp_head if hasattr(head, "mlp_head") else head.head)
-    if masks is None:
+    if masks is None and not running:
         masks = tuple(keep_mask((x.shape[0], lin.out_features), float(dr.p), x.device, generator) for lin, _, dr in blocks)
         if all(m is None for m in masks):
             masks = None
     params = []
     for lin, bn, _ in blocks:
         params += [lin.weight, lin.bias, bn.weight, bn.bias]
-    outs = HeadTrainFn.apply(x, tuple(float(bn.eps) for _, bn, _ in blocks), bool(sync), masks, *params, last.weight, last.bias)
-    for i, (_, bn, _) in enumerate(blocks):
-        update_running(bn, outs[1 + 2 * i], outs[2 + 2 * i])
+    outs = HeadTrainFn.apply(x, tuple(float(bn.eps) for _, bn, _ in blocks), bool(sync) and not running, None if running else masks,
+                             running_stats([bn for _, bn, _ in blocks]) if running else None, *params, last.weight, last.bias)
+    if not running:
+        for i, (_, bn, _) in enumerate(blocks):
+            update_running(bn, outs[1 + 2 * i], outs[2 + 2 * i])
     return outs[0]
 
 

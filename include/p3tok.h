@@ -366,6 +366,17 @@ P3TOK_API int p3tok_scatter_rows_add_f32(const float* dRows, const int32_t* idx,
  * input (the inference path never materialises it). */
 P3TOK_API int p3tok_build_rows_f32(const p3tok_rows* rows, float* X, void* stream);
 
+/* ---- gradients with respect to the input points (adversarial examples, saliency) -------------------------------------------
+ * Both functions ACCUMULATE into dX (the caller zeroes it) with fp32 atomic adds, like p3tok_scatter_rows_add_f32 and torch's
+ * own CUDA index backward: the result is reproducible to rounding, not bit for bit (the order of the adds varies). */
+/* Adjoint of p3tok_build_rows_f32 for kind 0 (APF): dRows (B*G*k, 2C) in the rows' output order (group j = input group
+ * perm[b,j]) -> dX (B,N,C) += d rel at x[b,nbr] and sum over the group's k rows of (d ctr - d rel) at x[b,ctr].  rows->x is not
+ * read; knn_idx is int64 or int32 (rows->idx_dtype). */
+P3TOK_API int p3tok_apf_rows_bwd_f32(const p3tok_rows* rows, const float* dRows, float* dX, void* stream);
+/* Adjoint of p3tok_gather_points: dOut (B,S,C), idx (B,S) int64 -> dX (B,N,C) += dOut at the gathered rows. */
+P3TOK_API int p3tok_gather_points_bwd_f32(const float* dOut, int64_t B, int64_t N, int64_t C, const int64_t* idx, int64_t S,
+                                          float* dX, void* stream);
+
 /* ---- training through the ViT block stack (SURVEY 8f "next" #4 on top of #3) -------------------------------------------
  * The reference keeps the blocks frozen but trains point_encoder / encoder_norm / head (src/models/apf.py:335-346), so a
  * training step differentiates APFViTLayer x depth (src/models/apf_utils.py:268-293) -> encoder_norm -> max over tokens ->
