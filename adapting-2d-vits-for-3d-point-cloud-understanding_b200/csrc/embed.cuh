@@ -42,6 +42,13 @@ int tc_linear_ex(const __nv_bfloat16* A, int64_t M, int K, const __nv_bfloat16* 
 // vit.cu
 int64_t apf_vit_workspace(int64_t B, int64_t G, int64_t D, int64_t H, int64_t R, bool x3);
 
+// train.cu: the column-strip reductions (rows per strip from the shapes only) and their deterministic finish
+bool ws_ok(const void* ws, int64_t ws_bytes, int64_t need);      // need bytes available, 16-byte aligned
+int64_t strip_rows(int64_t M, int N);
+int colsum_det_begin(const void* ws, int64_t ws_bytes, int64_t M, int64_t N, const char* who);
+// out0[c] / out1[c] = sum in ascending strip order of part[0][strip][c] / part[1][strip][c], part = [2][strips][N] fp64
+int strip_sum_f64(const double* part, int64_t M, int N, double* out0, double* out1, cudaStream_t s);
+
 static inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
 
 }  // namespace p3tok

@@ -22,6 +22,11 @@
 //   p3tok_build_rows_f32            the gathered row matrix of p3tok_rows    (forward input of the training path)
 //   p3tok_apf_rows_bwd_f32          adjoint of the APF rows: gradient to the input points (neighbour and centre terms)
 //   p3tok_gather_points_bwd_f32     adjoint of p3tok_gather_points (index_points, fps, the centres)
+//
+// The kernels that finish a sum with floating-point atomics (sgemm_tn, the three column-strip reductions, the three scatter
+// adjoints) also have deterministic instantiations behind the *_det_f32 entry points: the split-M GEMM and the strips store
+// their partials to a caller-owned workspace, summed afterwards in ascending slice / strip order in fp64; the scatters add
+// fixed-point integers (a per-cloud power-of-two scale) with 64-bit integer atomics, which is associative, and convert once.
 #include "embed.cuh"
 
 namespace p3tok {
@@ -31,8 +36,10 @@ static inline unsigned tr_grid(int64_t total, int threads, int64_t cap = 148 * 3
   return (unsigned)(b < 1 ? 1 : (b > cap ? cap : b));
 }
 
-// ---- dW[N,K] (+)= dY[M,N]^T X[M,K]: 64 x 64 outputs per CTA, 4 x 4 per thread, the M range split over gridDim.z
+// ---- dW[N,K] (+)= dY[M,N]^T X[M,K]: 64 x 64 outputs per CTA, 4 x 4 per thread, the M range split over gridDim.z.
+// kPartial: slice z stores its tile to dW[z][N][K] (a workspace) instead of adding it atomically.
 constexpr int TN_T = 64, TN_MM = 16;
+template <bool kPartial>
 __global__ void __launch_bounds__(256)
 sgemm_tn_kernel(const float* __restrict__ dY, const float* __restrict__ X, int64_t M, int N, int K, float* __restrict__ dW,
                 int64_t rows_per_slice) {
@@ -76,12 +83,29 @@ sgemm_tn_kernel(const float* __restrict__ dY, const float* __restrict__ X, int64
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int k = k0 + tk * 4 + j;
-      if (k < K) atomicAdd(&dW[(size_t)n * K + k], acc[i][j]);
+      if (k < K) {
+        if constexpr (kPartial) dW[((size_t)blockIdx.z * N + n) * K + k] = acc[i][j];
+        else atomicAdd(&dW[(size_t)n * K + k], acc[i][j]);
+      }
     }
   }
 }
 
-// ---- per-channel sums: every thread walks a strip of rows of ONE column group, fp32 inside the strip, fp64 across strips
+// dW[e] (+)= fp32 of the slices' partials part[z][e] summed in ascending z in fp64 (rounded once)
+__global__ void slice_sum_kernel(const float* __restrict__ part, int64_t slices, int64_t total, int accumulate,
+                                 float* __restrict__ dW) {
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    double s = 0.0;
+    for (int64_t z = 0; z < slices; ++z) s += (double)part[z * total + e];
+    const float r = (float)s;
+    dW[e] = accumulate ? dW[e] + r : r;
+  }
+}
+
+// ---- per-channel sums: every thread walks a strip of rows of ONE column group, fp32 inside the strip, fp64 across strips.
+// kPartial (here and in bn_bwd_stats_kernel / ln_param_grad_kernel): strip y stores its sums to sum[y][N] / sumsq[y][N] (a
+// workspace) instead of adding them atomically; strip_sum_kernel then adds the strips in order.
+template <bool kPartial>
 __global__ void __launch_bounds__(256)
 colstats_kernel(const float* __restrict__ X, int64_t M, int N, int64_t rows_per_block, double* __restrict__ sum,
                 double* __restrict__ sumsq) {
@@ -107,8 +131,13 @@ colstats_kernel(const float* __restrict__ X, int64_t M, int N, int64_t rows_per_
   if (rlane == 0 && c < N) {
 #pragma unroll
     for (int r = 1; r < 8; ++r) { s += rs[r][threadIdx.x & 31]; q += rq[r][threadIdx.x & 31]; }
-    atomicAdd(&sum[c], s);
-    atomicAdd(&sumsq[c], q);
+    if constexpr (kPartial) {
+      sum[(size_t)blockIdx.y * N + c] = s;
+      sumsq[(size_t)blockIdx.y * N + c] = q;
+    } else {
+      atomicAdd(&sum[c], s);
+      atomicAdd(&sumsq[c], q);
+    }
   }
 }
 
@@ -123,7 +152,20 @@ __global__ void bn_act_kernel(const float* __restrict__ Z, int64_t total, int N,
   }
 }
 
+// out0[c] / out1[c] = sum over strips, in ascending order, of part[0][strip][c] / part[1][strip][c] (fp64)
+__global__ void strip_sum_kernel(const double* __restrict__ part, int64_t strips, int N, double* __restrict__ out0,
+                                 double* __restrict__ out1) {
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < 2 * N; e += gridDim.x * blockDim.x) {
+    const int q = e >= N, c = e - q * N;
+    const double* p = part + (size_t)q * strips * N + c;
+    double s = 0.0;
+    for (int64_t y = 0; y < strips; ++y) s += p[y * N];
+    (q ? out1 : out0)[c] = s;
+  }
+}
+
 // s1[c] = sum dy', s2[c] = sum dy' xhat with dy' = dy * [y > 0] (ReLU) and xhat = (z - mean) rstd
+template <bool kPartial>
 __global__ void __launch_bounds__(256)
 bn_bwd_stats_kernel(const float* __restrict__ dY, const float* __restrict__ Z, int64_t M, int N, const float* __restrict__ mean,
                     const float* __restrict__ rstd, const float* __restrict__ gamma, const float* __restrict__ beta, int relu,
@@ -153,8 +195,13 @@ bn_bwd_stats_kernel(const float* __restrict__ dY, const float* __restrict__ Z, i
   if (rlane == 0 && c < N) {
 #pragma unroll
     for (int r = 1; r < 8; ++r) { a += ra[r][threadIdx.x & 31]; b += rb[r][threadIdx.x & 31]; }
-    atomicAdd(&s1[c], a);
-    atomicAdd(&s2[c], b);
+    if constexpr (kPartial) {
+      s1[(size_t)blockIdx.y * N + c] = a;
+      s2[(size_t)blockIdx.y * N + c] = b;
+    } else {
+      atomicAdd(&s1[c], a);
+      atomicAdd(&s2[c], b);
+    }
   }
 }
 
@@ -217,9 +264,72 @@ __global__ void group_sum_kernel(const float* __restrict__ X, int64_t G, int k, 
   }
 }
 
+// ---- how a scatter adjoint adds contribution v of cloud b to dst[i] (the last argument of the three kernels below)
+// The default: an fp32 atomic add; the order in which the adds arrive decides the rounding.
+struct AtomicF32Add {
+  __device__ __forceinline__ void operator()(float* dst, int64_t i, int64_t, float v) const { atomicAdd(dst + i, v); }
+};
+
+// Deterministic pass 1: the largest finite |v| of every cloud (float bits; for non-negative floats their unsigned order is
+// the float order), one atomicMax per group of lanes that share a cloud.
+struct CloudMaxAbs {
+  uint32_t* cmax;
+  __device__ __forceinline__ void operator()(float*, int64_t, int64_t b, float v) const {
+    uint32_t a = isfinite(v) ? __float_as_uint(fabsf(v)) : 0u;
+    const unsigned grp = __match_any_sync(__activemask(), (unsigned long long)b);
+    a = __reduce_max_sync(grp, a);
+    if ((int)(threadIdx.x & 31) == __ffs(grp) - 1 && a) atomicMax(&cmax[b], a);
+  }
+};
+
+// 2^s with s = 61 - cbits - e, where the cloud's largest |v| < 2^e and every destination receives at most 2^cbits
+// contributions: each rint(v 2^s) is at most 2^(61 - cbits) in magnitude, so no destination's sum exceeds 2^61.
+__device__ __forceinline__ int fixed_scale(uint32_t maxbits, int cbits) {
+  if (maxbits == 0) return 0;
+  const int ex = (int)(maxbits >> 23);
+  const int e = ex ? ex - 126 : (32 - __clz((int)maxbits)) - 149;   // normal: 1.m 2^(ex-127) < 2^(ex-126); subnormal: m 2^-149
+  return 61 - cbits - e;
+}
+
+// Deterministic pass 2: q = rint(v 2^s) added with 64-bit integer atomics (associative: the sum does not depend on the
+// order of arrival); a non-finite v sets a flag instead (1 NaN, 2 +inf, 4 -inf).  Slots: dst == out1 ? out1_slot + i : i.
+struct FixedAdd {
+  unsigned long long* acc;
+  uint32_t* flags;
+  const uint32_t* cmax;
+  int cbits;
+  const float* out1;
+  int64_t out1_slot;
+  __device__ __forceinline__ void operator()(float* dst, int64_t i, int64_t b, float v) const {
+    const int64_t slot = (dst == out1 ? out1_slot : 0) + i;
+    if (!isfinite(v)) {
+      atomicOr(&flags[slot], isnan(v) ? 1u : (v > 0.f ? 2u : 4u));
+      return;
+    }
+    const long long q = __double2ll_rn(ldexp((double)v, fixed_scale(cmax[b], cbits)));   // exact scaling, one rounding
+    atomicAdd(&acc[slot], (unsigned long long)q);
+  }
+};
+
+// out[e] += fp32(acc[e]) 2^-s, or the IEEE sum of the flagged non-finite contributions (slot e belongs to cloud e / per_cloud)
+__global__ void fixed_to_f32_kernel(const unsigned long long* __restrict__ acc, const uint32_t* __restrict__ flags,
+                                    const uint32_t* __restrict__ cmax, int cbits, int64_t per_cloud, int64_t total,
+                                    float* __restrict__ out) {
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const uint32_t f = flags[e];
+    float v;
+    if ((f & 1u) || (f & 6u) == 6u) v = __uint_as_float(0x7fc00000u);
+    else if (f & 2u) v = __uint_as_float(0x7f800000u);
+    else if (f & 4u) v = __uint_as_float(0xff800000u);
+    else v = (float)ldexp((double)__ll2float_rn((long long)acc[e]), -fixed_scale(cmax[e / per_cloud], cbits));
+    out[e] += v;
+  }
+}
+
 // gradient of the gather (pix4point.py:92-102): dRows (B,G,k,3+D) -> dP (B,N,3) += , dF (B,N,D) +=
+template <typename Fin>
 __global__ void scatter_rows_add_kernel(const float* __restrict__ dRows, const int32_t* __restrict__ idx, int64_t B, int64_t N,
-                                        int64_t Gk, int D, float* __restrict__ dP, float* __restrict__ dF) {
+                                        int64_t Gk, int D, float* __restrict__ dP, float* __restrict__ dF, Fin fin) {
   const int W = 3 + D;
   const int64_t total = B * Gk * W;
   for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
@@ -228,18 +338,18 @@ __global__ void scatter_rows_add_kernel(const float* __restrict__ dRows, const i
     const int64_t b = row / Gk;
     const int64_t p = b * N + idx[row];
     const float v = dRows[e];
-    if (c < 3) { if (dP) atomicAdd(&dP[p * 3 + c], v); }
-    else if (dF) atomicAdd(&dF[p * D + (c - 3)], v);
+    if (c < 3) { if (dP) fin(dP, p * 3 + c, b, v); }
+    else if (dF) fin(dF, p * D + (c - 3), b, v);
   }
 }
 
 // adjoint of the APF rows (build_rows kind 0): output group bj reads input group g = perm[bj]; its row n is
 // [x[nbr] - x[ctr] || x[ctr]].  One thread per (output group, channel): d rel goes to the neighbour (one atomic per element),
 // sum_n (d ctr - d rel) is reduced over the group's k rows in a register and added to the centre with one atomic.
-template <typename IdxT>
+template <typename IdxT, typename Fin>
 __global__ void apf_rows_bwd_kernel(const float* __restrict__ dRows, const int64_t* __restrict__ ctr_idx,
                                     const IdxT* __restrict__ knn_idx, const int64_t* __restrict__ perm, int64_t N, int64_t G,
-                                    int k, int C, int64_t BG, float* __restrict__ dX) {
+                                    int k, int C, int64_t BG, float* __restrict__ dX, Fin fin) {
   const int64_t total = BG * C;
   for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     const int c = (int)(e % C);
@@ -251,27 +361,40 @@ __global__ void apf_rows_bwd_kernel(const float* __restrict__ dRows, const int64
     float acc = 0.f;
     for (int n = 0; n < k; ++n) {
       const float drel = d[(int64_t)n * 2 * C], dctr = d[(int64_t)n * 2 * C + C];
-      atomicAdd(&dX[(b * N + (int64_t)nbr[n]) * C + c], drel);
+      fin(dX, (b * N + (int64_t)nbr[n]) * C + c, b, drel);
       acc += dctr - drel;
     }
-    atomicAdd(&dX[(b * N + ctr_idx[b * G + g]) * C + c], acc);
+    fin(dX, (b * N + ctr_idx[b * G + g]) * C + c, b, acc);
   }
 }
 
 // adjoint of gather_points: dX[b, idx[b,s], c] += dOut[b, s, c]
+template <typename Fin>
 __global__ void gather_points_bwd_kernel(const float* __restrict__ dOut, int64_t N, int C, const int64_t* __restrict__ idx,
-                                         int64_t S, int64_t total, float* __restrict__ dX) {
+                                         int64_t S, int64_t total, float* __restrict__ dX, Fin fin) {
   for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     const int c = (int)(e % C);
     const int64_t bs = e / C;
     const int64_t b = bs / S;
-    atomicAdd(&dX[(b * N + idx[bs]) * C + c], dOut[e]);
+    fin(dX, (b * N + idx[bs]) * C + c, b, dOut[e]);
   }
 }
 
 }  // namespace p3tok
 
 using namespace p3tok;
+
+// split-M decomposition of the weight-gradient GEMM, from the shapes only: enough M slices to fill the GPU (~4 CTAs per SM of
+// a B200: 148 * 4 is a constant, not a device query), each a multiple of the 16-row tile and at least 256 rows
+static int64_t tn_slices(int64_t M, int64_t N, int64_t K, int64_t* rows_per_slice) {
+  const int64_t gn = (N + TN_T - 1) / TN_T, gk = (K + TN_T - 1) / TN_T;
+  int64_t slices = (148 * 4 + gn * gk - 1) / (gn * gk);
+  int64_t rows = (M + slices - 1) / slices;
+  rows = (rows + 255) / 256 * 256;
+  *rows_per_slice = rows;
+  return (M + rows - 1) / rows;
+}
+
 
 extern "C" int p3tok_linear_tn_f32(const float* dY, const float* X, int64_t M, int64_t N, int64_t K, float* dW, int accumulate,
                                    void* stream) {
@@ -281,24 +404,83 @@ extern "C" int p3tok_linear_tn_f32(const float* dY, const float* X, int64_t M, i
   if (!accumulate) P3_CUDA(cudaMemsetAsync(dW, 0, (size_t)N * K * sizeof(float), s));
   if (M == 0) return P3TOK_OK;
   const int gn = (int)((N + TN_T - 1) / TN_T), gk = (int)((K + TN_T - 1) / TN_T);
-  // enough M slices to fill the GPU (~4 CTAs per SM), each a multiple of the 16-row tile and at least 256 rows
-  int64_t slices = (148 * 4 + gn * gk - 1) / (gn * gk);
-  int64_t rows = (M + slices - 1) / slices;
-  rows = (rows + 255) / 256 * 256;
-  slices = (M + rows - 1) / rows;
+  int64_t rows;
+  const int64_t slices = tn_slices(M, N, K, &rows);
   P3_REQUIRE(slices < 65536, P3TOK_ERR_UNSUPPORTED, "linear_tn_f32: too many rows");
-  sgemm_tn_kernel<<<dim3((unsigned)gn, (unsigned)gk, (unsigned)slices), 256, 0, s>>>(dY, X, M, (int)N, (int)K, dW, rows);
+  sgemm_tn_kernel<false><<<dim3((unsigned)gn, (unsigned)gk, (unsigned)slices), 256, 0, s>>>(dY, X, M, (int)N, (int)K, dW, rows);
   P3_LAUNCH_CHECK("sgemm_tn_kernel");
   return P3TOK_OK;
 }
 
-static int64_t strip_rows(int64_t M, int N) {
+extern "C" int64_t p3tok_linear_tn_det_workspace_bytes(int64_t M, int64_t N, int64_t K) {
+  if (M <= 0 || N <= 0 || K <= 0) return 0;
+  int64_t rows;
+  return tn_slices(M, N, K, &rows) * N * K * (int64_t)sizeof(float);
+}
+
+extern "C" int p3tok_linear_tn_det_f32(const float* dY, const float* X, int64_t M, int64_t N, int64_t K, float* dW, int accumulate,
+                                       void* workspace, int64_t workspace_bytes, void* stream) {
+  P3_REQUIRE(M >= 0 && N > 0 && K > 0 && N < (1 << 24) && K < (1 << 24), P3TOK_ERR_INVALID, "linear_tn_det_f32: bad shape");
+  P3_REQUIRE(dW && (M == 0 || (dY && X)), P3TOK_ERR_INVALID, "linear_tn_det_f32: null pointer");
+  cudaStream_t s = as_stream(stream);
+  if (M == 0) {
+    if (!accumulate) P3_CUDA(cudaMemsetAsync(dW, 0, (size_t)N * K * sizeof(float), s));
+    return P3TOK_OK;
+  }
+  P3_REQUIRE(ws_ok(workspace, workspace_bytes, p3tok_linear_tn_det_workspace_bytes(M, N, K)), P3TOK_ERR_WORKSPACE,
+             "linear_tn_det_f32: workspace below p3tok_linear_tn_det_workspace_bytes or not 16-byte aligned");
+  const int gn = (int)((N + TN_T - 1) / TN_T), gk = (int)((K + TN_T - 1) / TN_T);
+  int64_t rows;
+  const int64_t slices = tn_slices(M, N, K, &rows);
+  P3_REQUIRE(slices < 65536, P3TOK_ERR_UNSUPPORTED, "linear_tn_det_f32: too many rows");
+  float* part = static_cast<float*>(workspace);
+  sgemm_tn_kernel<true><<<dim3((unsigned)gn, (unsigned)gk, (unsigned)slices), 256, 0, s>>>(dY, X, M, (int)N, (int)K, part, rows);
+  P3_LAUNCH_CHECK("sgemm_tn_kernel");
+  slice_sum_kernel<<<tr_grid(N * K, 256), 256, 0, s>>>(part, slices, N * K, accumulate, dW);
+  P3_LAUNCH_CHECK("slice_sum_kernel");
+  return P3TOK_OK;
+}
+
+namespace p3tok {
+
+bool ws_ok(const void* ws, int64_t ws_bytes, int64_t need) {
+  return need <= ws_bytes && (need == 0 || (ws && ((uintptr_t)ws & 15) == 0));
+}
+
+int64_t strip_rows(int64_t M, int N) {
   const int64_t cgroups = (N + 31) / 32;
   int64_t strips = (148 * 8 + cgroups - 1) / cgroups;
   int64_t rows = (M + strips - 1) / strips;
   rows = (rows + 63) / 64 * 64;
   return rows < 64 ? 64 : rows;
 }
+
+}  // namespace p3tok
+
+extern "C" int64_t p3tok_colsum_det_workspace_bytes(int64_t M, int64_t N) {
+  if (M <= 0 || N <= 0 || N >= (1 << 24)) return 0;
+  const int64_t rows = strip_rows(M, (int)N);
+  return 2 * ((M + rows - 1) / rows) * N * (int64_t)sizeof(double);
+}
+
+namespace p3tok {
+
+int strip_sum_f64(const double* part, int64_t M, int N, double* out0, double* out1, cudaStream_t s) {
+  const int64_t rows = strip_rows(M, N);
+  strip_sum_kernel<<<tr_grid(2 * (int64_t)N, 256), 256, 0, s>>>(part, (M + rows - 1) / rows, N, out0, out1);
+  P3_LAUNCH_CHECK("strip_sum_kernel");
+  return P3TOK_OK;
+}
+
+int colsum_det_begin(const void* ws, int64_t ws_bytes, int64_t M, int64_t N, const char* who) {
+  P3_REQUIRE(ws_ok(ws, ws_bytes, p3tok_colsum_det_workspace_bytes(M, N)), P3TOK_ERR_WORKSPACE,
+             "%s: workspace below p3tok_colsum_det_workspace_bytes or not 16-byte aligned", who);
+  const int64_t rows = strip_rows(M, (int)N);
+  P3_REQUIRE((M + rows - 1) / rows < 65536, P3TOK_ERR_UNSUPPORTED, "%s: too many rows", who);
+  return P3TOK_OK;
+}
+
+}  // namespace p3tok
 
 extern "C" int p3tok_colstats_f32(const float* X, int64_t M, int64_t N, double* sum, double* sumsq, void* stream) {
   P3_REQUIRE(M >= 0 && N > 0 && N < (1 << 24), P3TOK_ERR_INVALID, "colstats_f32: bad shape");
@@ -310,9 +492,28 @@ extern "C" int p3tok_colstats_f32(const float* X, int64_t M, int64_t N, double* 
   const int64_t rows = strip_rows(M, (int)N);
   const int64_t strips = (M + rows - 1) / rows;
   P3_REQUIRE(strips < 65536, P3TOK_ERR_UNSUPPORTED, "colstats_f32: too many rows");
-  colstats_kernel<<<dim3((unsigned)((N + 31) / 32), (unsigned)strips), 256, 0, s>>>(X, M, (int)N, rows, sum, sumsq);
+  colstats_kernel<false><<<dim3((unsigned)((N + 31) / 32), (unsigned)strips), 256, 0, s>>>(X, M, (int)N, rows, sum, sumsq);
   P3_LAUNCH_CHECK("colstats_kernel");
   return P3TOK_OK;
+}
+
+extern "C" int p3tok_colstats_det_f32(const float* X, int64_t M, int64_t N, double* sum, double* sumsq, void* workspace,
+                                      int64_t workspace_bytes, void* stream) {
+  P3_REQUIRE(M >= 0 && N > 0 && N < (1 << 24), P3TOK_ERR_INVALID, "colstats_det_f32: bad shape");
+  P3_REQUIRE(sum && sumsq && (M == 0 || X), P3TOK_ERR_INVALID, "colstats_det_f32: null pointer");
+  cudaStream_t s = as_stream(stream);
+  if (M == 0) {
+    P3_CUDA(cudaMemsetAsync(sum, 0, (size_t)N * sizeof(double), s));
+    P3_CUDA(cudaMemsetAsync(sumsq, 0, (size_t)N * sizeof(double), s));
+    return P3TOK_OK;
+  }
+  const int rc = colsum_det_begin(workspace, workspace_bytes, M, N, "colstats_det_f32");
+  if (rc != P3TOK_OK) return rc;
+  const int64_t rows = strip_rows(M, (int)N), strips = (M + rows - 1) / rows;
+  double* part = static_cast<double*>(workspace);
+  colstats_kernel<true><<<dim3((unsigned)((N + 31) / 32), (unsigned)strips), 256, 0, s>>>(X, M, (int)N, rows, part, part + strips * N);
+  P3_LAUNCH_CHECK("colstats_kernel");
+  return strip_sum_f64(part, M, (int)N, sum, sumsq, s);
 }
 
 extern "C" int p3tok_bn_act_f32(const float* Z, int64_t M, int64_t N, const float* mean, const float* rstd, const float* gamma,
@@ -336,10 +537,32 @@ extern "C" int p3tok_bn_bwd_stats_f32(const float* dY, const float* Z, int64_t M
   const int64_t rows = strip_rows(M, (int)N);
   const int64_t strips = (M + rows - 1) / rows;
   P3_REQUIRE(strips < 65536, P3TOK_ERR_UNSUPPORTED, "bn_bwd_stats_f32: too many rows");
-  bn_bwd_stats_kernel<<<dim3((unsigned)((N + 31) / 32), (unsigned)strips), 256, 0, s>>>(dY, Z, M, (int)N, mean, rstd, gamma, beta, relu,
+  bn_bwd_stats_kernel<false><<<dim3((unsigned)((N + 31) / 32), (unsigned)strips), 256, 0, s>>>(dY, Z, M, (int)N, mean, rstd, gamma, beta, relu,
                                                                                         rows, s1, s2);
   P3_LAUNCH_CHECK("bn_bwd_stats_kernel");
   return P3TOK_OK;
+}
+
+extern "C" int p3tok_bn_bwd_stats_det_f32(const float* dY, const float* Z, int64_t M, int64_t N, const float* mean, const float* rstd,
+                                          const float* gamma, const float* beta, int relu, double* s1, double* s2, void* workspace,
+                                          int64_t workspace_bytes, void* stream) {
+  P3_REQUIRE(M >= 0 && N > 0 && N < (1 << 24), P3TOK_ERR_INVALID, "bn_bwd_stats_det_f32: bad shape");
+  P3_REQUIRE(s1 && s2 && (M == 0 || (dY && Z && mean && rstd && gamma && beta)), P3TOK_ERR_INVALID,
+             "bn_bwd_stats_det_f32: null pointer");
+  cudaStream_t s = as_stream(stream);
+  if (M == 0) {
+    P3_CUDA(cudaMemsetAsync(s1, 0, (size_t)N * sizeof(double), s));
+    P3_CUDA(cudaMemsetAsync(s2, 0, (size_t)N * sizeof(double), s));
+    return P3TOK_OK;
+  }
+  const int rc = colsum_det_begin(workspace, workspace_bytes, M, N, "bn_bwd_stats_det_f32");
+  if (rc != P3TOK_OK) return rc;
+  const int64_t rows = strip_rows(M, (int)N), strips = (M + rows - 1) / rows;
+  double* part = static_cast<double*>(workspace);
+  bn_bwd_stats_kernel<true><<<dim3((unsigned)((N + 31) / 32), (unsigned)strips), 256, 0, s>>>(dY, Z, M, (int)N, mean, rstd, gamma, beta,
+                                                                                              relu, rows, part, part + strips * N);
+  P3_LAUNCH_CHECK("bn_bwd_stats_kernel");
+  return strip_sum_f64(part, M, (int)N, s1, s2, s);
 }
 
 extern "C" int p3tok_bn_bwd_apply_f32(const float* dY, const float* Z, int64_t M, int64_t N, int64_t count, const float* mean,
@@ -382,13 +605,76 @@ extern "C" int p3tok_group_sum_f32(const float* X, int64_t G, int64_t k, int64_t
   return P3TOK_OK;
 }
 
+// ---- fixed-point scatters: workspace = acc int64 [B*N*C] | flags uint32 [B*N*C] | largest |v| per cloud uint32 [B]
+struct FixedWs {
+  unsigned long long* acc;
+  uint32_t* flags;
+  uint32_t* cmax;
+};
+
+static int ceil_log2(int64_t n) {
+  int c = 0;
+  while (((int64_t)1 << c) < n) ++c;
+  return c;
+}
+
+extern "C" int64_t p3tok_scatter_det_workspace_bytes(int64_t B, int64_t N, int64_t C) {
+  if (B <= 0 || N <= 0 || C <= 0) return 0;
+  return B * N * C * (int64_t)(sizeof(unsigned long long) + sizeof(uint32_t)) + B * (int64_t)sizeof(uint32_t);
+}
+
+static int fixed_begin(void* ws, int64_t ws_bytes, int64_t B, int64_t N, int64_t C, cudaStream_t s, FixedWs* f, const char* who) {
+  const int64_t need = p3tok_scatter_det_workspace_bytes(B, N, C);
+  P3_REQUIRE(ws_ok(ws, ws_bytes, need), P3TOK_ERR_WORKSPACE,
+             "%s: workspace below p3tok_scatter_det_workspace_bytes or not 16-byte aligned", who);
+  P3_CUDA(cudaMemsetAsync(ws, 0, (size_t)need, s));
+  f->acc = static_cast<unsigned long long*>(ws);
+  f->flags = reinterpret_cast<uint32_t*>(f->acc + B * N * C);
+  f->cmax = f->flags + B * N * C;
+  return P3TOK_OK;
+}
+
+static FixedAdd fixed_add(const FixedWs& f, int cbits, const float* out1 = nullptr, int64_t out1_slot = 0) {
+  return FixedAdd{f.acc, f.flags, f.cmax, cbits, out1, out1_slot};
+}
+
+// out (B, per_cloud) += the converted slots [slot0, slot0 + B * per_cloud)
+static int fixed_finish(const FixedWs& f, int64_t slot0, int64_t B, int64_t per_cloud, int cbits, float* out, cudaStream_t s) {
+  fixed_to_f32_kernel<<<tr_grid(B * per_cloud, 256), 256, 0, s>>>(f.acc + slot0, f.flags + slot0, f.cmax, cbits, per_cloud,
+                                                                   B * per_cloud, out);
+  P3_LAUNCH_CHECK("fixed_to_f32_kernel");
+  return P3TOK_OK;
+}
+
 extern "C" int p3tok_scatter_rows_add_f32(const float* dRows, const int32_t* idx, int64_t B, int64_t N, int64_t G, int64_t k, int64_t D,
                                           float* dP, float* dF, void* stream) {
   P3_REQUIRE(B >= 0 && N > 0 && G >= 0 && k > 0 && D >= 0, P3TOK_ERR_INVALID, "scatter_rows_add_f32: bad shape");
   if (B * G == 0) return P3TOK_OK;
   P3_REQUIRE(dRows && idx && (dP || dF), P3TOK_ERR_INVALID, "scatter_rows_add_f32: null pointer");
-  scatter_rows_add_kernel<<<tr_grid(B * G * k * (3 + D), 256), 256, 0, as_stream(stream)>>>(dRows, idx, B, N, G * k, (int)D, dP, dF);
+  scatter_rows_add_kernel<<<tr_grid(B * G * k * (3 + D), 256), 256, 0, as_stream(stream)>>>(dRows, idx, B, N, G * k, (int)D, dP, dF,
+                                                                                            AtomicF32Add{});
   P3_LAUNCH_CHECK("scatter_rows_add_kernel");
+  return P3TOK_OK;
+}
+
+// one accumulator for both outputs: dP's slots [0, B*N*3), dF's [B*N*3, B*N*(3+D)); every destination receives at most G*k rows
+extern "C" int p3tok_scatter_rows_add_det_f32(const float* dRows, const int32_t* idx, int64_t B, int64_t N, int64_t G, int64_t k,
+                                              int64_t D, float* dP, float* dF, void* workspace, int64_t workspace_bytes, void* stream) {
+  P3_REQUIRE(B >= 0 && N > 0 && G >= 0 && k > 0 && D >= 0, P3TOK_ERR_INVALID, "scatter_rows_add_det_f32: bad shape");
+  if (B * G == 0) return P3TOK_OK;
+  P3_REQUIRE(dRows && idx && (dP || dF), P3TOK_ERR_INVALID, "scatter_rows_add_det_f32: null pointer");
+  cudaStream_t s = as_stream(stream);
+  FixedWs f;
+  int rc = fixed_begin(workspace, workspace_bytes, B, N, 3 + D, s, &f, "scatter_rows_add_det_f32");
+  if (rc != P3TOK_OK) return rc;
+  const int cbits = ceil_log2(G * k);
+  const unsigned grid = tr_grid(B * G * k * (3 + D), 256);
+  scatter_rows_add_kernel<<<grid, 256, 0, s>>>(dRows, idx, B, N, G * k, (int)D, dP, dF, CloudMaxAbs{f.cmax});
+  P3_LAUNCH_CHECK("scatter_rows_add_kernel");
+  scatter_rows_add_kernel<<<grid, 256, 0, s>>>(dRows, idx, B, N, G * k, (int)D, dP, dF, fixed_add(f, cbits, dF, B * N * 3));
+  P3_LAUNCH_CHECK("scatter_rows_add_kernel");
+  if (dP && (rc = fixed_finish(f, 0, B, N * 3, cbits, dP, s)) != P3TOK_OK) return rc;
+  if (dF && D > 0 && (rc = fixed_finish(f, B * N * 3, B, N * D, cbits, dF, s)) != P3TOK_OK) return rc;
   return P3TOK_OK;
 }
 
@@ -402,23 +688,47 @@ extern "C" int p3tok_build_rows_f32(const p3tok_rows* rows, float* X, void* stre
   return build_rows_f32(rows, 0, rows->B * rows->G, X, as_stream(stream));
 }
 
-extern "C" int p3tok_apf_rows_bwd_f32(const p3tok_rows* rows, const float* dRows, float* dX, void* stream) {
-  P3_REQUIRE(rows && rows->kind == 0, P3TOK_ERR_INVALID, "apf_rows_bwd_f32: APF (kind 0) rows expected");
-  P3_REQUIRE(rows->B >= 0 && rows->N > 0 && rows->G >= 0 && rows->k > 0 && rows->k < (1 << 30) && rows->C > 0,
-             P3TOK_ERR_INVALID, "apf_rows_bwd_f32: bad shape");
-  P3_REQUIRE(rows->idx_dtype == P3TOK_I64 || rows->idx_dtype == P3TOK_I32, P3TOK_ERR_INVALID, "apf_rows_bwd_f32: bad idx_dtype");
+template <typename Fin>
+static int launch_apf_rows_bwd(const p3tok_rows* rows, const float* dRows, float* dX, Fin fin, cudaStream_t s) {
   const int64_t BG = rows->B * rows->G;
-  if (BG == 0) return P3TOK_OK;
-  P3_REQUIRE(dRows && dX && rows->ctr_idx && rows->knn_idx, P3TOK_ERR_INVALID, "apf_rows_bwd_f32: null pointer");
-  cudaStream_t s = as_stream(stream);
   if (rows->idx_dtype == P3TOK_I64)
     apf_rows_bwd_kernel<int64_t><<<tr_grid(BG * rows->C, 256), 256, 0, s>>>(
-        dRows, rows->ctr_idx, static_cast<const int64_t*>(rows->knn_idx), rows->perm, rows->N, rows->G, (int)rows->k, rows->C, BG, dX);
+        dRows, rows->ctr_idx, static_cast<const int64_t*>(rows->knn_idx), rows->perm, rows->N, rows->G, (int)rows->k, rows->C, BG, dX, fin);
   else
     apf_rows_bwd_kernel<int32_t><<<tr_grid(BG * rows->C, 256), 256, 0, s>>>(
-        dRows, rows->ctr_idx, static_cast<const int32_t*>(rows->knn_idx), rows->perm, rows->N, rows->G, (int)rows->k, rows->C, BG, dX);
+        dRows, rows->ctr_idx, static_cast<const int32_t*>(rows->knn_idx), rows->perm, rows->N, rows->G, (int)rows->k, rows->C, BG, dX, fin);
   P3_LAUNCH_CHECK("apf_rows_bwd_kernel");
   return P3TOK_OK;
+}
+
+static int apf_rows_bwd_check(const p3tok_rows* rows, const float* dRows, const float* dX, const char* who) {
+  P3_REQUIRE(rows && rows->kind == 0, P3TOK_ERR_INVALID, "%s: APF (kind 0) rows expected", who);
+  P3_REQUIRE(rows->B >= 0 && rows->N > 0 && rows->G >= 0 && rows->k > 0 && rows->k < (1 << 30) && rows->C > 0,
+             P3TOK_ERR_INVALID, "%s: bad shape", who);
+  P3_REQUIRE(rows->idx_dtype == P3TOK_I64 || rows->idx_dtype == P3TOK_I32, P3TOK_ERR_INVALID, "%s: bad idx_dtype", who);
+  if (rows->B * rows->G == 0) return P3TOK_OK;
+  P3_REQUIRE(dRows && dX && rows->ctr_idx && rows->knn_idx, P3TOK_ERR_INVALID, "%s: null pointer", who);
+  return P3TOK_OK;
+}
+
+extern "C" int p3tok_apf_rows_bwd_f32(const p3tok_rows* rows, const float* dRows, float* dX, void* stream) {
+  const int rc = apf_rows_bwd_check(rows, dRows, dX, "apf_rows_bwd_f32");
+  if (rc != P3TOK_OK || rows->B * rows->G == 0) return rc;
+  return launch_apf_rows_bwd(rows, dRows, dX, AtomicF32Add{}, as_stream(stream));
+}
+
+// every destination receives at most G*k neighbour terms and G centre terms
+extern "C" int p3tok_apf_rows_bwd_det_f32(const p3tok_rows* rows, const float* dRows, float* dX, void* workspace, int64_t workspace_bytes,
+                                          void* stream) {
+  int rc = apf_rows_bwd_check(rows, dRows, dX, "apf_rows_bwd_det_f32");
+  if (rc != P3TOK_OK || rows->B * rows->G == 0) return rc;
+  cudaStream_t s = as_stream(stream);
+  FixedWs f;
+  if ((rc = fixed_begin(workspace, workspace_bytes, rows->B, rows->N, rows->C, s, &f, "apf_rows_bwd_det_f32")) != P3TOK_OK) return rc;
+  const int cbits = ceil_log2(rows->G * (rows->k + 1));
+  if ((rc = launch_apf_rows_bwd(rows, dRows, dX, CloudMaxAbs{f.cmax}, s)) != P3TOK_OK) return rc;
+  if ((rc = launch_apf_rows_bwd(rows, dRows, dX, fixed_add(f, cbits), s)) != P3TOK_OK) return rc;
+  return fixed_finish(f, 0, rows->B, rows->N * rows->C, cbits, dX, s);
 }
 
 extern "C" int p3tok_gather_points_bwd_f32(const float* dOut, int64_t B, int64_t N, int64_t C, const int64_t* idx, int64_t S, float* dX,
@@ -427,7 +737,26 @@ extern "C" int p3tok_gather_points_bwd_f32(const float* dOut, int64_t B, int64_t
   const int64_t total = B * S * C;
   if (total == 0) return P3TOK_OK;
   P3_REQUIRE(dOut && idx && dX, P3TOK_ERR_INVALID, "gather_points_bwd_f32: null pointer");
-  gather_points_bwd_kernel<<<tr_grid(total, 256), 256, 0, as_stream(stream)>>>(dOut, N, (int)C, idx, S, total, dX);
+  gather_points_bwd_kernel<<<tr_grid(total, 256), 256, 0, as_stream(stream)>>>(dOut, N, (int)C, idx, S, total, dX, AtomicF32Add{});
   P3_LAUNCH_CHECK("gather_points_bwd_kernel");
   return P3TOK_OK;
+}
+
+// every destination receives at most S contributions
+extern "C" int p3tok_gather_points_bwd_det_f32(const float* dOut, int64_t B, int64_t N, int64_t C, const int64_t* idx, int64_t S,
+                                               float* dX, void* workspace, int64_t workspace_bytes, void* stream) {
+  P3_REQUIRE(B >= 0 && N > 0 && C > 0 && S >= 0, P3TOK_ERR_INVALID, "gather_points_bwd_det_f32: bad shape");
+  const int64_t total = B * S * C;
+  if (total == 0) return P3TOK_OK;
+  P3_REQUIRE(dOut && idx && dX, P3TOK_ERR_INVALID, "gather_points_bwd_det_f32: null pointer");
+  cudaStream_t s = as_stream(stream);
+  FixedWs f;
+  int rc = fixed_begin(workspace, workspace_bytes, B, N, C, s, &f, "gather_points_bwd_det_f32");
+  if (rc != P3TOK_OK) return rc;
+  const int cbits = ceil_log2(S);
+  gather_points_bwd_kernel<<<tr_grid(total, 256), 256, 0, s>>>(dOut, N, (int)C, idx, S, total, dX, CloudMaxAbs{f.cmax});
+  P3_LAUNCH_CHECK("gather_points_bwd_kernel");
+  gather_points_bwd_kernel<<<tr_grid(total, 256), 256, 0, s>>>(dOut, N, (int)C, idx, S, total, dX, fixed_add(f, cbits));
+  P3_LAUNCH_CHECK("gather_points_bwd_kernel");
+  return fixed_finish(f, 0, B, N * C, cbits, dX, s);
 }

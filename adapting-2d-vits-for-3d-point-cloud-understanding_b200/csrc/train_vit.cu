@@ -90,7 +90,9 @@ ln_bwd_kernel(const float* __restrict__ dY, const float* __restrict__ X, int64_t
   }
 }
 
-// dgamma[c] = sum_m dy xhat, dbeta[c] = sum_m dy: column strips, fp32 inside a strip of 64 rows per lane, fp64 across
+// dgamma[c] = sum_m dy xhat, dbeta[c] = sum_m dy: column strips, fp32 inside a strip of 64 rows per lane, fp64 across.
+// kPartial: strip y stores its sums to dgamma[y][D] / dbeta[y][D] (a workspace; strip_sum_f64 adds the strips in order).
+template <bool kPartial>
 __global__ void __launch_bounds__(256)
 ln_param_grad_kernel(const float* __restrict__ dY, const float* __restrict__ X, int64_t M, int D, const float* __restrict__ mean,
                      const float* __restrict__ rstd, int64_t rows_per_block, double* __restrict__ dgamma,
@@ -117,8 +119,13 @@ ln_param_grad_kernel(const float* __restrict__ dY, const float* __restrict__ X, 
   if (rlane == 0 && c < D) {
 #pragma unroll
     for (int r = 1; r < 8; ++r) { a += ra[r][threadIdx.x & 31]; b += rb[r][threadIdx.x & 31]; }
-    atomicAdd(&dgamma[c], a);
-    atomicAdd(&dbeta[c], b);
+    if constexpr (kPartial) {
+      dgamma[(size_t)blockIdx.y * D + c] = a;
+      dbeta[(size_t)blockIdx.y * D + c] = b;
+    } else {
+      atomicAdd(&dgamma[c], a);
+      atomicAdd(&dbeta[c], b);
+    }
   }
 }
 
@@ -322,9 +329,29 @@ extern "C" int p3tok_ln_param_grad_f32(const float* dY, const float* X, int64_t 
   rows = (rows + 63) / 64 * 64;
   strips = (M + rows - 1) / rows;
   P3_REQUIRE(strips < 65536, P3TOK_ERR_UNSUPPORTED, "ln_param_grad_f32: too many rows");
-  ln_param_grad_kernel<<<dim3((unsigned)cgroups, (unsigned)strips), 256, 0, s>>>(dY, X, M, (int)D, mean, rstd, rows, dgamma, dbeta);
+  ln_param_grad_kernel<false><<<dim3((unsigned)cgroups, (unsigned)strips), 256, 0, s>>>(dY, X, M, (int)D, mean, rstd, rows, dgamma, dbeta);
   P3_LAUNCH_CHECK("ln_param_grad_kernel");
   return P3TOK_OK;
+}
+
+extern "C" int p3tok_ln_param_grad_det_f32(const float* dY, const float* X, int64_t M, int64_t D, const float* mean, const float* rstd,
+                                           double* dgamma, double* dbeta, void* workspace, int64_t workspace_bytes, void* stream) {
+  P3_REQUIRE(M >= 0 && D > 0 && D < (1 << 24), P3TOK_ERR_INVALID, "ln_param_grad_det_f32: bad shape");
+  P3_REQUIRE(dgamma && dbeta && (M == 0 || (dY && X && mean && rstd)), P3TOK_ERR_INVALID, "ln_param_grad_det_f32: null pointer");
+  cudaStream_t s = as_stream(stream);
+  if (M == 0) {
+    P3_CUDA(cudaMemsetAsync(dgamma, 0, (size_t)D * sizeof(double), s));
+    P3_CUDA(cudaMemsetAsync(dbeta, 0, (size_t)D * sizeof(double), s));
+    return P3TOK_OK;
+  }
+  const int rc = colsum_det_begin(workspace, workspace_bytes, M, D, "ln_param_grad_det_f32");
+  if (rc != P3TOK_OK) return rc;
+  const int64_t rows = strip_rows(M, (int)D), strips = (M + rows - 1) / rows;   // the strips of p3tok_ln_param_grad_f32
+  double* part = static_cast<double*>(workspace);
+  ln_param_grad_kernel<true><<<dim3((unsigned)((D + 31) / 32), (unsigned)strips), 256, 0, s>>>(dY, X, M, (int)D, mean, rstd, rows, part,
+                                                                                               part + strips * D);
+  P3_LAUNCH_CHECK("ln_param_grad_kernel");
+  return strip_sum_f64(part, M, (int)D, dgamma, dbeta, s);
 }
 
 static int attn_shape_ok(int64_t B, int64_t G, int64_t heads, int64_t hd, int row_bufs, const char* who) {

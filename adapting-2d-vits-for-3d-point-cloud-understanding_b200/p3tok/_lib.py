@@ -107,6 +107,16 @@ _SIGNATURES = {
     "p3tok_layernorm_split": (_int, [_vp, _i64, _i64, _f32, _vp, _vp, _vp, _vp]),
     "p3tok_attention_x3": (_int, [_vp, _i64, _i64, _i64, _i64, _vp, _vp]),
     "p3tok_linear_bf16_ex": (_int, [_vp, _i64, _i64, _vp, _i64, _vp, _int, _i64, _vp, _f32, _f32, _vp, _vp, _vp]),
+    "p3tok_linear_tn_det_workspace_bytes": (_i64, [_i64, _i64, _i64]),
+    "p3tok_linear_tn_det_f32": (_int, [_vp, _vp, _i64, _i64, _i64, _vp, _int, _vp, _i64, _vp]),
+    "p3tok_colsum_det_workspace_bytes": (_i64, [_i64, _i64]),
+    "p3tok_colstats_det_f32": (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _i64, _vp]),
+    "p3tok_bn_bwd_stats_det_f32": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _int, _vp, _vp, _vp, _i64, _vp]),
+    "p3tok_ln_param_grad_det_f32": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "p3tok_scatter_det_workspace_bytes": (_i64, [_i64, _i64, _i64]),
+    "p3tok_scatter_rows_add_det_f32": (_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _i64, _vp]),
+    "p3tok_apf_rows_bwd_det_f32": (_int, [ctypes.POINTER(RowsStruct), _vp, _vp, _vp, _i64, _vp]),
+    "p3tok_gather_points_bwd_det_f32": (_int, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _vp, _i64, _vp]),
 }
 
 

@@ -415,8 +415,22 @@ def _(pnts, feats, idx):
 # ------------------------------------------------------------------------------- gradients of the gathers
 # gather_points, apf_group and group_gather are differentiable with respect to their point / feature inputs, as the
 # reference's index_points and advanced-index gathers are (sampler.py:77-94, apf.py:70-95, pix4point.py:92-102); index inputs
-# get no gradient.  Each adjoint is an op of its own over csrc/train.cu; it scatters with fp32 atomic adds, so the gradient
-# is reproducible to rounding, not bit for bit.
+# get no gradient.  Each adjoint is an op of its own over csrc/train.cu.  By default it scatters with fp32 atomic adds, so the
+# gradient is reproducible to rounding, not bit for bit.  Under torch.use_deterministic_algorithms (deterministic(), read when
+# the adjoint runs) it calls the *_det_f32 kernels instead: fixed-point integer sums with a per-cloud power-of-two scale,
+# converted to fp32 once per call - bit-identical from run to run, and each cloud's gradient independent of the rest of the batch.
+def deterministic() -> bool:
+    """True while torch.use_deterministic_algorithms is on (warn_only included).  The wrappers of the kernels that finish their
+    sums with floating-point atomics (these adjoints; train.linear_tn, colstats, bn_backward, GatherRowsFn;
+    train_vit.ln_param_grad) then launch their deterministic versions.  Read at call time, as torch's own ops do."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _scatter_ws(B: int, N: int, C: int, device) -> torch.Tensor:
+    """Scratch of a fixed-point scatter, on the current stream's allocator (the library allocates nothing)."""
+    return torch.empty(int(_L().p3tok_scatter_det_workspace_bytes(B, N, C)), dtype=torch.uint8, device=device)
+
+
 @torch.library.custom_op("p3tok::gather_points_bwd", mutates_args=(), device_types="cuda")
 def gather_points_bwd(grad: torch.Tensor, idx: torch.Tensor, N: int) -> torch.Tensor:
     """grad (*idx.shape, C) -> dX (B,N,C): the adjoint of gather_points (p3tok_gather_points_bwd_f32)."""
@@ -426,8 +440,13 @@ def gather_points_bwd(grad: torch.Tensor, idx: torch.Tensor, N: int) -> torch.Te
     flat = idx.to(torch.int64).reshape(B, -1).contiguous()
     dx = torch.zeros((B, N, C), dtype=torch.float32, device=g.device)
     with torch.cuda.device(g.device), _timed("gather_bwd"):
-        check(_L().p3tok_gather_points_bwd_f32(g.data_ptr(), B, N, C, flat.data_ptr(), int(flat.shape[1]), dx.data_ptr(), _stream()),
-              "gather_points_bwd")
+        if deterministic():
+            ws = _scatter_ws(B, N, C, g.device)
+            check(_L().p3tok_gather_points_bwd_det_f32(g.data_ptr(), B, N, C, flat.data_ptr(), int(flat.shape[1]), dx.data_ptr(),
+                                                       ws.data_ptr(), ws.numel(), _stream()), "gather_points_bwd_det")
+        else:
+            check(_L().p3tok_gather_points_bwd_f32(g.data_ptr(), B, N, C, flat.data_ptr(), int(flat.shape[1]), dx.data_ptr(), _stream()),
+                  "gather_points_bwd")
     return dx
 
 
@@ -466,16 +485,23 @@ def apf_rows_descriptor(B: int, N: int, C: int, fps_idx: torch.Tensor, knn_idx: 
 def apf_group_bwd(grad_neigh: Optional[torch.Tensor], grad_center: Optional[torch.Tensor], fps_idx: torch.Tensor,
                   knn_idx: torch.Tensor, perm: Optional[torch.Tensor], N: int, C: int) -> torch.Tensor:
     """The adjoint of apf_group -> dX (B,N,C): the neighbourhood rows through p3tok_apf_rows_bwd_f32, the centres (xyz of
-    x[b, fps_idx[b, perm[b,j]]]) through p3tok_gather_points_bwd_f32.  Either gradient may be None."""
+    x[b, fps_idx[b, perm[b,j]]]) through p3tok_gather_points_bwd_f32.  Either gradient may be None.  Deterministic mode: the
+    *_det_f32 versions, the neighbourhood part converted and added to dX first, then the centre part."""
     _need_cuda("apf_group_bwd", grad_neigh, grad_center, fps_idx, knn_idx, perm)
     B, G = int(knn_idx.shape[0]), int(knn_idx.shape[1])
     dx = torch.zeros((B, N, C), dtype=torch.float32, device=fps_idx.device)
     L = _L()
+    det = deterministic()
+    ws = _scatter_ws(B, N, C, dx.device) if det else None
     with torch.cuda.device(dx.device), _timed("apf_group_bwd"):
         if grad_neigh is not None:
             g = grad_neigh.float().contiguous()
             r, keep = apf_rows_descriptor(B, N, C, fps_idx, knn_idx, perm)
-            check(L.p3tok_apf_rows_bwd_f32(ctypes.byref(r), g.data_ptr(), dx.data_ptr(), _stream()), "apf_rows_bwd_f32")
+            if det:
+                check(L.p3tok_apf_rows_bwd_det_f32(ctypes.byref(r), g.data_ptr(), dx.data_ptr(), ws.data_ptr(), ws.numel(), _stream()),
+                      "apf_rows_bwd_det_f32")
+            else:
+                check(L.p3tok_apf_rows_bwd_f32(ctypes.byref(r), g.data_ptr(), dx.data_ptr(), _stream()), "apf_rows_bwd_f32")
             del keep
         if grad_center is not None:
             src = fps_idx.to(torch.int64)
@@ -484,8 +510,12 @@ def apf_group_bwd(grad_neigh: Optional[torch.Tensor], grad_center: Optional[torc
             if C != 3:                                     # the centres are channels 0..2 of the gathered rows
                 gc = torch.nn.functional.pad(gc, (0, C - 3))
             gc = gc.contiguous()
-            check(L.p3tok_gather_points_bwd_f32(gc.data_ptr(), B, N, C, src.data_ptr(), G, dx.data_ptr(), _stream()),
-                  "gather_points_bwd")
+            if det:
+                check(L.p3tok_gather_points_bwd_det_f32(gc.data_ptr(), B, N, C, src.data_ptr(), G, dx.data_ptr(), ws.data_ptr(),
+                                                        ws.numel(), _stream()), "gather_points_bwd_det")
+            else:
+                check(L.p3tok_gather_points_bwd_f32(gc.data_ptr(), B, N, C, src.data_ptr(), G, dx.data_ptr(), _stream()),
+                      "gather_points_bwd")
     return dx
 
 
@@ -526,8 +556,14 @@ def group_gather_bwd(grad_p: Optional[torch.Tensor], grad_f: Optional[torch.Tens
     dp = torch.zeros((B, N, 3) if need_p else (0,), dtype=torch.float32, device=dev)
     df = torch.zeros((B, N, D) if need_f else (0,), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev), _timed("group_gather_bwd"):
-        check(_L().p3tok_scatter_rows_add_f32(drows.data_ptr(), i32.data_ptr(), B, N, G, k, D, dp.data_ptr() if need_p else None,
-                                              df.data_ptr() if need_f else None, _stream()), "scatter_rows_add_f32")
+        if deterministic():
+            ws = _scatter_ws(B, N, 3 + D, dev)
+            check(_L().p3tok_scatter_rows_add_det_f32(drows.data_ptr(), i32.data_ptr(), B, N, G, k, D, dp.data_ptr() if need_p else None,
+                                                      df.data_ptr() if need_f else None, ws.data_ptr(), ws.numel(), _stream()),
+                  "scatter_rows_add_det_f32")
+        else:
+            check(_L().p3tok_scatter_rows_add_f32(drows.data_ptr(), i32.data_ptr(), B, N, G, k, D, dp.data_ptr() if need_p else None,
+                                                  df.data_ptr() if need_f else None, _stream()), "scatter_rows_add_f32")
     return dp, df
 
 

@@ -17,6 +17,12 @@ eval-mode modules whose input wants a gradient (adversarial attacks, saliency) -
 variance, no update, no all-reduce), and the weight-gradient products of parameters that do not require grad are skipped.
 ApfRowsFn builds the APF rows and sends their gradient back to the input points.
 
+Reproducible runs: under torch.use_deterministic_algorithms (`deterministic()`, read when each wrapper runs) the kernels that
+finish their sums with floating-point atomics - the weight-gradient GEMM, the column sums of the BatchNorm statistics and bias
+gradients, the BatchNorm backward sums and the gather adjoints - are replaced by ordered reductions (per-slice / per-strip
+partials in a workspace, summed in ascending order in fp64) and fixed-point scatters; the step is then bit-identical from run to
+run.  Results differ from the default path in the last bits.
+
 fp32 on CUDA cores; per-channel sums in fp64.  The eval-mode (serving) path is the tensor-core one; this path exists so that
 the kernels can replace the reference inside its trainers and wherever the reference is differentiated.  Opt-in:
 P3TOK_TRAIN_TC=1 (or `set_tensor_core_gemms(1)`) sends the forward and dX products through the fp32-accurate bf16x3 tensor-core GEMM (`p3tok_linear_x3_f32`: operands split into bf16
@@ -33,6 +39,7 @@ import torch
 
 from . import _lib, ops
 from ._lib import check
+from .ops import deterministic
 
 
 def _L():
@@ -61,6 +68,10 @@ def set_tensor_core_gemms(level: int) -> int:
     global _TC_LEVEL
     prev, _TC_LEVEL = _TC_LEVEL, int(level)
     return prev
+
+
+def _workspace(nbytes: int, device) -> torch.Tensor:
+    return torch.empty(int(nbytes), dtype=torch.uint8, device=device)
 
 
 def _linear_x3(a: torch.Tensor, w: torch.Tensor, b, g, rows_per_group: int) -> torch.Tensor:
@@ -100,8 +111,14 @@ def linear_tn(dy: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
     M, N = dy.shape
     K = x.shape[1]
     out = torch.empty((N, K), dtype=torch.float32, device=dy.device)
+    L = _L()
     with torch.cuda.device(dy.device):
-        check(_L().p3tok_linear_tn_f32(dy.data_ptr(), x.data_ptr(), M, N, K, out.data_ptr(), 0, _s()), "linear_tn_f32")
+        if deterministic():
+            ws = _workspace(L.p3tok_linear_tn_det_workspace_bytes(M, N, K), dy.device)
+            check(L.p3tok_linear_tn_det_f32(dy.data_ptr(), x.data_ptr(), M, N, K, out.data_ptr(), 0, ws.data_ptr(), ws.numel(), _s()),
+                  "linear_tn_det_f32")
+        else:
+            check(L.p3tok_linear_tn_f32(dy.data_ptr(), x.data_ptr(), M, N, K, out.data_ptr(), 0, _s()), "linear_tn_f32")
     return out
 
 
@@ -110,8 +127,14 @@ def colstats(x: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
     M, N = x.shape
     s = torch.empty(N, dtype=torch.float64, device=x.device)
     q = torch.empty(N, dtype=torch.float64, device=x.device)
+    L = _L()
     with torch.cuda.device(x.device):
-        check(_L().p3tok_colstats_f32(x.data_ptr(), M, N, s.data_ptr(), q.data_ptr(), _s()), "colstats_f32")
+        if deterministic():
+            ws = _workspace(L.p3tok_colsum_det_workspace_bytes(M, N), x.device)
+            check(L.p3tok_colstats_det_f32(x.data_ptr(), M, N, s.data_ptr(), q.data_ptr(), ws.data_ptr(), ws.numel(), _s()),
+                  "colstats_det_f32")
+        else:
+            check(L.p3tok_colstats_f32(x.data_ptr(), M, N, s.data_ptr(), q.data_ptr(), _s()), "colstats_f32")
     return s, q
 
 
@@ -212,9 +235,15 @@ def bn_backward(dy: torch.Tensor, z: torch.Tensor, st: BNState, gamma: torch.Ten
     s12 = (torch.empty if stats else torch.zeros)(2 * N, dtype=torch.float64, device=z.device)
     local = None
     with torch.cuda.device(z.device):
-        if stats:
+        if stats and deterministic():
+            ws = _workspace(_L().p3tok_colsum_det_workspace_bytes(M, N), z.device)
+            check(_L().p3tok_bn_bwd_stats_det_f32(dy.data_ptr(), z.data_ptr(), M, N, st.mean.data_ptr(), st.rstd.data_ptr(),
+                                                  g.data_ptr(), b.data_ptr(), int(relu), s12.data_ptr(), s12.data_ptr() + 8 * N,
+                                                  ws.data_ptr(), ws.numel(), _s()), "bn_bwd_stats_det_f32")
+        elif stats:
             check(_L().p3tok_bn_bwd_stats_f32(dy.data_ptr(), z.data_ptr(), M, N, st.mean.data_ptr(), st.rstd.data_ptr(), g.data_ptr(),
                                               b.data_ptr(), int(relu), s12.data_ptr(), s12.data_ptr() + 8 * N, _s()), "bn_bwd_stats_f32")
+        if stats:
             local = s12.clone()
             if st.running:
                 s12.zero_()
@@ -401,10 +430,15 @@ class GatherRowsFn(torch.autograd.Function):
         dp = torch.zeros((B, N, 3), dtype=torch.float32, device=drows.device) if ctx.needs_input_grad[0] else None
         df = torch.zeros((B, N, D), dtype=torch.float32, device=drows.device) if ctx.needs_input_grad[1] else None
         if dp is not None or df is not None:
+            pp, fp = (dp.data_ptr() if dp is not None else None), (df.data_ptr() if df is not None else None)
             with torch.cuda.device(drows.device):
-                check(_L().p3tok_scatter_rows_add_f32(drows.data_ptr(), i32.data_ptr(), B, N, G, k, D,
-                                                      dp.data_ptr() if dp is not None else None,
-                                                      df.data_ptr() if df is not None else None, _s()), "scatter_rows_add_f32")
+                if deterministic():
+                    ws = _workspace(_L().p3tok_scatter_det_workspace_bytes(B, N, 3 + D), drows.device)
+                    check(_L().p3tok_scatter_rows_add_det_f32(drows.data_ptr(), i32.data_ptr(), B, N, G, k, D, pp, fp, ws.data_ptr(),
+                                                              ws.numel(), _s()), "scatter_rows_add_det_f32")
+                else:
+                    check(_L().p3tok_scatter_rows_add_f32(drows.data_ptr(), i32.data_ptr(), B, N, G, k, D, pp, fp, _s()),
+                          "scatter_rows_add_f32")
         return dp, df, None
 
 

@@ -20,7 +20,7 @@ import torch
 
 from . import _lib
 from ._lib import check
-from .train import _L, _f32, _s, _t, bn_backward, bn_forward, colstats, colsum, group_max_arg, group_max_bwd, linear, linear_tn
+from .train import _L, _f32, _s, _t, deterministic, bn_backward, bn_forward, colstats, colsum, group_max_arg, group_max_bwd, linear, linear_tn
 
 # parameter order of one APFViTLayer (state_dict names relative to the layer)
 LAYER_PARAMS = ("norm1.weight", "norm1.bias", "attention.qkv.weight", "attention.qkv.bias", "attention.proj.weight",
@@ -66,8 +66,13 @@ def ln_param_grad(dy: torch.Tensor, x: torch.Tensor, mean: torch.Tensor, rstd: t
     M, D = x.shape
     g = torch.empty(2 * D, dtype=torch.float64, device=x.device)
     with torch.cuda.device(x.device):
-        check(_L().p3tok_ln_param_grad_f32(dy.data_ptr(), x.data_ptr(), M, D, mean.data_ptr(), rstd.data_ptr(), g.data_ptr(),
-                                           g.data_ptr() + 8 * D, _s()), "ln_param_grad_f32")
+        if deterministic():
+            ws = torch.empty(int(_L().p3tok_colsum_det_workspace_bytes(M, D)), dtype=torch.uint8, device=x.device)
+            check(_L().p3tok_ln_param_grad_det_f32(dy.data_ptr(), x.data_ptr(), M, D, mean.data_ptr(), rstd.data_ptr(), g.data_ptr(),
+                                                   g.data_ptr() + 8 * D, ws.data_ptr(), ws.numel(), _s()), "ln_param_grad_det_f32")
+        else:
+            check(_L().p3tok_ln_param_grad_f32(dy.data_ptr(), x.data_ptr(), M, D, mean.data_ptr(), rstd.data_ptr(), g.data_ptr(),
+                                               g.data_ptr() + 8 * D, _s()), "ln_param_grad_f32")
     return g[:D].float(), g[D:].float()
 
 

@@ -368,7 +368,8 @@ P3TOK_API int p3tok_build_rows_f32(const p3tok_rows* rows, float* X, void* strea
 
 /* ---- gradients with respect to the input points (adversarial examples, saliency) -------------------------------------------
  * Both functions ACCUMULATE into dX (the caller zeroes it) with fp32 atomic adds, like p3tok_scatter_rows_add_f32 and torch's
- * own CUDA index backward: the result is reproducible to rounding, not bit for bit (the order of the adds varies). */
+ * own CUDA index backward: the result is reproducible to rounding, not bit for bit (the order of the adds varies; the *_det_f32
+ * versions further down are bit-reproducible). */
 /* Adjoint of p3tok_build_rows_f32 for kind 0 (APF): dRows (B*G*k, 2C) in the rows' output order (group j = input group
  * perm[b,j]) -> dX (B,N,C) += d rel at x[b,nbr] and sum over the group's k rows of (d ctr - d rel) at x[b,ctr].  rows->x is not
  * read; knn_idx is int64 or int32 (rows->idx_dtype). */
@@ -376,6 +377,48 @@ P3TOK_API int p3tok_apf_rows_bwd_f32(const p3tok_rows* rows, const float* dRows,
 /* Adjoint of p3tok_gather_points: dOut (B,S,C), idx (B,S) int64 -> dX (B,N,C) += dOut at the gathered rows. */
 P3TOK_API int p3tok_gather_points_bwd_f32(const float* dOut, int64_t B, int64_t N, int64_t C, const int64_t* idx, int64_t S,
                                           float* dX, void* stream);
+
+/* ---- deterministic reductions (for torch.use_deterministic_algorithms) ----------------------------------------------------
+ * The functions above that finish their sums with floating-point atomics (p3tok_linear_tn_f32, p3tok_colstats_f32,
+ * p3tok_bn_bwd_stats_f32, p3tok_ln_param_grad_f32, p3tok_scatter_rows_add_f32, p3tok_apf_rows_bwd_f32,
+ * p3tok_gather_points_bwd_f32) round in the order the CTAs arrive.  Each *_det_f32 below computes the same quantity with the same
+ * arguments plus a caller-owned workspace (16-byte aligned, at least the matching *_workspace_bytes(); the library allocates
+ * nothing), and its result is a function of the inputs and shapes only: bit-identical across calls, streams, concurrent load and
+ * processes.  Launch geometry comes from the shapes, never from a device query.
+ *
+ * Ordered reductions.  p3tok_linear_tn_det_f32 splits M into the slices p3tok_linear_tn_f32 uses (rows per slice: a multiple of
+ * 256 such that ceil(148*4 / (ceil(N/64) ceil(K/64))) slices cover M); slice z stores its fp32 partial dY_z^T X_z to
+ * workspace[z][N][K], and dW = fp32(sum over z ascending, in fp64) (+ the old dW once when accumulate).  The three column-strip
+ * reductions store the fp64 partials of strip y (the strips of the *_f32 versions) to workspace[0][y][N] (sum / s1 / dgamma) and
+ * workspace[1][y][N] (sumsq / s2 / dbeta) and add the strips in ascending order in fp64.
+ *
+ * Fixed-point scatters.  Per cloud b, m_b = the largest finite |contribution| and K = a bound on the contributions one destination
+ * receives (gather_points: S; apf_rows: G*(k+1); scatter_rows: G*k), s_b = 61 - ceil(log2 K) - e with m_b < 2^e (frexp; s_b = 0
+ * when m_b = 0).  Each contribution v adds rint(v 2^s_b) to an int64 accumulator (one per call, shared by all of the call's
+ * outputs; the APF centre term sum_n (d ctr - d rel), summed in fp32 in ascending n, is one contribution), and dX +=
+ * fp32(sum) 2^-s_b.  Non-finite contributions follow IEEE addition per destination (any NaN or +inf with -inf: NaN; otherwise the
+ * infinity).  A cloud's result does not depend on the other clouds of the batch. */
+P3TOK_API int64_t p3tok_linear_tn_det_workspace_bytes(int64_t M, int64_t N, int64_t K);
+P3TOK_API int p3tok_linear_tn_det_f32(const float* dY, const float* X, int64_t M, int64_t N, int64_t K, float* dW, int accumulate,
+                                      void* workspace, int64_t workspace_bytes, void* stream);
+/* workspace of p3tok_colstats_det_f32, p3tok_bn_bwd_stats_det_f32 and p3tok_ln_param_grad_det_f32 (N = D) */
+P3TOK_API int64_t p3tok_colsum_det_workspace_bytes(int64_t M, int64_t N);
+P3TOK_API int p3tok_colstats_det_f32(const float* X, int64_t M, int64_t N, double* sum, double* sumsq, void* workspace,
+                                     int64_t workspace_bytes, void* stream);
+P3TOK_API int p3tok_bn_bwd_stats_det_f32(const float* dY, const float* Z, int64_t M, int64_t N, const float* mean, const float* rstd,
+                                         const float* gamma, const float* beta, int relu, double* s1, double* s2, void* workspace,
+                                         int64_t workspace_bytes, void* stream);
+P3TOK_API int p3tok_ln_param_grad_det_f32(const float* dY, const float* X, int64_t M, int64_t D, const float* mean, const float* rstd,
+                                          double* dgamma, double* dbeta, void* workspace, int64_t workspace_bytes, void* stream);
+/* workspace of the scatters for B clouds of N points with C channels (p3tok_scatter_rows_add_det_f32: C = 3 + D):
+ * 12 bytes per (point, channel) + 4 per cloud */
+P3TOK_API int64_t p3tok_scatter_det_workspace_bytes(int64_t B, int64_t N, int64_t C);
+P3TOK_API int p3tok_scatter_rows_add_det_f32(const float* dRows, const int32_t* idx, int64_t B, int64_t N, int64_t G, int64_t k,
+                                             int64_t D, float* dP, float* dF, void* workspace, int64_t workspace_bytes, void* stream);
+P3TOK_API int p3tok_apf_rows_bwd_det_f32(const p3tok_rows* rows, const float* dRows, float* dX, void* workspace, int64_t workspace_bytes,
+                                         void* stream);
+P3TOK_API int p3tok_gather_points_bwd_det_f32(const float* dOut, int64_t B, int64_t N, int64_t C, const int64_t* idx, int64_t S,
+                                              float* dX, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- training through the ViT block stack (SURVEY 8f "next" #4 on top of #3) -------------------------------------------
  * The reference keeps the blocks frozen but trains point_encoder / encoder_norm / head (src/models/apf.py:335-346), so a
